@@ -189,6 +189,96 @@ def mini_batches(lens, max_bases):
     return out
 
 
+DUMP_BUDGET = 64000000  # bytes of all --dump-outputs arrays together
+
+
+def dump_outputs(out_dir, n, result_of):
+    """Write what mg_map_batch() returned for a fixed, seeded sample of the n reads as out_dir/<name>.npy.  Reads are taken in
+    the order of a seeded permutation while all arrays together stay within DUMP_BUDGET bytes; rows are in read order and
+    "row" columns number the reads (or graph chains) of the sample from 0.  float64 holds every integer exactly: 64-bit
+    anchors are split into 32-bit halves.  result_of(i) is the mg_gchains_t pointer of read i (NULL: no result object).
+      read_index [R]      read number in the input
+      reads      [R, 4]   n_gc, n_lc, n_a, rep_len (all -1: no result object)
+      gchains    [G, 28]  read row, id, parent, off, cnt, n_anchor, score, qs, qe, plen, ps, pe, blen, mlen, div, hash, subsc, n_sub,
+                          mapq, flt, n_cigar, cigar mlen, blen, aplen, ss, ee (-1 from n_cigar on: no CIGAR), ds len, n_off (-1: no ds)
+      cigar      [C, 3]   gchain row, operation length, operation code
+      lchains    [L, 6]   read row, off, cnt, v, score, ed
+      anchors    [A, 5]   read row, x >> 32, x & 0xffffffff, y >> 32, y & 0xffffffff
+      ds         [D]      the ds strings of the graph chains in gchain order, one byte per element (float32)
+      ds_off     [O, 2]   gchain row, offset
+    Returns (number of reads written, bytes written)."""
+    import random
+    import numpy as np
+    from minigraph_b200 import capi
+
+    def size_of(p):  # bytes the read adds to the arrays
+        if not p:
+            return 8 * 5
+        gs, b = p.contents, 8 * (5 + 6 * p.contents.n_lc + 5 * p.contents.n_a)
+        for j in range(gs.n_gc):
+            g = gs.gc[j]
+            b += 8 * 28 + (24 * g.p.contents.n_cigar if g.p else 0) + (4 * g.ds.len + 16 * g.ds.n_off if g.ds.ds else 0)
+        return b
+    picked, total = [], 8 * 128  # the .npy headers
+    for i in random.Random(12345).sample(range(n), n):
+        b = size_of(result_of(i))
+        if total + b > DUMP_BUDGET:
+            break
+        picked.append(i)
+        total += b
+    picked.sort()
+    out = {k: [] for k in ("reads", "gchains", "cigar", "lchains", "anchors", "ds", "ds_off")}
+    n_gc_rows = 0
+    for r, i in enumerate(picked):
+        p = result_of(i)
+        if not p:
+            out["reads"].append(np.full((1, 4), -1.0))
+            continue
+        gs = p.contents
+        out["reads"].append(np.array([[gs.n_gc, gs.n_lc, gs.n_a, gs.rep_len]], dtype=np.float64))
+        for j in range(gs.n_gc):
+            g, row = gs.gc[j], n_gc_rows + j
+            cols = [r, g.id, g.parent, g.off, g.cnt, g.n_anchor, g.score, g.qs, g.qe, g.plen, g.ps, g.pe, g.blen, g.mlen, g.div, g.hash,
+                    g.subsc, g.n_sub, g.mapq, g.flt]
+            if g.p:
+                c = g.p.contents
+                cols += [c.n_cigar, c.mlen, c.blen, c.aplen, c.ss, c.ee]
+                ops = np.frombuffer((C.c_uint64 * c.n_cigar).from_address(C.addressof(c) + C.sizeof(capi.mg_cigar_t)), dtype=np.uint64)
+                out["cigar"].append(np.stack([np.full(c.n_cigar, float(row)), (ops >> np.uint64(4)).astype(np.float64),
+                                              (ops & np.uint64(15)).astype(np.float64)], axis=1))
+            else:
+                cols += [-1] * 6
+            if g.ds.ds:
+                cols += [g.ds.len, g.ds.n_off]
+                out["ds"].append(np.frombuffer(C.string_at(g.ds.ds, g.ds.len), dtype=np.uint8).astype(np.float32))
+                offs = np.ctypeslib.as_array(g.ds.off, shape=(g.ds.n_off,)).astype(np.float64) if g.ds.n_off else np.zeros(0)
+                out["ds_off"].append(np.stack([np.full(g.ds.n_off, float(row)), offs], axis=1))
+            else:
+                cols += [-1, -1]
+            out["gchains"].append(np.array([cols], dtype=np.float64))
+        n_gc_rows += gs.n_gc
+        for j in range(gs.n_lc):
+            lc = gs.lc[j]
+            out["lchains"].append(np.array([[r, lc.off, lc.cnt, lc.v, lc.score, lc.ed]], dtype=np.float64))
+        if gs.n_a > 0:
+            a = np.frombuffer((C.c_uint64 * (2 * gs.n_a)).from_address(C.addressof(gs.a.contents)), dtype=np.uint64).reshape(-1, 2)
+            hi, lo = (a >> np.uint64(32)).astype(np.float64), (a & np.uint64(0xffffffff)).astype(np.float64)
+            out["anchors"].append(np.stack([np.full(gs.n_a, float(r)), hi[:, 0], lo[:, 0], hi[:, 1], lo[:, 1]], axis=1))
+    width = {"reads": 4, "gchains": 28, "cigar": 3, "lchains": 6, "anchors": 5, "ds_off": 2}
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"read_index": np.array(picked, dtype=np.float64)}
+    for k, v in out.items():
+        empty = np.zeros(0, dtype=np.float32) if k == "ds" else np.zeros((0, width[k]))
+        arrays[k] = np.concatenate(v) if v else empty
+    written = 0
+    for k, v in arrays.items():
+        fn = os.path.join(out_dir, k + ".npy")
+        np.save(fn, v)
+        written += os.path.getsize(fn)
+    assert written <= DUMP_BUDGET, written
+    return len(picked), written
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -201,7 +291,11 @@ def main():
     ap.add_argument("--pipe", type=int, default=3, help="host threads calling mg_map_batch() at once")
     ap.add_argument("--no-cpu", action="store_true", help="skip the reference run on the host cores (no cpu_baseline, no parity check): profiling runs")
     ap.add_argument("--check", default="all", help="'all': after the timed region the GAF text of every read of rank 0 is compared with the reference binary's, byte for byte; N: the first N reads; 0: skip")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned for a seeded sample of rank 0's reads "
+                    "as DIR/<name>.npy (float32/float64, at most 64 MB; see dump_outputs) to compare two builds output for output")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     # stdout carries exactly one JSON line: everything libraries print to fd 1 (NCCL's version banner, ...) goes to stderr instead
     sys.stdout.flush()
     json_out = os.fdopen(os.dup(1), "w")
@@ -322,8 +416,11 @@ def main():
     kern = [0.0] * 10
     last_st = capi.mgb_stats_t()
 
-    def run_steps(n_steps, pipelined, record):
-        """n_steps passes over the reads.  pipelined: n_pipe threads map successive mini-batches, a writer formats them in order."""
+    last = {}  # --dump-outputs: mini-batch -> results of the last step of the last timed region, freed once written out
+
+    def run_steps(n_steps, pipelined, record, keep_last=False):
+        """n_steps passes over the reads.  pipelined: n_pipe threads map successive mini-batches, a writer formats them in order.
+        keep_last: the writer keeps the results of the last step in `last` instead of freeing them."""
         jobs = [(s, k) for s in range(n_steps) for k in range(M)]
         results = queue.Queue(maxsize=2 * n_pipe + 2)
         nxt = [0]
@@ -376,7 +473,10 @@ def main():
                     t0 = time.perf_counter()
                     lib.mgb_write_gaf_batch(g, hi - lo, gcs, sub(qlens, C.c_int, lo), sub(cnames, C.c_char_p, lo), mo.flag, gaf_threads,
                                             C.byref(gaf_buf[k]), C.byref(gaf_len[k]), C.byref(gaf_cap[k]))
-                    lib.mgb_free_batch(hi - lo, gcs)
+                    if keep_last and jobs[want][0] == n_steps - 1:
+                        last[k] = gcs
+                    else:
+                        lib.mgb_free_batch(hi - lo, gcs)
                     if record:
                         acc["gaf"] += (time.perf_counter() - t0) * 1e3
                     want += 1
@@ -410,7 +510,7 @@ def main():
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
-    run_steps(a.steps, False, True)
+    run_steps(a.steps, False, True, keep_last=bool(a.dump_outputs) and rank == 0)
     torch.cuda.synchronize()
     t_kern = acc["span"] / 1e3
     if world > 1:
@@ -433,6 +533,16 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+
+    dumped = None
+    if a.dump_outputs:
+        def result_of(i):
+            k = next(k for k, (lo, hi) in enumerate(mbs) if lo <= i < hi)
+            return last[k][i - mbs[k][0]]
+        n_dump, dump_bytes = dump_outputs(a.dump_outputs, n, result_of)
+        for k, (lo, hi) in enumerate(mbs):
+            lib.mgb_free_batch(hi - lo, last[k])
+        dumped = {"dir": a.dump_outputs, "reads": n_dump, "bytes": dump_bytes}
 
     # ---- untimed: the reference on the host cores, once: CPU baseline and, from its output, the parity check ----
     check, cpu = None, None
@@ -502,6 +612,8 @@ def main():
         "cpu_baseline": cpu, "parity_check": check,
         "clocks": sampler.summary(),
     }
+    if dumped:
+        out["outputs_dumped"] = dumped
     if dry:
         out["INVALID"] = "MGB_BENCH_DRY: CPU simulator, not a measurement"
     json_out.write(json.dumps(out) + "\n")

@@ -5,8 +5,6 @@ import os
 import mgtest as T
 
 
-class capi_u128(__import__("ctypes").Structure):
-    _fields_ = [("x", __import__("ctypes").c_uint64), ("y", __import__("ctypes").c_uint64)]
 from minigraph_b200 import capi  # noqa: E402
 
 G = os.path.join(T.REPO, "tests", "golden")
@@ -35,7 +33,7 @@ def case_golden_large(lib, workdir, which=("L2", "L3", "L4")):
         pre, reads = os.path.join(workdir, "svL"), os.path.join(workdir, "svL.reads.fa")
         T.sim_graph(pre, 1000000, 8, 7)
         T.sim_reads(pre + ".hap.fa", reads, 240, 15000, "ont", 105)
-        check_gaf(lib, pre + ".gfa", reads, "lr", golden_gz("L3_sv1m_h8_s7_240x15k_ont_s105.lr.gaf.gz"))
+        check_gaf_lines(lib, pre + ".gfa", reads, "lr", golden("L3_sv1m_h8_s7_240x15k_ont_s105.lr.gaf.b2").split())
     if "L4" in which:
         reads = os.path.join(workdir, "mthL.reads.fa")
         T.sim_reads(os.path.join(T.FIX, "MT-human.fa"), reads, 200, 20000, "hifi", 113, circular=True)
@@ -58,6 +56,19 @@ def check_gaf(lib, gfa, fasta, preset, want, flag_extra=0):
     names, seqs = T.read_fasta(fasta)
     got, st = T.gaf_with_engine(lib, gfa, names, seqs, preset, flag_extra=flag_extra)
     assert got == want, first_diff(got, want)
+    return st
+
+
+def check_gaf_lines(lib, gfa, fasta, preset, want):
+    """the GAF text against a golden file that keeps one 64-bit BLAKE2b digest (hex) per line instead of the line"""
+    import hashlib
+    names, seqs = T.read_fasta(fasta)
+    got, st = T.gaf_with_engine(lib, gfa, names, seqs, preset)
+    lines = got.split(b"\n")
+    assert lines[-1] == b"", "GAF text does not end with a newline"
+    assert len(lines) - 1 == len(want), "line count %d != %d" % (len(lines) - 1, len(want))
+    for i, (ln, w) in enumerate(zip(lines, want)):
+        assert hashlib.blake2b(ln, digest_size=8).hexdigest().encode() == w, "line %d differs from the reference's: %r" % (i, ln[:200])
     return st
 
 
@@ -101,10 +112,9 @@ def case_edge(lib, workdir):
     assert got[0] is None                      # qlen == 0 -> no result object
     for r in got[1:4]:
         assert r is not None and r["n_gc"] == 0
-    if T.have_ref():
-        want, _ = T.map_with_ref(gfa, names, seqs, "lr")
-        for i, (a, b) in enumerate(zip(want, got)):
-            assert T.diff_results(a, b) is None, (i, T.diff_results(a, b))
+    want, _ = T.map_with_ref(gfa, names, seqs, "lr")
+    for i, (a, b) in enumerate(zip(want, got)):
+        assert T.diff_results(a, b) is None, (i, T.diff_results(a, b))
 
 
 def case_struct_random(lib, workdir, n_reads=150, seed=23):
@@ -122,37 +132,11 @@ def case_struct_random(lib, workdir, n_reads=150, seed=23):
     return st
 
 
-_mwf = None
-
-
-def _mwf_types():
-    """ctypes view of miniwfa.h:36-51 (mwf_opt_t, mwf_rst_t) and the prototypes of the reference functions used as the checker"""
-    global _mwf
-    if _mwf is None:
-        import ctypes as C
-        ref = T.load_ref()
-
-        class mwf_opt_t(C.Structure):
-            _fields_ = [("flag", C.c_int32), ("x", C.c_int32), ("o1", C.c_int32), ("e1", C.c_int32), ("o2", C.c_int32), ("e2", C.c_int32),
-                        ("step", C.c_int32), ("max_s", C.c_int32), ("max_iter", C.c_int64), ("max_occ", C.c_int32), ("kmer", C.c_int32), ("min_len", C.c_int32)]
-
-        class mwf_rst_t(C.Structure):
-            _fields_ = [("s", C.c_int32), ("n_cigar", C.c_int32), ("n_iter", C.c_int64), ("cigar", C.POINTER(C.c_uint32))]
-        for f in (ref.mwf_wfa_exact, ref.mwf_wfa_chain):
-            f.restype = None
-            f.argtypes = [C.c_void_p, C.POINTER(mwf_opt_t), C.c_int32, C.c_char_p, C.c_int32, C.c_char_p, C.POINTER(mwf_rst_t)]
-        ref.mwf_opt_init.argtypes = [C.POINTER(mwf_opt_t)]
-        _mwf = (mwf_opt_t, mwf_rst_t)
-    return _mwf
-
-
 def case_wfa_fallback(lib, n_cases=12, seed=5):
     """gaps whose exact WFA exceeds the cell cap take the reference's chaining heuristic + low-memory checkpoints
     (miniwfa.c:551-601,776-834): same CIGAR and score as mwf_wfa_exact(max_iter) -> mwf_wfa_chain(step) of the reference"""
     import ctypes as C
     import random
-    ref = T.load_ref()
-    mwf_opt_t, mwf_rst_t = _mwf_types()
     rng = random.Random(seed)
 
     def mutate(s, rate):
@@ -182,24 +166,15 @@ def case_wfa_fallback(lib, n_cases=12, seed=5):
         max_iter, step = rng.choice([(2000, 40), (20000, 25), (50000, 100), (10 ** 8, 5000)])
         if it == 0:
             max_iter, step = 10 ** 8, 5000
-        opt = mwf_opt_t()
-        ref.mwf_opt_init(C.byref(opt))
-        opt.flag |= 1
-        opt.step, opt.max_iter = 0, max_iter
-        rst = mwf_rst_t()
-        ref.mwf_wfa_exact(None, C.byref(opt), len(ts), ts, len(qs), qs, C.byref(rst))
-        if rst.s < 0:
-            n_fallback += 1
-            opt.step, opt.max_iter = step, -1
-            ref.mwf_wfa_chain(None, C.byref(opt), len(ts), ts, len(qs), qs, C.byref(rst))
-        want = [rst.cigar[i] for i in range(rst.n_cigar)]
+        gave_up, want_s, want = T.ref_wfa(ts, qs, max_iter, step)
+        n_fallback += gave_up
         cap = len(ts) + len(qs) + 8
         buf = (C.c_uint32 * cap)()
         score = C.c_int(0)
         nc = lib.mgb_test_wfa(ts, len(ts), qs, len(qs), max_iter, step, buf, cap, C.byref(score))
         assert nc >= 0, (it, nc)
         got = [buf[i] for i in range(nc)]
-        assert got == want and score.value == rst.s, "case %d (tl=%d ql=%d max_iter=%d step=%d): score %d vs %d" % (it, len(ts), len(qs), max_iter, step, score.value, rst.s)
+        assert got == want and score.value == want_s, "case %d (tl=%d ql=%d max_iter=%d step=%d): score %d vs %d" % (it, len(ts), len(qs), max_iter, step, score.value, want_s)
     assert n_fallback >= 3
 
 
@@ -261,11 +236,12 @@ def case_full_size(lib, workdir, n_reads=10000, n_sub=300, n_ref=100, seed=11):
     lib.mgb_free_batch(m, gcs2)
     lib.mg_idx_destroy(gi)
     lib.mgb_gfa_destroy(g)
-    if T.have_ref() and n_ref > 0:
+    if n_ref > 0:
         pick = sub[:n_ref]
         want, _ = T.map_with_ref(gfa, [names[i] for i in pick], [seqs[i] for i in pick], "lr")
         for i, w in zip(pick, want):
-            check_cigar_invariants(w, len(seqs[i]))  # the invariants are the reference's, not ours
+            if not isinstance(w, T.Digest):  # a stored result is known by its digest only
+                check_cigar_invariants(w, len(seqs[i]))  # the invariants are the reference's, not ours
             d = T.diff_results(full[i], w)
             assert d is None, "read %d vs reference: %s" % (i, d)
 
@@ -275,8 +251,6 @@ def case_wfa_divergent(lib, n_cases=24, seed=5):
     (miniwfa.c:144-171) -- what the tier-3 ring has to get right when slots are reused by narrower wavefronts"""
     import ctypes as C
     import random
-    ref = T.load_ref()
-    mwf_opt_t, mwf_rst_t = _mwf_types()
     rng = random.Random(seed)
     for it in range(n_cases):
         tl = rng.choice([150, 300, 500, 800])
@@ -287,19 +261,13 @@ def case_wfa_divergent(lib, n_cases=24, seed=5):
             core = "".join(rng.choice("ACGT") for _ in range(100))
             t, q = t[:tl // 2] + core + t[tl // 2:], q[:ql // 3] + core + q[ql // 3:]
         ts, qs = t.encode(), q.encode()
-        opt = mwf_opt_t()
-        ref.mwf_opt_init(C.byref(opt))
-        opt.flag |= 1
-        opt.step, opt.max_iter = 0, 10 ** 8
-        rst = mwf_rst_t()
-        ref.mwf_wfa_exact(None, C.byref(opt), len(ts), ts, len(qs), qs, C.byref(rst))
-        assert rst.s >= 0
-        want = [rst.cigar[i] for i in range(rst.n_cigar)]
+        _, want_s, want = T.ref_wfa(ts, qs, 10 ** 8)
+        assert want_s >= 0
         cap = len(ts) + len(qs) + 8
         buf = (C.c_uint32 * cap)()
         score = C.c_int(0)
         nc = lib.mgb_test_wfa(ts, len(ts), qs, len(qs), 10 ** 8, 5000, buf, cap, C.byref(score))
-        assert nc >= 0 and [buf[i] for i in range(nc)] == want and score.value == rst.s, (it, tl, ql, score.value, rst.s)
+        assert nc >= 0 and [buf[i] for i in range(nc)] == want and score.value == want_s, (it, tl, ql, score.value, want_s)
 
 
 def case_wfa_band_shrinks(lib, n_cases=48, seed=99):
@@ -308,8 +276,6 @@ def case_wfa_band_shrinks(lib, n_cases=48, seed=99):
     last 17 wavefronts comes from the last-good-score slice.  Same CIGAR and score as the reference's mwf_wfa_exact()."""
     import ctypes as C
     import random
-    ref = T.load_ref()
-    mwf_opt_t, mwf_rst_t = _mwf_types()
     rng = random.Random(seed)
     n_shrunk = 0
     for it in range(n_cases):
@@ -335,20 +301,14 @@ def case_wfa_band_shrinks(lib, n_cases=48, seed=99):
         if not q:
             continue
         ts, qs = t.encode(), q.encode()
-        opt = mwf_opt_t()
-        ref.mwf_opt_init(C.byref(opt))
-        opt.flag |= 1
-        opt.step, opt.max_iter = 0, 10 ** 8
-        rst = mwf_rst_t()
-        ref.mwf_wfa_exact(None, C.byref(opt), len(ts), ts, len(qs), qs, C.byref(rst))
-        assert rst.s >= 0
-        n_shrunk += rst.s >= 256
-        want = [rst.cigar[i] for i in range(rst.n_cigar)]
+        _, want_s, want = T.ref_wfa(ts, qs, 10 ** 8)
+        assert want_s >= 0
+        n_shrunk += want_s >= 256
         cap = len(ts) + len(qs) + 8
         buf = (C.c_uint32 * cap)()
         score = C.c_int(0)
         nc = lib.mgb_test_wfa(ts, len(ts), qs, len(qs), 10 ** 8, 5000, buf, cap, C.byref(score))
-        assert nc >= 0 and [buf[i] for i in range(nc)] == want and score.value == rst.s, (it, len(ts), len(qs), score.value, rst.s, nc)
+        assert nc >= 0 and [buf[i] for i in range(nc)] == want and score.value == want_s, (it, len(ts), len(qs), score.value, want_s, nc)
     assert n_shrunk >= n_cases // 2
 
 
@@ -359,9 +319,6 @@ def case_radix_exact(lib, n_cases=60, seed=17):
     import ctypes as C
     import random
     from minigraph_b200 import capi
-    ref = T.load_ref()
-    ref.radix_sort_128x.restype = None
-    ref.radix_sort_128x.argtypes = [C.POINTER(capi.mg128_t), C.POINTER(capi.mg128_t)]
     lib.mgb_test_radix128.restype = C.c_int
     lib.mgb_test_radix128.argtypes = [C.POINTER(capi.mg128_t), C.c_int64, C.c_int, C.c_int]
     rng = random.Random(seed)
@@ -374,19 +331,20 @@ def case_radix_exact(lib, n_cases=60, seed=17):
             keys = [base + ((rng.randrange(nk) << sh) if rng.random() < 0.1 else (3 << sh)) for _ in range(n)]
         else:
             keys = [base + (rng.randrange(nk) << sh) for _ in range(n)]
-        want = (capi.mg128_t * n)()
-        for i, x in enumerate(keys):
-            want[i].x, want[i].y = x, i
-        ref.radix_sort_128x(want, C.cast(C.byref(want, C.sizeof(want)), C.POINTER(capi.mg128_t)))
+        want = T.ref_radix_sort([(x, i) for i, x in enumerate(keys)])
         for walk, hot in ((0, 0), (1, 0), (1, 16384), (1, n // 4 + 3400), (0, 16384)):  # (n/4 + 3400: what the callers ask of the on-chip slice; the digits then go to the arena)
             got = (capi.mg128_t * n)()
             for i, x in enumerate(keys):
                 got[i].x, got[i].y = x, i
             rc = lib.mgb_test_radix128(got, n, walk, hot)
             assert rc == 0, (it, n, walk, hot, rc)
-            bad = next((i for i in range(n) if got[i].y != want[i].y or got[i].x != want[i].x), None)
+            gl = [(got[i].x, got[i].y) for i in range(n)]
+            if isinstance(want, T.Digest):
+                assert gl == want, "case %d (n=%d, %d keys << %d, walk=%d, hot=%d): not the reference's order" % (it, n, nk, sh, walk, hot)
+                continue
+            bad = next((i for i in range(n) if gl[i] != want[i]), None)
             assert bad is None, "case %d (n=%d, %d keys << %d, walk=%d, hot=%d): position %d holds element %d, the reference has %d" % (
-                it, n, nk, sh, walk, hot, bad, got[bad].y, want[bad].y)
+                it, n, nk, sh, walk, hot, bad, gl[bad][1], want[bad][1])
 
 
 def case_wfa_tiers(lib, workdir, n_struct=60):
@@ -399,13 +357,12 @@ def case_wfa_tiers(lib, workdir, n_struct=60):
         prof = {n: st.prof[i] for i, n in enumerate(capi.PROF_NAMES)}
         assert prof["wfa_fast_n"] > 500, prof
         assert fn is case_c4 or prof["wfa_mid_n"] > 500, prof
-    if T.have_ref():
-        case_struct_random(lib, workdir, n_reads=n_struct, seed=37)
-        case_tier_routing(lib, workdir)
-        case_short_reads(lib, workdir, n_pairs=20)  # sr preset: tier 1 only, two-segment fragments
-        case_wfa_fallback(lib)  # tier 3 against miniwfa: scores far past 256 (band re-centring), capped runs, a gap beyond the 16-bit ring
-        case_wfa_divergent(lib)
-        case_wfa_band_shrinks(lib)
+    case_struct_random(lib, workdir, n_reads=n_struct, seed=37)
+    case_tier_routing(lib, workdir)
+    case_short_reads(lib, workdir, n_pairs=20)  # sr preset: tier 1 only, two-segment fragments
+    case_wfa_fallback(lib)  # tier 3 against miniwfa: scores far past 256 (band re-centring), capped runs, a gap beyond the 16-bit ring
+    case_wfa_divergent(lib)
+    case_wfa_band_shrinks(lib)
 
 
 def case_gchain_labels(lib, workdir, n_reads=150, graph_len=1000000):
@@ -552,33 +509,42 @@ def case_index_big(lib, workdir, graph_len=50000000, n_probe=40000):
     with open(pre + ".gfa", "a") as f:
         for i, t in enumerate(dup):
             f.write("\t".join([t[0], "dup%d" % i] + t[2:]))
-    ref = T.load_ref()
-    rg = ref.gfa_read((pre + ".gfa").encode())
-    io, rmo = options.opt_set("lr")
-    rgi = ref.mg_index(rg, C.byref(io), 8, C.byref(rmo))
-    assert rgi
-    ref.mg_idx_get.restype = C.POINTER(C.c_uint64)
-    # probes: the minimizers of random stretches of the graph (through the reference's own sketch), plus random keys
-    ref.mg_sketch.restype = None
-    ref.mg_sketch.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_void_p]
-
-    class V(C.Structure):
-        _fields_ = [("n", C.c_size_t), ("m", C.c_size_t), ("a", C.POINTER(capi_u128))]
+    # probes: the minimizers of random stretches of the graph (through the oracle's sketch, which is the reference's: test_oracle.py),
+    # plus random keys
+    orc = T.load_oracle()
+    io, _ = options.opt_set("lr")
+    g = lib.mgb_gfa_read((pre + ".gfa").encode())
     rnd = random.Random(5)
     keys = set()
-    n_seg = rg.contents.n_seg
+    n_seg = g.contents.n_seg
     while len(keys) < n_probe:
-        seg = rg.contents.seg[rnd.randrange(n_seg) if len(keys) % 4 else n_seg - 1 - rnd.randrange(60)]
+        seg = g.contents.seg[rnd.randrange(n_seg) if len(keys) % 4 else n_seg - 1 - rnd.randrange(60)]
         if seg.len < 200:
             continue
         st = rnd.randrange(seg.len - 199)
-        v = V(0, 0, None)
-        ref.mg_sketch(None, C.string_at(C.addressof(seg.seq.contents) + st, 200) if False else C.string_at(seg.seq, seg.len)[st:st + 200], 200, io.w, io.k, 0, C.byref(v))
-        for i in range(v.n):
-            keys.add(v.a[i].x >> 8)
-        C.CDLL(None).free(v.a)
+        for x, _ in T.orc_sketch(orc, C.string_at(seg.seq, seg.len)[st:st + 200], io.w, io.k, 0):
+            keys.add(x >> 8)
+    lib.mgb_gfa_destroy(g)
     keys = sorted(keys) + [rnd.getrandbits(2 * io.k) for _ in range(2000)]
-    n1, n2 = C.c_int(0), C.c_int(0)
+
+    def compute():
+        ref = T.load_ref()
+        rg = ref.gfa_read((pre + ".gfa").encode())
+        io_r, rmo = options.opt_set("lr")
+        rgi = ref.mg_index(rg, C.byref(io_r), 8, C.byref(rmo))
+        assert rgi
+        n1 = C.c_int(0)
+        lists = []
+        for k in keys:
+            a = ref.mg_idx_get(rgi, k, C.byref(n1))
+            lists.append([a[i] for i in range(n1.value)])
+        ref.mg_idx_destroy(rgi)
+        ref.gfa_destroy(rg)
+        return [rmo.occ_max1, rmo.lc_max_occ, rmo.bw_long], lists, sum(len(x) > 1 for x in lists)
+    want_mo, want, n_multi = T.reference("mg_idx_get", (T.file_digest(pre + ".gfa"), bytes(io), T.digest(keys)), compute,
+                                         lambda v: [v[0], T.digest(v[1]), v[2]], lambda s: (s[0], T.Digest(s[1]), s[2]))
+    assert n_multi > 100, n_multi
+    n2 = C.c_int(0)
     for index_dev in (1, 0):
         assert lib.mgb_set_param(b"index_dev", index_dev) == 0
         try:
@@ -586,20 +552,19 @@ def case_index_big(lib, workdir, graph_len=50000000, n_probe=40000):
             io2, mo = options.opt_set("lr")
             gi = lib.mg_index(g, C.byref(io2), 1, C.byref(mo))
             assert gi, lib.mgb_last_error()
-            assert (mo.occ_max1, mo.lc_max_occ, mo.bw_long) == (rmo.occ_max1, rmo.lc_max_occ, rmo.bw_long)
-            n_multi = 0
+            assert [mo.occ_max1, mo.lc_max_occ, mo.bw_long] == want_mo
+            got = []
             for k in keys:
-                a, b = ref.mg_idx_get(rgi, k, C.byref(n1)), lib.mg_idx_get(gi, k, C.byref(n2))
-                assert n1.value == n2.value, (hex(k), n1.value, n2.value)
-                assert [a[i] for i in range(n1.value)] == [b[i] for i in range(n2.value)], hex(k)
-                n_multi += n1.value > 1
-            assert n_multi > 100, n_multi
+                b = lib.mg_idx_get(gi, k, C.byref(n2))
+                got.append([b[i] for i in range(n2.value)])
+            if isinstance(want, T.Digest):
+                assert got == want, "index_dev=%d: the occurrence lists of the probed keys are not the reference's" % index_dev
+            for k, x, y in zip(keys, got, [] if isinstance(want, T.Digest) else want):
+                assert x == y, (hex(k), len(x), len(y))
             lib.mg_idx_destroy(gi)
             lib.mgb_gfa_destroy(g)
         finally:
             lib.mgb_set_param(b"index_dev", 1)
-    ref.mg_idx_destroy(rgi)
-    ref.gfa_destroy(rg)
 
 
 def case_multi_device(lib, workdir, devices="0,0,0", n_reads=100):
@@ -687,48 +652,54 @@ def case_multi_segment(lib, workdir, n_frag=40):
     fields as the reference (map-algo.c:34-45,356-360,402,407,464,475)"""
     import ctypes as C
     import random
-    from minigraph_b200 import capi, options
-    ref = T.load_ref()
+    from minigraph_b200 import options
     hap, reads = os.path.join(workdir, "mt.hap.fa"), os.path.join(workdir, "mt.seg.fa")
     T.sim_mt_haps(hap)
     T.sim_reads(hap, reads, n_frag, 9000, "ont", 53)
     names, seqs = T.read_fasta(reads)
     rng = random.Random(7)
-    gfa = os.path.join(T.FIX, "MT.gfa")
-    io, mo = options.opt_set("lr", True)
-    g_e = lib.mgb_gfa_read(gfa.encode())
-    gi_e = lib.mg_index(g_e, C.byref(io), 1, C.byref(mo))
-    assert gi_e, lib.mgb_last_error()
-    io_r, mo_r = options.opt_set("lr", True)
-    g_r = ref.gfa_read(gfa.encode())
-    gi_r = ref.mg_index(g_r, C.byref(io_r), 1, C.byref(mo_r))
-    b_r, b_e = ref.mg_tbuf_init(), lib.mg_tbuf_init()
-    for f in (lib.mg_map_frag, ref.mg_map_frag):
-        f.restype = None
-        f.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_char_p), C.POINTER(C.POINTER(capi.mg_gchains_t)), C.c_void_p, C.c_void_p, C.c_char_p]
-    n_mapped = 0
+    frags = []
     for nm, s in zip(names, seqs):
         n_seg = rng.choice([2, 2, 3])
         cut = sorted(rng.sample(range(1500, len(s) - 1500), n_seg - 1))
         parts = [s[a:b] for a, b in zip([0] + cut, cut + [len(s)])]
         if rng.random() < 0.3:
             parts[-1] = parts[-1][:40]  # a segment too short to be sketched in chunks
-        ql = (C.c_int * n_seg)(*[len(x) for x in parts])
-        sq = (C.c_char_p * n_seg)(*parts)
-        res = []
-        for lb, gi, mo_x, tb in ((ref, gi_r, mo_r, b_r), (lib, gi_e, mo, b_e)):
-            gcs = (C.POINTER(capi.mg_gchains_t) * n_seg)()
-            lb.mg_map_frag(C.cast(gi, C.c_void_p), n_seg, ql, sq, gcs, tb, C.cast(C.pointer(mo_x), C.c_void_p), nm)
-            assert all(not gcs[i] for i in range(1, n_seg))
-            res.append(T.gchains_to_py(gcs[0]))
-            lb.mg_gchain_free(gcs[0])
-        d = T.diff_results(res[0], res[1])
+        frags.append((nm, parts))
+    gfa = os.path.join(T.FIX, "MT.gfa")
+    want = T.map_frag_with_ref(gfa, frags, "lr", True)
+    io, mo = options.opt_set("lr", True)
+    g = lib.mgb_gfa_read(gfa.encode())
+    gi = lib.mg_index(g, C.byref(io), 1, C.byref(mo))
+    assert gi, lib.mgb_last_error()
+    got = map_frags(lib, gi, mo, frags)
+    lib.mg_idx_destroy(gi)
+    n_mapped = 0
+    for (nm, parts), w, r in zip(frags, want, got):
+        d = T.diff_results(w, r)
         assert d is None, (nm, [len(x) for x in parts], d)
-        if res[0] and res[0]["n_gc"] > 0:
+        if w and w["n_gc"] > 0:
             n_mapped += 1
     assert n_mapped >= n_frag // 2
-    ref.mg_tbuf_destroy(b_r), lib.mg_tbuf_destroy(b_e)
-    lib.mg_idx_destroy(gi_e), ref.mg_idx_destroy(gi_r)
+
+
+def map_frags(lib, gi, mo, frags):
+    """mg_map_frag() of an engine library on every fragment (name, [segment sequences]), one call each"""
+    import ctypes as C
+    b = lib.mg_tbuf_init()
+    lib.mg_map_frag.restype = None
+    lib.mg_map_frag.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_char_p), C.POINTER(C.POINTER(capi.mg_gchains_t)), C.c_void_p, C.c_void_p, C.c_char_p]
+    res = []
+    for nm, parts in frags:
+        n_seg = len(parts)
+        gcs = (C.POINTER(capi.mg_gchains_t) * n_seg)()
+        lib.mg_map_frag(C.cast(gi, C.c_void_p), n_seg, (C.c_int * n_seg)(*[len(x) for x in parts]), (C.c_char_p * n_seg)(*parts), gcs, b,
+                        C.cast(C.pointer(mo), C.c_void_p), nm)
+        assert all(not gcs[i] for i in range(1, n_seg))
+        res.append(T.gchains_to_py(gcs[0]))
+        lib.mg_gchain_free(gcs[0])
+    lib.mg_tbuf_destroy(b)
+    return res
 
 
 def case_short_reads(lib, workdir, n_pairs=60):
@@ -737,7 +708,6 @@ def case_short_reads(lib, workdir, n_pairs=60):
     import ctypes as C
     import random
     from minigraph_b200 import capi, options
-    ref = T.load_ref()
     hap, reads = os.path.join(workdir, "mt.hap.fa"), os.path.join(workdir, "mt.sr.fa")
     T.sim_mt_haps(hap)
     T.sim_reads(hap, reads, n_pairs, 500, "hifi", 61)
@@ -745,38 +715,24 @@ def case_short_reads(lib, workdir, n_pairs=60):
     comp = bytes.maketrans(b"ACGT", b"TGCA")
     rng = random.Random(3)
     gfa = os.path.join(T.FIX, "MT.gfa")
-    io, mo = options.opt_set("sr", False)
-    g_e = lib.mgb_gfa_read(gfa.encode())
-    gi_e = lib.mg_index(g_e, C.byref(io), 1, C.byref(mo))
-    assert gi_e, lib.mgb_last_error()
-    io_r, mo_r = options.opt_set("sr", False)
-    g_r = ref.gfa_read(gfa.encode())
-    gi_r = ref.mg_index(g_r, C.byref(io_r), 1, C.byref(mo_r))
-    b_r, b_e = ref.mg_tbuf_init(), lib.mg_tbuf_init()
-    for f in (lib.mg_map_frag, ref.mg_map_frag):
-        f.restype = None
-        f.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_char_p), C.POINTER(C.POINTER(capi.mg_gchains_t)), C.c_void_p, C.c_void_p, C.c_char_p]
-    n_mapped = 0
-    frags, per_frag = [], []
+    frags = []
     for nm, s in zip(names, seqs):
         if rng.random() < 0.7:  # a pair: 150 bases from each end, the mate reverse-complemented
             parts = [s[:150], s[-150:].translate(comp)[::-1]]
         else:
             parts = [s[:rng.choice([100, 150, 250])]]
         frags.append((nm, parts))
-        n_seg = len(parts)
-        ql = (C.c_int * n_seg)(*[len(x) for x in parts])
-        sq = (C.c_char_p * n_seg)(*parts)
-        res = []
-        for lb, gi, mo_x, tb in ((ref, gi_r, mo_r, b_r), (lib, gi_e, mo, b_e)):
-            gcs = (C.POINTER(capi.mg_gchains_t) * n_seg)()
-            lb.mg_map_frag(C.cast(gi, C.c_void_p), n_seg, ql, sq, gcs, tb, C.cast(C.pointer(mo_x), C.c_void_p), nm)
-            res.append(T.gchains_to_py(gcs[0]))
-            lb.mg_gchain_free(gcs[0])
-        d = T.diff_results(res[0], res[1])
+    want = T.map_frag_with_ref(gfa, frags, "sr", False)
+    io, mo = options.opt_set("sr", False)
+    g_e = lib.mgb_gfa_read(gfa.encode())
+    gi_e = lib.mg_index(g_e, C.byref(io), 1, C.byref(mo))
+    assert gi_e, lib.mgb_last_error()
+    got = map_frags(lib, gi_e, mo, frags)
+    n_mapped = 0
+    for (nm, parts), w, r in zip(frags, want, got):
+        d = T.diff_results(w, r)
         assert d is None, (nm, [len(x) for x in parts], d)
-        per_frag.append(res[0])
-        if res[0] and res[0]["n_gc"] > 0:
+        if w and w["n_gc"] > 0:
             n_mapped += 1
     assert n_mapped >= n_pairs // 2, n_mapped
     # the same fragments in one call of the batch entry point
@@ -791,12 +747,11 @@ def case_short_reads(lib, workdir, n_pairs=60):
     off = 0
     for f, (nm, parts) in enumerate(frags):
         assert all(not gcs[off + j] for j in range(1, len(parts)))
-        d = T.diff_results(per_frag[f], T.gchains_to_py(gcs[off]))
+        d = T.diff_results(want[f], T.gchains_to_py(gcs[off]))
         assert d is None, (nm, d)
         off += len(parts)
     lib.mgb_free_batch(n_tot, gcs)
-    ref.mg_tbuf_destroy(b_r), lib.mg_tbuf_destroy(b_e)
-    lib.mg_idx_destroy(gi_e), ref.mg_idx_destroy(gi_r)
+    lib.mg_idx_destroy(gi_e)
 
 
 def case_no_diag(lib, workdir):

@@ -1,5 +1,9 @@
-"""Shared helpers of the test-suite: oracle bindings, FASTA reader, deep comparison of mg_gchains_t objects."""
+"""Shared helpers of the test-suite: oracle bindings, FASTA reader, deep comparison of mg_gchains_t objects, and the
+stored results of the reference (tests/golden/reference_results.json) that stand in for it where it is not built."""
+import atexit
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -14,10 +18,91 @@ REF_SO = os.path.join(REPO, "oracle", "_ref", "libmgref.so")
 REF_BIN = os.path.join(REPO, "oracle", "_ref", "minigraph")
 HOSTSIM_SO = os.path.join(REPO, "tests", "hostsim", "libmgb_hostsim.so")
 MGSIM = os.path.join(REPO, "tools", "mgsim")
+REF_STORE = os.path.join(REPO, "tests", "golden", "reference_results.json")
 
 
 def have_ref():
     return os.path.exists(REF_SO) and os.path.exists(REF_BIN)
+
+
+def digest(obj):
+    """64-bit BLAKE2b of repr(obj): what the store keeps of a reference result (ints, bytes, floats, lists, dicts)"""
+    return hashlib.blake2b(repr(obj).encode(), digest_size=8).hexdigest()
+
+
+class Digest:
+    """A reference result known by its digest only (and, for a mapping result, its number of graph chains).
+    It equals any value whose digest it is, so `got == want` and diff_results() work on it as on the full value."""
+
+    def __init__(self, h, n_gc=None):
+        self.h, self.n_gc = h, n_gc
+
+    def __eq__(self, other):
+        return self.h == (other.h if isinstance(other, Digest) else digest(other))
+
+    def __ne__(self, other):
+        return not self == other
+
+    __hash__ = None
+
+    def __getitem__(self, k):
+        assert k == "n_gc", k
+        return self.n_gc
+
+    def __repr__(self):
+        return "<reference result %s>" % self.h
+
+
+_store, _recorded = None, {}
+
+
+def _record_to(path):
+    old = {}
+    if os.path.exists(path):
+        with open(path) as f:
+            old = json.load(f)
+    old.update(_recorded)
+    with open(path, "w") as f:  # one entry per line
+        f.write("{\n" + ",\n".join("%s: %s" % (json.dumps(k), json.dumps(old[k], separators=(",", ":"))) for k in sorted(old)) + "\n}\n")
+
+
+def reference(kind, inputs, compute, stored_form, from_stored):
+    """The reference's answer to `inputs`.  With oracle/_ref built: compute() on it (full value, for a detailed diff), checked
+    against the stored form when the store has one.  Without: from_stored(the stored form), digests in place of large values.
+    MGB_REF_RECORD=<file> adds the stored forms of every computed answer to that JSON file (regenerates the store)."""
+    global _store
+    if _store is None:
+        with open(REF_STORE) as f:
+            _store = json.load(f)
+    key = digest((kind,) + tuple(inputs))
+    if have_ref():
+        val = compute()
+        rec = json.loads(json.dumps(stored_form(val)))
+        assert key not in _store or _store[key] == rec, "%s: the stored reference result differs from the reference's" % kind
+        if os.environ.get("MGB_REF_RECORD"):
+            if not _recorded:
+                atexit.register(_record_to, os.environ["MGB_REF_RECORD"])
+            _recorded[key] = rec
+        return val
+    assert key in _store, "%s: no stored reference result for these inputs (regenerate with oracle/_ref built and MGB_REF_RECORD set)" % kind
+    return from_stored(_store[key])
+
+
+def file_digest(path):
+    h = hashlib.blake2b(digest_size=16)
+    with open(path, "rb") as f:
+        for blk in iter(lambda: f.read(1 << 20), b""):
+            h.update(blk)
+    return h.hexdigest()
+
+
+def result_form(r):
+    """stored form of one mapping result (gchains_to_py), and back"""
+    return None if r is None else [digest(r), r["n_gc"]]
+
+
+def result_from(s):
+    return None if s is None else Digest(s[0], s[1])
 
 
 _ref = None
@@ -36,6 +121,35 @@ def load_ref():
         C.c_int.in_dll(lib, "mg_verbose").value = 1
         _ref = lib
     return _ref
+
+
+_oracle = None
+
+
+def load_oracle():
+    """oracle/liboracle.so: the plain-C restatement of reference functions (oracle/mgoracle.c)"""
+    global _oracle
+    if _oracle is None:
+        subprocess.check_call(["make", "-s", "-C", os.path.join(REPO, "oracle"), "liboracle.so"])
+        lib = C.CDLL(os.path.join(REPO, "oracle", "liboracle.so"))
+        lib.orc_sketch.restype = C.c_int64
+        lib.orc_sketch.argtypes = [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_uint32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int64]
+        lib.orc_radix_sort_128x.restype = None
+        lib.orc_radix_sort_128x.argtypes = [C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int64]
+        lib.orc_hash_str.restype = C.c_uint32
+        lib.orc_hash_str.argtypes = [C.c_char_p]
+        lib.orc_chain_score.restype = C.c_int32
+        lib.orc_chain_score.argtypes = [C.c_uint64] * 4 + [C.c_int32] * 3 + [C.c_float] * 2
+        _oracle = lib
+    return _oracle
+
+
+def orc_sketch(orc, seq, w, k, rid):
+    cap = len(seq) + 16
+    x, y = (C.c_uint64 * cap)(), (C.c_uint64 * cap)()
+    n = orc.orc_sketch(seq, len(seq), w, k, rid, x, y, cap)
+    assert n <= cap
+    return [[x[i], y[i]] for i in range(n)]
 
 
 _hostsim = None
@@ -119,6 +233,8 @@ def diff_results(a, b):
     """Return a short description of the first difference, or None."""
     if a is None or b is None:
         return None if a is b else "one result is NULL"
+    if isinstance(a, Digest) or isinstance(b, Digest):
+        return None if a == b else "%r != %r" % (a if isinstance(a, Digest) else digest(a), b if isinstance(b, Digest) else digest(b))
     for k in ("n_gc", "n_lc", "n_a", "rep_len"):
         if a[k] != b[k]:
             return "%s: %r != %r" % (k, a[k], b[k])
@@ -137,24 +253,138 @@ def diff_results(a, b):
 
 def map_with_ref(gfa_path, names, seqs, preset="lr", cigar=True, tweak=None):
     """Run the reference's own mg_index/mg_map on every read (CPU).  tweak(mo) may change mapping options after the preset."""
-    ref = load_ref()
-    g = ref.gfa_read(gfa_path.encode())
-    assert g, "gfa_read failed"
     io, mo = options.opt_set(preset, cigar)
     if tweak:
         tweak(mo)
-    gi = ref.mg_index(g, C.byref(io), 1, C.byref(mo))
-    assert gi
-    b = ref.mg_tbuf_init()
-    res = []
-    for nm, s in zip(names, seqs):
-        p = ref.mg_map(gi, len(s), s, b, C.byref(mo), nm)
-        res.append(gchains_to_py(p))
-        ref.mg_gchain_free(p)
-    ref.mg_tbuf_destroy(b)
-    ref.mg_idx_destroy(gi)
-    ref.gfa_destroy(g)
-    return res, mo
+
+    def compute():
+        ref = load_ref()
+        g = ref.gfa_read(gfa_path.encode())
+        assert g, "gfa_read failed"
+        gi = ref.mg_index(g, C.byref(io), 1, C.byref(mo))
+        assert gi
+        b = ref.mg_tbuf_init()
+        res = []
+        for nm, s in zip(names, seqs):
+            p = ref.mg_map(gi, len(s), s, b, C.byref(mo), nm)
+            res.append(gchains_to_py(p))
+            ref.mg_gchain_free(p)
+        ref.mg_tbuf_destroy(b)
+        ref.mg_idx_destroy(gi)
+        ref.gfa_destroy(g)
+        return res, mo
+    return reference("mg_map", (file_digest(gfa_path), bytes(io), bytes(mo), digest(list(names)), digest(list(seqs))), compute,
+                     lambda v: {"mo": bytes(v[1]).hex(), "r": [result_form(r) for r in v[0]]},
+                     lambda s: ([result_from(r) for r in s["r"]], capi.mg_mapopt_t.from_buffer_copy(bytes.fromhex(s["mo"]))))
+
+
+def map_frag_with_ref(gfa_path, frags, preset="lr", cigar=True):
+    """The reference's mg_map_frag() on every fragment (name, [segment sequences]): the result of each fragment, which the
+    reference returns in its first segment's slot (the others stay NULL)."""
+    io, mo = options.opt_set(preset, cigar)
+
+    def compute():
+        ref = load_ref()
+        ref.mg_map_frag.restype = None
+        ref.mg_map_frag.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_char_p), C.POINTER(C.POINTER(capi.mg_gchains_t)),
+                                    C.c_void_p, C.c_void_p, C.c_char_p]
+        g = ref.gfa_read(gfa_path.encode())
+        assert g, "gfa_read failed"
+        gi = ref.mg_index(g, C.byref(io), 1, C.byref(mo))
+        assert gi
+        b = ref.mg_tbuf_init()
+        res = []
+        for nm, parts in frags:
+            n_seg = len(parts)
+            gcs = (C.POINTER(capi.mg_gchains_t) * n_seg)()
+            ref.mg_map_frag(C.cast(gi, C.c_void_p), n_seg, (C.c_int * n_seg)(*[len(x) for x in parts]), (C.c_char_p * n_seg)(*parts), gcs, b,
+                            C.cast(C.pointer(mo), C.c_void_p), nm)
+            assert all(not gcs[i] for i in range(1, n_seg))
+            res.append(gchains_to_py(gcs[0]))
+            ref.mg_gchain_free(gcs[0])
+        ref.mg_tbuf_destroy(b)
+        ref.mg_idx_destroy(gi)
+        ref.gfa_destroy(g)
+        return res
+    return reference("mg_map_frag", (file_digest(gfa_path), bytes(io), bytes(mo), digest(list(frags))), compute,
+                     lambda v: [result_form(r) for r in v], lambda s: [result_from(r) for r in s])
+
+
+def ref_wfa(ts, qs, max_iter, step=None):
+    """miniwfa of the reference: mwf_wfa_exact(max_iter); with `step`, mwf_wfa_chain(step) where the exact run gives up
+    (score < 0), in the order of mwf_wfa_auto (miniwfa.c:824-834).  Returns (exact run gave up, score, CIGAR)."""
+    def compute():
+        ref = load_ref()
+        mwf_opt_t, mwf_rst_t = _mwf_types()
+        opt = mwf_opt_t()
+        ref.mwf_opt_init(C.byref(opt))
+        opt.flag |= 1
+        opt.step, opt.max_iter = 0, max_iter
+        rst = mwf_rst_t()
+        ref.mwf_wfa_exact(None, C.byref(opt), len(ts), ts, len(qs), qs, C.byref(rst))
+        gave_up = rst.s < 0
+        if gave_up and step is not None:
+            opt.step, opt.max_iter = step, -1
+            ref.mwf_wfa_chain(None, C.byref(opt), len(ts), ts, len(qs), qs, C.byref(rst))
+        return gave_up, rst.s, [rst.cigar[i] for i in range(rst.n_cigar)]
+    return reference("mwf_wfa", (digest(ts), digest(qs), max_iter, step), compute, lambda v: [v[0], v[1], digest(v[2])],
+                     lambda s: (s[0], s[1], Digest(s[2])))
+
+
+_mwf = None
+
+
+def _mwf_types():
+    """ctypes view of miniwfa.h:36-51 (mwf_opt_t, mwf_rst_t) and the prototypes of the reference functions used as the checker"""
+    global _mwf
+    if _mwf is None:
+        ref = load_ref()
+
+        class mwf_opt_t(C.Structure):
+            _fields_ = [("flag", C.c_int32), ("x", C.c_int32), ("o1", C.c_int32), ("e1", C.c_int32), ("o2", C.c_int32), ("e2", C.c_int32),
+                        ("step", C.c_int32), ("max_s", C.c_int32), ("max_iter", C.c_int64), ("max_occ", C.c_int32), ("kmer", C.c_int32), ("min_len", C.c_int32)]
+
+        class mwf_rst_t(C.Structure):
+            _fields_ = [("s", C.c_int32), ("n_cigar", C.c_int32), ("n_iter", C.c_int64), ("cigar", C.POINTER(C.c_uint32))]
+        for f in (ref.mwf_wfa_exact, ref.mwf_wfa_chain):
+            f.restype = None
+            f.argtypes = [C.c_void_p, C.POINTER(mwf_opt_t), C.c_int32, C.c_char_p, C.c_int32, C.c_char_p, C.POINTER(mwf_rst_t)]
+        ref.mwf_opt_init.argtypes = [C.POINTER(mwf_opt_t)]
+        _mwf = (mwf_opt_t, mwf_rst_t)
+    return _mwf
+
+
+def ref_radix_sort(pairs):
+    """klib's radix_sort_128x() of the reference (ksort.h:112-162, not stable) on [(x, y), ...]: the sorted pairs"""
+    def compute():
+        ref = load_ref()
+        ref.radix_sort_128x.restype = None
+        ref.radix_sort_128x.argtypes = [C.POINTER(capi.mg128_t), C.POINTER(capi.mg128_t)]
+        n = len(pairs)
+        a = (capi.mg128_t * n)()
+        for i, (x, y) in enumerate(pairs):
+            a[i].x, a[i].y = x, y
+        ref.radix_sort_128x(a, C.cast(C.byref(a, C.sizeof(a)), C.POINTER(capi.mg128_t)))
+        return [(a[i].x, a[i].y) for i in range(n)]
+    return reference("radix_sort_128x", (digest(list(pairs)),), compute, digest, Digest)
+
+
+class mg128_v(C.Structure):
+    _fields_ = [("n", C.c_size_t), ("m", C.c_size_t), ("a", C.POINTER(capi.mg128_t))]
+
+
+def ref_sketch(seq, w, k, rid):
+    """mg_sketch() of the reference (sketch.c): the minimizers of `seq` as [[x, y], ...]"""
+    def compute():
+        ref = load_ref()
+        ref.mg_sketch.restype = None
+        ref.mg_sketch.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_uint32, C.POINTER(mg128_v)]
+        v = mg128_v()
+        ref.mg_sketch(None, seq, len(seq), w, k, rid, C.byref(v))
+        out = [[v.a[i].x, v.a[i].y] for i in range(v.n)]
+        C.CDLL(None).free(v.a)
+        return out
+    return reference("mg_sketch", (digest(seq), w, k, rid), compute, digest, Digest)
 
 
 def map_with_engine(lib, gfa_path, names, seqs, preset="lr", cigar=True, gfa_loader=None, tweak=None):

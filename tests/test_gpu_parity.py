@@ -1,4 +1,5 @@
-"""GPU parity tests: libmgb200.so (CUDA, sm_100a) through the C ABI against the golden GAF and oracle/_ref."""
+"""GPU parity tests: libmgb200.so (CUDA, sm_100a) through the C ABI against the golden GAF and the reference (oracle/_ref or its
+stored results)."""
 import os
 
 import pytest
@@ -40,17 +41,14 @@ def test_edge_reads(lib, workdir):
     cases.case_edge(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_multi_segment_fragments(lib, workdir):
     cases.case_multi_segment(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_short_read_preset(lib, workdir):
     cases.case_short_reads(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_no_diag_flag(lib, workdir):
     cases.case_no_diag(lib, workdir)
 
@@ -63,12 +61,10 @@ def test_engine_switches_keep_results(lib, workdir):
     cases.case_switches(lib, workdir, device=True)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not there")
 def test_upload_modes(lib, workdir):
     cases.case_upload_modes(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_index_of_a_50mb_graph(lib, workdir):
     cases.case_index_big(lib, workdir)
 
@@ -83,12 +79,10 @@ def test_concurrent_callers(lib, workdir):
     cases.case_concurrent_calls(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_small_max_lc_skip(lib, workdir):
     cases.case_chain_skip(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_struct_fields_vs_reference(lib, workdir):
     cases.case_struct_random(lib, workdir, n_reads=400)
 
@@ -111,7 +105,6 @@ def test_index_matches_oracle_sketch(lib):
 
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_graph_chaining_label_table(lib, workdir):
     cases.case_gchain_labels(lib, workdir, n_reads=600, graph_len=2000000)
 
@@ -120,7 +113,6 @@ def test_gap_alignment_tiers(lib, workdir):
     cases.case_wfa_tiers(lib, workdir, n_struct=150)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_wfa_iteration_cap_fallback(lib):
     cases.case_wfa_fallback(lib, n_cases=10)
     cases.case_wfa_divergent(lib)

@@ -3,7 +3,6 @@ two-summaries-per-block outer query of chain_rmq_fill_w; the same case runs in b
 import pytest
 
 import cases
-import mgtest as T
 from minigraph_b200 import capi
 
 pytestmark = pytest.mark.gpu
@@ -14,6 +13,5 @@ def lib():
     return capi.load_product()
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not shipped")
 def test_rmq_chaining_with_interleaved_diagonals(lib, workdir):
     cases.case_tandem_diagonals(lib, workdir, n_reads=200)

@@ -13,9 +13,6 @@ import pytest
 import cases
 import mgtest as T
 
-pytestmark = pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
-
-
 @pytest.fixture(scope="module")
 def lib():
     return T.load_hostsim32()

@@ -1,5 +1,5 @@
 """CPU-only parity tests: the device code compiled as a single-lane simulator (tests/hostsim) against the committed
-golden GAF of the unmodified reference, and against oracle/_ref when it is present. Exercises host logic (GFA loader,
+golden GAF of the unmodified reference, and against oracle/_ref or its stored results. Exercises host logic (GFA loader,
 index build, batch dispatcher, result assembly, GAF writer) and the control flow of every kernel stage."""
 import pytest
 
@@ -36,17 +36,14 @@ def test_edge_reads(lib, workdir):
     cases.case_edge(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_multi_segment_fragments(lib, workdir):
     cases.case_multi_segment(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_short_read_preset(lib, workdir):
     cases.case_short_reads(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_no_diag_flag(lib, workdir):
     cases.case_no_diag(lib, workdir)
 
@@ -59,12 +56,10 @@ def test_engine_switches_keep_results(lib, workdir):
     cases.case_switches(lib, workdir, device=False)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not there")
 def test_upload_modes(lib, workdir):
     cases.case_upload_modes(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_index_vs_reference_lists(lib, workdir):
     cases.case_index_big(lib, workdir, graph_len=2000000, n_probe=5000)
 
@@ -79,17 +74,14 @@ def test_concurrent_callers(lib, workdir):
     cases.case_concurrent_calls(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_small_max_lc_skip(lib, workdir):
     cases.case_chain_skip(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_struct_fields_vs_reference(lib, workdir):
     cases.case_struct_random(lib, workdir, n_reads=60)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_graph_chaining_label_table(lib, workdir):
     cases.case_gchain_labels(lib, workdir, n_reads=150)
 
@@ -98,14 +90,12 @@ def test_gap_alignment_tiers(lib, workdir):
     cases.case_wfa_tiers(lib, workdir)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_wfa_iteration_cap_fallback(lib):
     cases.case_wfa_fallback(lib)
     cases.case_wfa_divergent(lib)
     cases.case_wfa_band_shrinks(lib)
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_full_size_properties_small(lib, workdir):
     """the logic of the GPU suite's full-size test (tests/test_gpu_zz_full_size.py) at a size the simulator finishes"""
     cases.case_full_size(lib, workdir, n_reads=120, n_sub=40, n_ref=20)

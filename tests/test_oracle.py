@@ -1,5 +1,5 @@
 """Pins oracle/mgoracle.c (plain-C restatement) against the golden vectors generated from the unmodified reference,
-and, when oracle/_ref is present, against the reference library itself on fresh random inputs."""
+and against the reference library itself (or its stored results) on seeded random inputs."""
 import ctypes as C
 import json
 import os
@@ -15,25 +15,10 @@ GOLD = os.path.join(T.REPO, "tests", "golden", "vectors.json")
 
 @pytest.fixture(scope="module")
 def orc():
-    subprocess.check_call(["make", "-s", "-C", os.path.join(T.REPO, "oracle"), "liboracle.so"])
-    lib = C.CDLL(os.path.join(T.REPO, "oracle", "liboracle.so"))
-    lib.orc_sketch.restype = C.c_int64
-    lib.orc_sketch.argtypes = [C.c_char_p, C.c_int32, C.c_int32, C.c_int32, C.c_uint32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int64]
-    lib.orc_radix_sort_128x.restype = None
-    lib.orc_radix_sort_128x.argtypes = [C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int64]
-    lib.orc_hash_str.restype = C.c_uint32
-    lib.orc_hash_str.argtypes = [C.c_char_p]
-    lib.orc_chain_score.restype = C.c_int32
-    lib.orc_chain_score.argtypes = [C.c_uint64] * 4 + [C.c_int32] * 3 + [C.c_float] * 2
-    return lib
+    return T.load_oracle()
 
 
-def orc_sketch(orc, seq, w, k, rid):
-    cap = len(seq) + 16
-    x, y = (C.c_uint64 * cap)(), (C.c_uint64 * cap)()
-    n = orc.orc_sketch(seq, len(seq), w, k, rid, x, y, cap)
-    assert n <= cap
-    return [[x[i], y[i]] for i in range(n)]
+orc_sketch = T.orc_sketch
 
 
 def orc_sort(orc, arr):
@@ -58,37 +43,20 @@ def test_radix_sort_golden_tie_order(orc):
         assert ys == c["out_y"], "tie order differs from klib's unstable radix sort (n=%d)" % len(c["in"])
 
 
-@pytest.mark.skipif(not T.have_ref(), reason="oracle/_ref not built")
 def test_against_reference_random(orc):
-    ref = T.load_ref()
-
-    class mg128_v(C.Structure):
-        _fields_ = [("n", C.c_size_t), ("m", C.c_size_t), ("a", C.POINTER(T.capi.mg128_t))]
-    ref.mg_sketch.restype = None
-    ref.mg_sketch.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_int, C.c_int, C.c_uint32, C.POINTER(mg128_v)]
-    ref.radix_sort_128x.restype = None
-    ref.radix_sort_128x.argtypes = [C.POINTER(T.capi.mg128_t), C.POINTER(T.capi.mg128_t)]
     rng = random.Random(7)
     for it in range(60):
         n = rng.choice([30, 200, 1000, 5000])
         alpha = rng.choice(["ACGT", "ACGTN", "AC", "ACGTacgtnN"])
         s = "".join(rng.choice(alpha) for _ in range(n)).encode()
         w, k = rng.choice([(11, 17), (10, 19), (3, 7), (20, 28)])
-        v = mg128_v()
-        ref.mg_sketch(None, s, len(s), w, k, 5, C.byref(v))
-        want = [[v.a[i].x, v.a[i].y] for i in range(v.n)]
-        C.CDLL(None).free(v.a)
-        assert orc_sketch(orc, s, w, k, 5) == want, (it, w, k)
+        assert orc_sketch(orc, s, w, k, 5) == T.ref_sketch(s, w, k, 5), (it, w, k)
     for it in range(40):
         n = rng.choice([3, 64, 65, 500, 4000])
         nk = rng.choice([2, 10, 1000, 2 ** 50])
         arr = [[rng.randrange(nk) << rng.choice([0, 8, 33]), i] for i in range(n)]
-        a = (T.capi.mg128_t * n)()
-        for i, (x, y) in enumerate(arr):
-            a[i].x, a[i].y = x, y
-        ref.radix_sort_128x(a, C.cast(C.byref(a, C.sizeof(a)), C.POINTER(T.capi.mg128_t)))
-        _, ys = orc_sort(orc, arr)
-        assert ys == [a[i].y for i in range(n)], it
+        xs, ys = orc_sort(orc, arr)
+        assert list(zip(xs, ys)) == T.ref_radix_sort([tuple(a) for a in arr]), it
 
 
 def test_name_hash(orc):
