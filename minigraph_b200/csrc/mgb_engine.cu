@@ -40,9 +40,7 @@ static int64_t p_arena_mb = 6;        // per worker, first pass
 static int64_t p_arena_big_mb = 1024; // per worker, retry pass
 static int64_t p_workers_per_sm = 32;
 static int64_t p_device = 0;
-static int64_t p_block_warps = 4;
 static int64_t p_host_threads = 0; // 0: min(16, hardware threads)
-static int64_t p_thread_mask = 0;      // bit s set: stage s runs one item per thread instead of one per warp (experiments)
 static int64_t p_slots = 3;            // mg_map_batch calls that may run at once on one index (each on its own slot: stream, buffers, arenas)
 static int64_t p_slot_workers = 0;
 static int64_t p_tier_learn = 1;       // 0: every gap tries every tier (no routing)
@@ -51,15 +49,50 @@ static int64_t p_gpu_lock = 1;         // 0: the kernels of concurrent calls may
 static int64_t p_pack2 = 1;            // 0: reads are uploaded as ASCII (1 byte per base) instead of 2 bits per base
 static int64_t p_lab_cache = 1;        // 0: graph chaining searches its walks per read instead of keeping per-source labels in HBM (mgb_gclabel.cuh)
 
-// launch shape per stage: warps per block and blocks per SM wanted (tunable for experiments: "sw<stage>", "mb<stage>")
+// ---- the kernel stages, one row each ----
+// A stage's number is its key in mgb_set_param ("sw<N>", "mb<N>"), its slot in mgb_stats_t::t_kernel_ms (stages below 10) and what
+// the profiles call it.  Columns: kernel, stage, number; the kernel's __launch_bounds__ (threads per block, blocks per SM); the
+// launch shape (warps per block, blocks per SM wanted) until "sw<N>" / "mb<N>" lower it; shared memory per warp; how an item is
+// entered; items taken per ticket.  Entry: ENTER_WARP, all lanes of the warp run the item; ENTER_LANE0, lane 0 alone with the whole
+// arena of its warp; ENTER_THREAD, every thread runs its own item in 1/32 of the warp's arena (the hardware interleaves the 32
+// diverged lanes, so their memory latencies overlap).  k_wfa_mid is the one kernel launched in smaller blocks than it is compiled for.
 #ifndef MGB_BIG_MINB
 #define MGB_BIG_MINB 4 // blocks of k_wfa_big per SM (its register budget follows: 80 at 6, 96 at 5, 128 at 4)
 #endif
 #ifndef MGB_GWFA_MINB
 #define MGB_GWFA_MINB 4
 #endif
-static int STAGE_MINB[20] = { 8, 2, 8, 8, 5, 8, 7, MGB_BIG_MINB, MGB_GWFA_MINB, 4, 0, 0, 0, 0, 0, 0, 0, 8, 8, 2 }; // indexed by stage number (10-16 unused)
-static int STAGE_WARPS[20] = { 4, 7, 4, 4, 4, 4, 2, 4, 4, 4, 0, 0, 0, 0, 0, 0, 0, 4, 4, 6 }; // k_chain: 2 x 7 slices of 16 KB per SM, k_chain_rescue: 2 x 6 of 18 KB
+#define MGB_STAGES(X) \
+	X(k_seed,          ST_SEED,          0, (128, 8),             4, 8,             SKETCH_SMEM_BYTES,       ENTER_WARP,   1) /* K1-K3: sketch, index lookup, seed sort */ \
+	X(k_chain,         ST_CHAIN,         1, (224, 2),             7, 2,             CHAIN_SMEM_BYTES,        ENTER_WARP,   1) /* K4/K5: linear chaining on chip (seeds bulk-loaded into shared memory; 2 x 7 slices of 16 KB per SM) */ \
+	X(k_gchain,        ST_GCHAIN,        2, (128, 8),             4, 8,             0,                       ENTER_WARP,   1) /* K6: graph chaining DP + k-shortest walks, overlap resolution, bridging plan */ \
+	X(k_index_sketch,  ST_INDEX_SKETCH,  3, (128, 8),             4, 8,             0,                       ENTER_LANE0,  1) /* index build: sketch of graph segments */ \
+	X(k_wfa_small,     ST_WFA1,          4, (128, 5),             4, 5,             WfTier1::STRIDE,         ENTER_WARP,   4) /* K8a tier 1: small gaps, wavefronts + traceback bytes in shared memory */ \
+	X(k_finish,        ST_FINISH,        5, (128, 8),             4, 8,             0,                       ENTER_WARP,   1) /* K8b: CIGAR stitching, ds strings, result blobs */ \
+	X(k_wfa_mid,       ST_WFA2,          6, (128, 5),             2, 7,             WfTier2::STRIDE,         ENTER_WARP,   4) /* K8a tier 2: mid-size gaps, wavefronts in shared memory */ \
+	X(k_wfa_big,       ST_WFA3,          7, (128, MGB_BIG_MINB),  4, MGB_BIG_MINB,  0,                       ENTER_WARP,   1) /* K8a tier 3: anything else, wavefronts in the worker arena */ \
+	X(k_gwfa,          ST_GWFA,          8, (128, MGB_GWFA_MINB), 4, MGB_GWFA_MINB, GWFA_SMEM_ARENA,         ENTER_WARP,   1) /* K7a: bridging alignments (graph wavefront), one warp per bridge */ \
+	X(k_gchain_gen,    ST_GCHAIN_GEN,    9, (128, 4),             4, 4,             0,                       ENTER_WARP,   1) /* K7b: graph-chain materialisation, post filters, mapq, alignment plan */ \
+	X(k_gc_labels,     ST_LABELS,       17, (128, 8),             4, 8,             0,                       ENTER_THREAD, 1) /* reachability labels of new source vertices (mgb_gclabel.cuh) */ \
+	X(k_gc_labels_big, ST_LABELS_BIG,   18, (128, 8),             4, 8,             0,                       ENTER_LANE0,  1) /* the few sources whose search outgrew a thread's share of the arena */ \
+	X(k_chain_rescue,  ST_CHAIN_RESCUE, 19, (192, 2),             6, 2,             CHAIN_RESCUE_SMEM_BYTES, ENTER_WARP,   1) /* K5: long-join rescue (RMQ chaining) of the reads k_chain listed (2 x 6 slices of 18 KB) */
+enum StageEntry { ENTER_WARP, ENTER_LANE0, ENTER_THREAD };
+enum Stage {
+#define MGB_STAGE_ENUM(kern, st, num, ...) st = num,
+	MGB_STAGES(MGB_STAGE_ENUM)
+#undef MGB_STAGE_ENUM
+};
+struct StageShapes { int warps[20], minb[20]; }; // indexed by stage number
+static StageShapes default_shapes()
+{
+	StageShapes s = {};
+#define MGB_STAGE_SHAPE(kern, st, num, bounds, w, b, ...) s.warps[num] = (w), s.minb[num] = (b);
+	MGB_STAGES(MGB_STAGE_SHAPE)
+#undef MGB_STAGE_SHAPE
+	return s;
+}
+static StageShapes g_shape = default_shapes(); // the launch shape in use
+
 extern "C" const char *mgb_last_error(void) { return g_last_error.c_str(); }
 extern "C" const char *mgb_version(void) { return "mgb200-r1"; }
 extern "C" int mgb_set_param(const char *key, int64_t value)
@@ -68,9 +101,7 @@ extern "C" int mgb_set_param(const char *key, int64_t value)
 	else if (!strcmp(key, "arena_big_mb")) p_arena_big_mb = value;
 	else if (!strcmp(key, "workers_per_sm")) p_workers_per_sm = value;
 	else if (!strcmp(key, "device")) p_device = value;
-	else if (!strcmp(key, "block_warps")) p_block_warps = value;
 	else if (!strcmp(key, "host_threads")) p_host_threads = value;
-	else if (!strcmp(key, "thread_mask")) p_thread_mask = value;
 	else if (!strcmp(key, "slots")) p_slots = value;
 	else if (!strcmp(key, "slot_workers")) p_slot_workers = value;
 	else if (!strcmp(key, "lab_cache")) p_lab_cache = value;
@@ -78,8 +109,8 @@ extern "C" int mgb_set_param(const char *key, int64_t value)
 	else if (!strcmp(key, "gpu_lock")) p_gpu_lock = value;
 	else if (!strcmp(key, "index_dev")) p_index_dev = value;
 	else if (!strcmp(key, "tier_learn")) p_tier_learn = value;
-	else if (!strncmp(key, "sw", 2) && key[2] >= '0' && key[2] <= '9' && !key[3] && value >= 1 && value <= 4) STAGE_WARPS[key[2] - '0'] = (int)value;
-	else if (!strncmp(key, "mb", 2) && key[2] >= '0' && key[2] <= '9' && !key[3] && value >= 1 && value <= 32) STAGE_MINB[key[2] - '0'] = (int)value;
+	else if (!strncmp(key, "sw", 2) && key[2] >= '0' && key[2] <= '9' && !key[3] && value >= 1 && value <= 4) g_shape.warps[key[2] - '0'] = (int)value;
+	else if (!strncmp(key, "mb", 2) && key[2] >= '0' && key[2] <= '9' && !key[3] && value >= 1 && value <= 32) g_shape.minb[key[2] - '0'] = (int)value;
 	else return -1;
 	return 0;
 }
@@ -88,9 +119,17 @@ extern "C" int mgb_set_param(const char *key, int64_t value)
 // device memory shim
 // ---------------------------------------------------------------------------------------------------------------
 
+static double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
+// kernels launched by the calling thread (every launcher counts its own): mgb_stats_t::n_launches is the difference over a batch
+static thread_local int64_t t_launches = 0;
+
 #ifdef MGB_HOSTSIM
+typedef void *DevStream;
+typedef double DevEvent; // the host clock when it was recorded
 struct MgbError { int code; };
 static bool dev_ok(int dev = -1) { (void)dev; return true; }
+static void set_device(int dev) { (void)dev; }
+static void set_stream(DevStream s) { (void)s; }
 static void *dmalloc(size_t n) { void *p = malloc(n? n : 16); return p; }
 static void dfree(void *p) { free(p); }
 static void h2d(void *d, const void *h, size_t n) { if (n) memcpy(d, h, n); }
@@ -99,13 +138,21 @@ static void dzero(void *d, size_t n) { if (n) memset(d, 0, n); }
 static void d2d(void *d, const void *s, size_t n) { if (n) memcpy(d, s, n); }
 static void dfill(void *d, int v, size_t n) { if (n) memset(d, v, n); }
 static void dsync() {}
+static void h2d_async(void *d, const void *h, size_t n) { if (n) memcpy(d, h, n); }
+static void d2h_async(void *h, const void *d, size_t n) { if (n) memcpy(h, d, n); }
+static void ev_record(DevEvent &e) { e = now_ms(); }
+static void ev_wait(DevEvent e) { (void)e; }
+static double ev_elapsed_ms(DevEvent a, DevEvent b) { return b - a; }
 static int dev_sm_count() { return 2; }
 static size_t dev_free_mem() { return (size_t)8 << 30; }
+struct EvTimer { double t0 = 0, t1 = 0; void start() { t0 = now_ms(); } void stop() { t1 = now_ms(); } double ms() { return t1 - t0; } void clear() { t0 = t1 = 0; } };
 #else
 // A failed CUDA call (out of memory, a fault in a kernel) unwinds to the C entry point, which returns NULL / a negative code with
 // the reason in mgb_last_error(); the library never ends the host process on its own.
 struct MgbError { int code; };
 #define CUDA_OK(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { set_error(std::string(#call) + ": " + cudaGetErrorString(_e)); throw MgbError{MGB_E_INTERNAL}; } } while (0)
+typedef cudaStream_t DevStream;
+typedef cudaEvent_t DevEvent;
 // every host thread that drives a slot of the batch pipeline works on its own stream
 static thread_local cudaStream_t t_stream = 0;
 static bool dev_ok(int dev = -1)
@@ -115,6 +162,8 @@ static bool dev_ok(int dev = -1)
 	if (cudaSetDevice(dev >= 0? dev : (int)p_device) != cudaSuccess) return false;
 	return true;
 }
+static void set_device(int dev) { cudaSetDevice(dev); }
+static void set_stream(DevStream s) { t_stream = s; }
 static void *dmalloc(size_t n) { void *p = 0; CUDA_OK(cudaMalloc(&p, n? n : 16)); return p; }
 static void dfree(void *p) { if (p) cudaFree(p); }
 static void dsync() { CUDA_OK(cudaStreamSynchronize(t_stream)); }
@@ -123,9 +172,35 @@ static void d2h(void *h, const void *d, size_t n) { if (n) { CUDA_OK(cudaMemcpyA
 static void dzero(void *d, size_t n) { if (n) CUDA_OK(cudaMemsetAsync(d, 0, n, t_stream)); }
 static void d2d(void *d, const void *s, size_t n) { if (n) CUDA_OK(cudaMemcpyAsync(d, s, n, cudaMemcpyDeviceToDevice, t_stream)); }
 static void dfill(void *d, int v, size_t n) { if (n) CUDA_OK(cudaMemsetAsync(d, v, n, t_stream)); }
+static void h2d_async(void *d, const void *h, size_t n) { if (n) CUDA_OK(cudaMemcpyAsync(d, h, n, cudaMemcpyHostToDevice, t_stream)); }
+static void d2h_async(void *h, const void *d, size_t n) { if (n) CUDA_OK(cudaMemcpyAsync(h, d, n, cudaMemcpyDeviceToHost, t_stream)); }
+static void ev_record(DevEvent e) { CUDA_OK(cudaEventRecord(e, t_stream)); }
+static void ev_wait(DevEvent e) { CUDA_OK(cudaEventSynchronize(e)); }
+static double ev_elapsed_ms(DevEvent a, DevEvent b) { float t = 0; return cudaEventElapsedTime(&t, a, b) == cudaSuccess? t : 0; }
+struct EvTimer {
+	cudaEvent_t a, b; bool used;
+	EvTimer() : used(false) { cudaEventCreate(&a); cudaEventCreate(&b); }
+	~EvTimer() { cudaEventDestroy(a); cudaEventDestroy(b); }
+	void start() { cudaEventRecord(a, t_stream); used = true; }
+	void stop() { cudaEventRecord(b, t_stream); }
+	double ms() { if (!used) return 0; float t = 0; cudaEventSynchronize(b); cudaEventElapsedTime(&t, a, b); return t; }
+	void clear() { used = false; }
+};
 static int dev_sm_count() { static int v = 0; if (v == 0) { int d = 0; CUDA_OK(cudaGetDevice(&d)); CUDA_OK(cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, d)); } return v; } // (the devices of one box are alike)
 static size_t dev_free_mem() { size_t f = 0, t = 0; CUDA_OK(cudaMemGetInfo(&f, &t)); return f; }
 #endif
+
+// the timers of a batch's first pass
+struct SlotTimers {
+	EvTimer h2d, seed, chain, align, wfa, fin, d2h, lab, k[10]; // k: per kernel slot of mgb_stats_t::t_kernel_ms
+	void reset() { EvTimer *all[] = {&h2d, &seed, &chain, &align, &wfa, &fin, &d2h, &lab}; for (EvTimer *t : all) t->clear(); for (int i = 0; i < 10; ++i) k[i].clear(); }
+};
+// a timer around a scope; none: the scope is not timed
+struct Span {
+	EvTimer *t;
+	explicit Span(EvTimer *t_) : t(t_) { if (t) t->start(); }
+	~Span() { if (t) t->stop(); }
+};
 
 template<typename T> static T *dalloc_copy(const std::vector<T> &v)
 {
@@ -138,6 +213,8 @@ template<typename T> static T *dalloc_copy(const std::vector<T> &v)
 struct GrowBuf {
 	void *p; size_t cap; bool host;
 	GrowBuf(bool host_ = false) : p(0), cap(0), host(host_) {}
+	GrowBuf(const GrowBuf &) = delete;
+	~GrowBuf() { release(); }
 	void release()
 	{
 		if (p == 0) return;
@@ -163,12 +240,18 @@ struct GrowBuf {
 	}
 };
 
+static int n_host_threads() // "host_threads"; 0: min(16, hardware threads)
+{
+	const int nt = (int)p_host_threads;
+	if (nt > 0) return nt;
+	return std::min(16, std::max(1, (int)std::thread::hardware_concurrency()));
+}
+
 namespace {
 static mgb::HostPool g_host_pool; // packing, result assembly, index build (one caller at a time)
 template<typename F> void parallel_for(int64_t n, F fn)
 {
-	int nt = (int)p_host_threads;
-	if (nt <= 0) { nt = (int)std::thread::hardware_concurrency(); if (nt > 16) nt = 16; if (nt < 1) nt = 1; }
+	const int nt = n_host_threads();
 	if (n < 64 || nt == 1) { for (int64_t i = 0; i < n; ++i) fn(i); return; }
 	const std::function<void(int64_t)> f = fn;
 	g_host_pool.run(n, nt, f);
@@ -189,32 +272,34 @@ struct LaunchArgs {
 	uint64_t arena_bytes;
 	uint64_t *arena_peak;    // per worker
 	int64_t job_start;       // first job of this launch (stage 4)
-	int thread_mode;         // 1: one item per thread (stage_loop_thread)
 	// segment sketch (index build)
 	Pool *pool_mz; u128 *mz;
 };
 
-// stages: 0 seed (K1-K3), 1 chain (K4/K5), 2 graph chaining DP + bridge plan (K6), 8 bridging jobs (K7a), 9 graph-chain
-//         materialisation + alignment plan (K7b), 4/6/7 WFA jobs tier 1/2/3 (K8a), 5 finish: CIGAR stitching + ds + result
-//         blob (K8b), 3 segment sketch for the index, 17 reachability labels of the sources graph chaining asks for (one per thread)
-#define MGB_IS_WFA(STAGE) ((STAGE) == 4 || (STAGE) == 6 || (STAGE) == 7)
-#define MGB_IS_WARP(STAGE) (MGB_IS_WFA(STAGE) || (STAGE) == 8 || (STAGE) == 1 || (STAGE) == 2 || (STAGE) == 0 || (STAGE) == 5 || (STAGE) == 9 || (STAGE) == 19) // stages entered by all lanes of the warp
+// the columns of the stage table that the device code reads
+template<int STAGE> struct StageRow;
+#define MGB_STAGE_ROW(kern, st, num, bounds, warps, blocks, smem, entry, grab) \
+	template<> struct StageRow<st> { static constexpr int SMEM = smem, GRAB = grab; static constexpr StageEntry ENTRY = entry; };
+MGB_STAGES(MGB_STAGE_ROW)
+#undef MGB_STAGE_ROW
+
 template<int STAGE>
 MG_HD inline int run_stage(const LaunchArgs &L, int item, Arena &A, int lane, int32_t *smem)
 {
-	if (STAGE == 0) return stage_seed(L.c, item, A, lane, smem);
-	if (STAGE == 1) return stage_chain<0>(L.c, item, A, lane, smem);
-	if (STAGE == 19) return stage_chain<1>(L.c, L.c.rescue_list[item], A, lane, smem); // the reads k_chain listed
-	if (STAGE == 2) return stage_gchain(L.c, L.routs, item, A, lane);
-	if (STAGE == 17) return label_job(A, L.c.g, L.c.lab, item, 0);
-	if (STAGE == 18) return label_job(A, L.c.g, L.c.lab, item, 1); // lane 0 with the whole arena of its warp
-	if (STAGE == 5) return stage_finish(L.c, L.routs, item, A, lane);
-	if (STAGE == 8) return gwfa_job_run(A, L.c, L.job_start + item, lane, smem);
-	if (STAGE == 9) return stage_gchain_gen(L.c, L.routs, item, A, lane);
-	if (STAGE == 4) return wfa_job_run(A, L.c, L.job_start + item, lane, smem, 1);
-	if (STAGE == 6) return wfa_job_run(A, L.c, L.c.jobq[0][item], lane, smem, 2);
-	if (STAGE == 7) return wfa_job_run(A, L.c, L.c.jobq[1][item], lane, smem, 3);
-	if (STAGE == 3) { // sketch one graph segment for the index (reference: index.c:200-205)
+	switch (STAGE) {
+	case ST_SEED: return stage_seed(L.c, item, A, lane, smem);
+	case ST_CHAIN: return stage_chain<0>(L.c, item, A, lane, smem);
+	case ST_CHAIN_RESCUE: return stage_chain<1>(L.c, L.c.rescue_list[item], A, lane, smem); // the reads k_chain listed
+	case ST_GCHAIN: return stage_gchain(L.c, L.routs, item, A, lane);
+	case ST_LABELS: return label_job(A, L.c.g, L.c.lab, item, 0);
+	case ST_LABELS_BIG: return label_job(A, L.c.g, L.c.lab, item, 1);
+	case ST_FINISH: return stage_finish(L.c, L.routs, item, A, lane);
+	case ST_GWFA: return gwfa_job_run(A, L.c, L.job_start + item, lane, smem);
+	case ST_GCHAIN_GEN: return stage_gchain_gen(L.c, L.routs, item, A, lane);
+	case ST_WFA1: return wfa_job_run(A, L.c, L.job_start + item, lane, smem, 1);
+	case ST_WFA2: return wfa_job_run(A, L.c, L.c.jobq[0][item], lane, smem, 2);
+	case ST_WFA3: return wfa_job_run(A, L.c, L.c.jobq[1][item], lane, smem, 3);
+	case ST_INDEX_SKETCH: { // sketch one graph segment for the index (reference: index.c:200-205)
 		AVec<u128> mv;
 		avec_init(mv);
 		int32_t len = L.c.g.seg_len[item];
@@ -226,6 +311,7 @@ MG_HD inline int run_stage(const LaunchArgs &L, int item, Arena &A, int lane, in
 		for (int64_t i = 0; i < mv.n; ++i) dst[i] = mv.a[i];
 		return 0;
 	}
+	}
 	return MGB_E_INTERNAL;
 }
 
@@ -233,18 +319,25 @@ MG_HD inline int run_stage(const LaunchArgs &L, int item, Arena &A, int lane, in
 template<int STAGE>
 MG_HD inline void stage_fail(const LaunchArgs &L, int item, int rc)
 {
-	if (STAGE == 17 || STAGE == 18) return; // a source that could not be finished is searched again by the read that needs it
-	if (STAGE == 3) {
+	int rid = item; // the read the item belongs to
+	switch (STAGE) {
+	case ST_LABELS: case ST_LABELS_BIG: return; // a source that could not be finished is searched again by the read that needs it
+	case ST_INDEX_SKETCH:
 #if MGB_ON_DEVICE
 		atomicMin((int*)L.routs, rc);
 #else
 		if (rc < *(int*)L.routs) *(int*)L.routs = rc;
 #endif
 		return;
+	case ST_CHAIN_RESCUE: rid = L.c.rescue_list[item]; break;
+	case ST_GWFA: rid = L.c.gjobs[L.job_start + item].rid; break;
+	case ST_WFA1: rid = L.c.jobs[L.job_start + item].rid; break;
+	case ST_WFA2: rid = L.c.jobs[L.c.jobq[0][item]].rid; break;
+	case ST_WFA3: rid = L.c.jobs[L.c.jobq[1][item]].rid; break;
+	default: break;
 	}
-	int rid = STAGE == 8? L.c.gjobs[L.job_start + item].rid : STAGE == 4? L.c.jobs[L.job_start + item].rid : STAGE == 6? L.c.jobs[L.c.jobq[0][item]].rid : STAGE == 7? L.c.jobs[L.c.jobq[1][item]].rid : STAGE == 19? L.c.rescue_list[item] : item;
 	L.c.meta[rid].status = rc; // benign race between jobs of one read: any negative code triggers the redo
-	if (STAGE == 2 || MGB_IS_WARP(STAGE) || STAGE == 5 || STAGE == 9) L.routs[rid].status = rc;
+	L.routs[rid].status = rc;
 }
 
 #ifndef MGB_HOSTSIM
@@ -258,13 +351,13 @@ __device__ __forceinline__ void stage_loop(const LaunchArgs &L)
 	Arena A;
 	arena_init(A, L.arena_base + (uint64_t)worker * L.arena_bytes, L.arena_bytes);
 	extern __shared__ int4 dyn_smem[];
-	const int smem_stride = STAGE == 4? WfTier1::STRIDE : STAGE == 6? WfTier2::STRIDE : STAGE == 0? SKETCH_SMEM_BYTES : STAGE == 8? GWFA_SMEM_ARENA : STAGE == 1? CHAIN_SMEM_BYTES : STAGE == 19? CHAIN_RESCUE_SMEM_BYTES : 0;
+	const int smem_stride = StageRow<STAGE>::SMEM;
 	int32_t *smem = smem_stride? (int32_t*)((char*)dyn_smem + (size_t)(threadIdx.x >> 5) * smem_stride) : 0;
-	if (STAGE == 1 || STAGE == 19) chain_smem_init(smem, lane);
-	if ((STAGE == 4 || STAGE == 6) && lane == 0) { unsigned long long *ck = wfa_cig_chunk(smem, STAGE == 4? 1 : 2); ck[0] = ck[1] = 0; } // no slice of the CIGAR pool yet
+	if (STAGE == ST_CHAIN || STAGE == ST_CHAIN_RESCUE) chain_smem_init(smem, lane);
+	if ((STAGE == ST_WFA1 || STAGE == ST_WFA2) && lane == 0) { unsigned long long *ck = wfa_cig_chunk(smem, STAGE == ST_WFA1? 1 : 2); ck[0] = ck[1] = 0; } // no slice of the CIGAR pool yet
 	prof_block_begin();
 	const int n_work = L.n_work_dev? (int)*L.n_work_dev : L.n_work;
-	const int grab = STAGE == 4 || STAGE == 6? 4 : 1; // the short jobs of the on-chip WFA tiers are taken four at a time: one contended ticket per four jobs
+	const int grab = StageRow<STAGE>::GRAB; // the short jobs of the on-chip WFA tiers are taken four at a time: one contended ticket per four jobs
 	int next_item = 0, have = 0;
 	for (;;) {
 		if (have == 0) {
@@ -276,7 +369,7 @@ __device__ __forceinline__ void stage_loop(const LaunchArgs &L)
 		--have;
 		if (item >= n_work) break;
 		if (L.rid_list) item = L.rid_list[item];
-		if (MGB_IS_WARP(STAGE)) {
+		if (StageRow<STAGE>::ENTRY == ENTER_WARP) {
 			A.top = 0;
 			int rc = run_stage<STAGE>(L, item, A, lane, smem);
 			if (rc < 0 && lane == 0) stage_fail<STAGE>(L, item, rc);
@@ -291,8 +384,8 @@ __device__ __forceinline__ void stage_loop(const LaunchArgs &L)
 	prof_block_end(L.c.prof);
 }
 
-// Thread-per-item variant for the stages whose control flow is sequential: every THREAD pulls its own item and owns
-// 1/32 of the warp's arena.  The 32 lanes of a warp diverge completely, but the hardware interleaves the diverged
+// Thread-per-item variant (ENTER_THREAD) for the stages whose control flow is sequential: every THREAD pulls its own item
+// and owns 1/32 of the warp's arena.  The 32 lanes of a warp diverge completely, but the hardware interleaves the diverged
 // lanes, so 32x more items are in flight per warp and their memory latencies overlap.
 template<int STAGE>
 __device__ __forceinline__ void stage_loop_thread(const LaunchArgs &L)
@@ -316,36 +409,17 @@ __device__ __forceinline__ void stage_loop_thread(const LaunchArgs &L)
 	prof_block_end(L.c.prof);
 }
 
-// named entry points (one per stage, so that profiles read well); blocks of 4 warps, MINB blocks per SM wanted
-#define MGB_KERNEL_T(name, STAGE, THREADS, MINB) __global__ void __launch_bounds__(THREADS, MINB) name(LaunchArgs L) { if (!MGB_IS_WARP(STAGE) && L.thread_mode) stage_loop_thread<STAGE>(L); else stage_loop<STAGE>(L); } // (no thread-per-item copy of the warp-wide stages in the kernel)
-#define MGB_KERNEL(name, STAGE, MINB) MGB_KERNEL_T(name, STAGE, 128, MINB)
-MGB_KERNEL(k_seed, 0, 8)          // K1-K3: sketch, index lookup, seed sort
-MGB_KERNEL_T(k_chain, 1, 224, 2)         // K4/K5: linear chaining on chip (seeds bulk-loaded into shared memory)
-MGB_KERNEL_T(k_chain_rescue, 19, 192, 2) // K5: long-join rescue (RMQ chaining) of the reads k_chain listed
-MGB_KERNEL(k_gchain, 2, 8)        // K6: graph chaining DP + k-shortest walks, overlap resolution, bridging plan
-MGB_KERNEL(k_gwfa, 8, MGB_GWFA_MINB)          // K7a: bridging alignments (graph wavefront), one warp per bridge
-MGB_KERNEL(k_gchain_gen, 9, 4)    // K7b: graph-chain materialisation, post filters, mapq, alignment plan
-MGB_KERNEL(k_index_sketch, 3, 8)  // index build: sketch of graph segments
-MGB_KERNEL(k_wfa_small, 4, 5)     // K8a tier 1: small gaps, wavefronts + traceback bytes in shared memory
-MGB_KERNEL(k_wfa_mid, 6, 5)       // K8a tier 2: mid-size gaps, wavefronts in shared memory (blocks of 2 warps)
-MGB_KERNEL(k_wfa_big, 7, MGB_BIG_MINB) // K8a tier 3: anything else, wavefronts in the worker arena
-MGB_KERNEL(k_finish, 5, 8)        // K8b: CIGAR stitching, ds strings, result blobs
-MGB_KERNEL(k_gc_labels, 17, 8)    // reachability labels of new source vertices, one search per thread (mgb_gclabel.cuh)
-MGB_KERNEL(k_gc_labels_big, 18, 8) // the few sources whose search outgrew a thread's share of the arena: one per warp
-template<int STAGE> struct StageKernel;
-template<> struct StageKernel<0> { static void (*get())(LaunchArgs) { return k_seed; } };
-template<> struct StageKernel<1> { static void (*get())(LaunchArgs) { return k_chain; } };
-template<> struct StageKernel<2> { static void (*get())(LaunchArgs) { return k_gchain; } };
-template<> struct StageKernel<3> { static void (*get())(LaunchArgs) { return k_index_sketch; } };
-template<> struct StageKernel<4> { static void (*get())(LaunchArgs) { return k_wfa_small; } };
-template<> struct StageKernel<6> { static void (*get())(LaunchArgs) { return k_wfa_mid; } };
-template<> struct StageKernel<7> { static void (*get())(LaunchArgs) { return k_wfa_big; } };
-template<> struct StageKernel<8> { static void (*get())(LaunchArgs) { return k_gwfa; } };
-template<> struct StageKernel<9> { static void (*get())(LaunchArgs) { return k_gchain_gen; } };
-template<> struct StageKernel<5> { static void (*get())(LaunchArgs) { return k_finish; } };
-template<> struct StageKernel<19> { static void (*get())(LaunchArgs) { return k_chain_rescue; } };
-template<> struct StageKernel<17> { static void (*get())(LaunchArgs) { return k_gc_labels; } };
-template<> struct StageKernel<18> { static void (*get())(LaunchArgs) { return k_gc_labels_big; } };
+// One named kernel per stage (so that profiles read well), each running the one loop its entry needs.  The choice is a plain if
+// on a constant, not if constexpr: with the unused loop left out of the source, nvcc stops inlining chain_rmq_fill_seq into
+// k_chain_rescue, which then needs more registers and stack.
+typedef void (*StageFn)(LaunchArgs);
+template<int STAGE> static StageFn stage_kernel();
+#define MGB_STAGE_KERNEL(kern, st, num, bounds, ...) \
+	__global__ void __launch_bounds__ bounds kern(LaunchArgs L) \
+	{ if (StageRow<st>::ENTRY == ENTER_THREAD) stage_loop_thread<st>(L); else stage_loop<st>(L); } \
+	template<> StageFn stage_kernel<st>() { return kern; }
+MGB_STAGES(MGB_STAGE_KERNEL)
+#undef MGB_STAGE_KERNEL
 #endif
 
 // Longest-first order of a job list (a tail of a few long jobs otherwise decides the kernel time).  Jobs are binned by
@@ -357,12 +431,13 @@ MG_HD inline int order_bin(uint32_t key)
 	int b = (int)(lz * 4 + (lz >= 2? ((x >> (lz - 2)) & 3) : 0));
 	return 63 - (b > 63? 63 : b);
 }
-// kind 0: bridging jobs [job_start, job_start+n), key = query length; kind 1: alignment jobs listed in q[0..n), key = tl + ql;
-// kind 2: reads 0..n-1, key = number of linear chains
+// ORDER_BRIDGES: bridging jobs [job_start, job_start+n), key = query length; ORDER_GAPS: alignment jobs listed in q[0..n), key = tl + ql;
+// ORDER_READS: reads 0..n-1, key = number of linear chains
+enum { NO_ORDER = -1, ORDER_BRIDGES, ORDER_GAPS, ORDER_READS };
 MG_HD inline uint32_t order_key(const LaunchArgs &L, int kind, const int32_t *q, int i)
 {
-	if (kind == 0) return (uint32_t)L.c.gjobs[L.job_start + i].ql;
-	if (kind == 2) return (uint32_t)L.c.meta[i].n_lc; // reads by their number of linear chains (graph chaining is roughly quadratic in it)
+	if (kind == ORDER_BRIDGES) return (uint32_t)L.c.gjobs[L.job_start + i].ql;
+	if (kind == ORDER_READS) return (uint32_t)L.c.meta[i].n_lc; // reads by their number of linear chains (graph chaining is roughly quadratic in it)
 	const WfaJob &J = L.c.jobs[q[i]];
 	return (uint32_t)(J.tl + J.ql);
 }
@@ -381,8 +456,9 @@ __global__ void __launch_bounds__(1024) k_job_order(LaunchArgs L, int kind, cons
 	for (int i = tid; i < n; i += 1024) order[atomicAdd(&cnt[order_bin(order_key(L, kind, q, i))], 1u)] = i;
 }
 #endif
-static void make_job_order(const LaunchArgs &L, int kind, const int32_t *q, int n, int32_t *order, const unsigned int *n_dev = 0)
+static void make_job_order(const LaunchArgs &L, int kind, const int32_t *q, int n, int32_t *order, const unsigned int *n_dev)
 {
+	++t_launches;
 #ifndef MGB_HOSTSIM
 	k_job_order<<<1, 1024, 0, t_stream>>>(L, kind, q, n, n_dev, order);
 	CUDA_OK(cudaGetLastError());
@@ -448,6 +524,7 @@ __global__ void __launch_bounds__(256) k_out_pack(PackArgs P)
 #endif
 static void pack_results(const PackArgs &P)
 {
+	t_launches += 2;
 #ifndef MGB_HOSTSIM
 	k_out_scan<<<1, 1024, 0, t_stream>>>(P);
 	k_out_pack<<<dev_sm_count() * 8, 256, 0, t_stream>>>(P);
@@ -544,6 +621,16 @@ __global__ void __launch_bounds__(256) k_unpack(UnpackArgs U)
 	}
 }
 #endif
+static void unpack_reads(const UnpackArgs &U)
+{
+	++t_launches;
+#ifndef MGB_HOSTSIM
+	k_unpack<<<dev_sm_count() * 8, 256, 0, t_stream>>>(U);
+	CUDA_OK(cudaGetLastError());
+#else
+	for (int r = 0; r < U.n_reads; ++r) if (U.pk_off[r] != ~0ULL) for (int64_t wd = 0; wd * 32 < U.seq_len[r]; ++wd) unpack_word(U, r, wd);
+#endif
+}
 
 // ---- the few words the host needs between two kernels (pool fill levels, queue lengths) ----
 // They do not travel by cudaMemcpy: a copy of 16 bytes queues behind whatever another call in flight has put on the copy engines
@@ -575,8 +662,19 @@ MG_HD inline void job_counts(const Pool *pools, int i_gjobs, int i_jobs, unsigne
 #ifndef MGB_HOSTSIM
 __global__ void k_job_counts(const Pool *pools, int i_gjobs, int i_jobs, unsigned int gjobs_done, unsigned int jobs_done, unsigned int *cnt) { job_counts(pools, i_gjobs, i_jobs, gjobs_done, jobs_done, cnt); }
 #endif
+static void count_jobs(const Pool *pools, int i_gjobs, int i_jobs, unsigned int gjobs_done, unsigned int jobs_done, unsigned int *cnt)
+{
+	++t_launches;
+#ifndef MGB_HOSTSIM
+	k_job_counts<<<1, 1, 0, t_stream>>>(pools, i_gjobs, i_jobs, gjobs_done, jobs_done, cnt);
+	CUDA_OK(cudaGetLastError());
+#else
+	job_counts(pools, i_gjobs, i_jobs, gjobs_done, jobs_done, cnt);
+#endif
+}
 static void fetch_mail(const MailSrc &m, Mail *mail)
 {
+	++t_launches;
 #ifndef MGB_HOSTSIM
 	k_mail<<<1, 32, 0, t_stream>>>(m, mail);
 	CUDA_OK(cudaGetLastError());
@@ -597,25 +695,30 @@ struct Workers {
 	uint64_t arena_bytes;
 	char *arena;
 	uint64_t *peak;
+	void release() { dfree(arena), dfree(peak); memset(this, 0, sizeof(*this)); }
 };
 
 template<int STAGE>
-static void launch_stage(LaunchArgs &L, const Workers &W, int warps_override = 0)
+static void launch_stage(LaunchArgs &L, const Workers &W)
 {
 	L.arena_base = W.arena, L.arena_bytes = W.arena_bytes, L.arena_peak = W.peak;
 	dzero(L.c.next_read, sizeof(unsigned int)); // in stream order: no host round trip per launch
+	++t_launches;
 #ifdef MGB_HOSTSIM
+	constexpr StageEntry entry = StageRow<STAGE>::ENTRY;
 	Arena A;
-	arena_init(A, W.arena, STAGE == 17? (W.arena_bytes / 32) & ~(uint64_t)15 : W.arena_bytes); // one item per thread: a thread's share, as on the device
-	std::vector<int32_t> sim_smem(std::max<size_t>(std::max<size_t>(WfTier1::STRIDE, WfTier2::STRIDE), std::max<size_t>(std::max<size_t>(GWFA_SMEM_ARENA, CHAIN_RESCUE_SMEM_BYTES), SKETCH_SMEM_BYTES)) / 4);
-	if (STAGE == 1 || STAGE == 19) { mbar_init((uint64_t*)sim_smem.data(), 1); sim_smem[2] = 0; }
+	arena_init(A, W.arena, entry == ENTER_THREAD? (W.arena_bytes / 32) & ~(uint64_t)15 : W.arena_bytes); // one item per thread: a thread's share, as on the device
+#define MGB_STAGE_SMEM(kern, st, num, bounds, warps, blocks, smem, ...) , (int)(smem)
+	std::vector<int32_t> sim_smem(std::max({0 MGB_STAGES(MGB_STAGE_SMEM)}) / 4); // the largest of all stages
+#undef MGB_STAGE_SMEM
+	if (STAGE == ST_CHAIN || STAGE == ST_CHAIN_RESCUE) { mbar_init((uint64_t*)sim_smem.data(), 1); sim_smem[2] = 0; }
 	const int n_work_sim = L.n_work_dev? (int)*L.n_work_dev : L.n_work;
 	for (int it = 0; it < n_work_sim; ++it) {
 		int item = L.rid_list? L.rid_list[it] : it;
 		A.top = 0;
 		int rc;
 #if MGB_W > 1
-		if (MGB_IS_WARP(STAGE)) { // all lanes of the simulated warp enter, each with its own copy of the arena header (as in registers on the device)
+		if (entry == ENTER_WARP) { // all lanes of the simulated warp enter, each with its own copy of the arena header (as in registers on the device)
 			int rcs[MGB_W];
 			uint64_t peaks[MGB_W];
 			sim::tag()[0] = STAGE, sim::tag()[1] = item;
@@ -629,24 +732,19 @@ static void launch_stage(LaunchArgs &L, const Workers &W, int warps_override = 0
 			for (int l = 0; l < MGB_W; ++l) if (peaks[l] > A.peak) A.peak = peaks[l];
 		} else
 #endif
-		rc = run_stage<STAGE>(L, item, A, 0, MGB_IS_WARP(STAGE)? sim_smem.data() : 0);
+		rc = run_stage<STAGE>(L, item, A, 0, entry == ENTER_WARP? sim_smem.data() : 0);
 		if (rc < 0 && getenv("MGB_HOSTSIM_TRACE")) fprintf(stderr, "[hostsim] stage %d item %d failed with %d\n", STAGE, item, rc);
 		if (rc < 0) stage_fail<STAGE>(L, item, rc);
 	}
 	if (W.peak && A.peak > W.peak[0]) W.peak[0] = A.peak;
 #else
-	const int warps = warps_override > 0? warps_override : STAGE_WARPS[STAGE], threads = warps * 32;
-	int want = dev_sm_count() * STAGE_MINB[STAGE] * STAGE_WARPS[STAGE]; // resident warps this stage can keep on the chip
-	int n_w = std::min(W.n_workers, want);
-	int blocks = std::max(1, n_w / warps);
-	size_t smem = STAGE == 4? (size_t)warps * WfTier1::STRIDE : STAGE == 6? (size_t)warps * WfTier2::STRIDE : STAGE == 0? (size_t)warps * SKETCH_SMEM_BYTES : STAGE == 8? (size_t)warps * GWFA_SMEM_ARENA : STAGE == 1? (size_t)warps * CHAIN_SMEM_BYTES : STAGE == 19? (size_t)warps * CHAIN_RESCUE_SMEM_BYTES : 0;
-	void (*kern)(LaunchArgs) = StageKernel<STAGE>::get();
+	const int warps = g_shape.warps[STAGE];
+	const int want = dev_sm_count() * g_shape.minb[STAGE] * warps; // resident warps this stage can keep on the chip
+	const int blocks = std::max(1, std::min(W.n_workers, want) / warps);
+	const size_t smem = (size_t)warps * StageRow<STAGE>::SMEM;
+	const StageFn kern = stage_kernel<STAGE>();
 	if (smem > 48 * 1024) CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-	L.thread_mode = (p_thread_mask >> STAGE) & 1;
-	if (MGB_IS_WARP(STAGE)) L.thread_mode = 0;
-	if (STAGE == 17) L.thread_mode = 1;
-	if (L.thread_mode) smem = 0;
-	kern<<<blocks, threads, smem, t_stream>>>(L);
+	kern<<<blocks, warps * 32, smem, t_stream>>>(L);
 	CUDA_OK(cudaGetLastError());
 #endif
 }
@@ -688,14 +786,19 @@ struct Model {
 		mgb::HostPool host_pool; // packing and result assembly of the batch on this slot
 		Workers W;
 		mgb_stats_t st;
-		double ev_first_ms, ev_last_ms; // first kernel start / last kernel end relative to the batch reference event
-#ifndef MGB_HOSTSIM
-		cudaStream_t stream;
-		cudaEvent_t ev_first, ev_last, ev_piece[4];
-#endif
-		struct SlotTimers *timers = 0;
+		DevStream stream;
+		DevEvent ev_first, ev_last, ev_piece[4]; // first kernel start, last kernel end; the pieces of the result copy
+		SlotTimers *timers = 0;
 		bool ready;
 		Slot() : ready(false) { memset(&W, 0, sizeof(W)); }
+		~Slot() // (on the model's device; the GrowBufs release themselves)
+		{
+			delete timers;
+			W.release();
+#ifndef MGB_HOSTSIM
+			if (ready) { cudaStreamDestroy(stream); cudaEventDestroy(ev_first); cudaEventDestroy(ev_last); for (int i = 0; i < 4; ++i) cudaEventDestroy(ev_piece[i]); }
+#endif
+		}
 	};
 	enum { MAX_SLOTS = 8 };
 	Slot slots[MAX_SLOTS];
@@ -712,34 +815,16 @@ struct Model {
 	uint64_t lab_cap = 0; int32_t lab_max_dist_g = -1; int64_t lab_sources = 0;
 };
 
-struct SlotTimers;
-static void timers_free(SlotTimers *t);
 static void model_free(Model *M)
 {
 	for (Model *P : M->peers) model_free(P);
 	M->peers.clear();
-#ifndef MGB_HOSTSIM
-	cudaSetDevice(M->device);
-#endif
+	set_device(M->device);
 	for (void *p : M->dev_ptrs) dfree(p);
-	if (M->W.arena) dfree(M->W.arena);
-	if (M->W.peak) dfree(M->W.peak);
-	if (M->Wbig.arena) dfree(M->Wbig.arena);
-	if (M->Wbig.peak) dfree(M->Wbig.peak);
+	M->W.release(), M->Wbig.release();
 	if (M->d_logf) dfree(M->d_logf);
 	dfree(M->d_lab_off), dfree(M->d_lab_hdr), dfree(M->d_lab_pool), dfree(M->d_occ_sorted);
-	for (int k = 0; k < Model::MAX_SLOTS; ++k) {
-		Model::Slot &sl = M->slots[k];
-		sl.h_seq.release(), sl.h_out.release(), sl.h_small.release(), sl.h_pk.release(), sl.h_mail.release(), sl.h_routs.release(), sl.d_pk.release(), sl.d_seq.release(), sl.d_meta.release(), sl.d_routs.release(), sl.d_small.release(), sl.d_jobq.release(), sl.d_order.release(), sl.d_packed.release(), sl.d_packoff.release(), sl.d_segs.release(), sl.d_lab_new.release();
-		for (int i = 0; i < 10; ++i) sl.d_pool[i].release();
-		if (sl.timers) timers_free(sl.timers);
-		if (sl.W.arena) dfree(sl.W.arena);
-		if (sl.W.peak) dfree(sl.W.peak);
-#ifndef MGB_HOSTSIM
-		if (sl.ready) { cudaStreamDestroy(sl.stream); cudaEventDestroy(sl.ev_first); cudaEventDestroy(sl.ev_last); for (int i = 0; i < 4; ++i) cudaEventDestroy(sl.ev_piece[i]); }
-#endif
-	}
-	delete M;
+	delete M; // (the slots release their own)
 }
 
 static unsigned char comp_tab[256];
@@ -756,8 +841,7 @@ static void init_comp_tab() // reference: gfa-base.c:509-526 gfa_comp_table
 static void ensure_workers(Workers &W, int n_workers, uint64_t arena_bytes)
 {
 	if (W.arena && W.n_workers == n_workers && W.arena_bytes == arena_bytes) return;
-	if (W.arena) dfree(W.arena);
-	if (W.peak) dfree(W.peak);
+	W.release();
 	W.n_workers = n_workers, W.arena_bytes = arena_bytes;
 	W.arena = (char*)dmalloc((size_t)n_workers * arena_bytes);
 	W.peak = (uint64_t*)dmalloc((size_t)n_workers * sizeof(uint64_t));
@@ -771,6 +855,38 @@ static int default_workers()
 #else
 	return dev_sm_count() * (int)p_workers_per_sm;
 #endif
+}
+
+// The minimizer table built on the host: grouped by minimizer, occurrence lists ascending (reference: index.c:115-165 mg_idx_a2h)
+static void index_on_host(Model *M, std::vector<u128> &mz)
+{
+	std::sort(mz.begin(), mz.end(), [](const u128 &a, const u128 &b) { return (a.x >> 8) != (b.x >> 8)? (a.x >> 8) < (b.x >> 8) : a.y < b.y; });
+	size_t n_keys = 0;
+	for (size_t i = 0; i < mz.size(); ++i) if (i == 0 || (mz[i].x >> 8) != (mz[i-1].x >> 8)) ++n_keys;
+	uint64_t n_slots = 16;
+	while (n_slots < n_keys * 2) n_slots <<= 1;
+	M->n_slots_mask = n_slots - 1;
+	M->slot.assign(n_slots, u128{~0ULL, ~0ULL});
+	M->occ.reserve(n_keys);
+	for (size_t i = 0; i < mz.size();) {
+		size_t j = i;
+		uint64_t key = mz[i].x >> 8;
+		while (j < mz.size() && (mz[j].x >> 8) == key) ++j;
+		uint64_t h = idx_slot_hash(key) & M->n_slots_mask;
+		while (M->slot[h].x != ~0ULL) h = (h + 1) & M->n_slots_mask;
+		if (j - i == 1) {
+			M->slot[h].x = key << 1 | 1, M->slot[h].y = mz[i].y;
+			M->occ.push_back(1);
+		} else {
+			M->slot[h].x = key << 1, M->slot[h].y = (uint64_t)M->pos.size() << 32 | (uint64_t)(j - i);
+			for (size_t t = i; t < j; ++t) M->pos.push_back(mz[t].y);
+			M->occ.push_back((uint32_t)(j - i));
+		}
+		i = j;
+	}
+	M->ix.n_slots_mask = M->n_slots_mask;
+	M->ix.slot = dalloc_copy(M->slot), M->dev_ptrs.push_back((void*)M->ix.slot);
+	M->ix.pos = dalloc_copy(M->pos), M->dev_ptrs.push_back((void*)M->ix.pos);
 }
 
 static Model *model_build(gfa_t *g, int k, int w)
@@ -848,7 +964,7 @@ static Model *model_build(gfa_t *g, int k, int w)
 			memset(&L, 0, sizeof(L));
 			L.c.g = M->g, L.c.ix = M->ix, L.c.next_read = d_next;
 			L.routs = (ReadOut*)d_status, L.rid_list = 0, L.n_work = (int32_t)n_seg, L.pool_mz = d_pool, L.mz = d_mz;
-			launch_stage<3>(L, M->W);
+			launch_stage<ST_INDEX_SKETCH>(L, M->W);
 			dsync();
 			d2h(&st0, d_status, sizeof(int));
 			d2h(&hp, d_pool, sizeof(Pool));
@@ -859,8 +975,7 @@ static Model *model_build(gfa_t *g, int k, int w)
 #ifndef MGB_HOSTSIM
 			if (!retry && p_index_dev) { // group, lay out and insert on the device (mgb_index.cuh)
 				DevIndexOut out;
-				dfree(M->W.arena), dfree(M->W.peak); // the sketch arenas are not needed again; the sort wants the memory
-				memset(&M->W, 0, sizeof(Workers));
+				M->W.release(); // the sketch arenas are not needed again; the sort wants the memory
 				cudaError_t e = build_index_device(d_mz, hp.used / sizeof(u128), 2 * k, t_stream, &out);
 				dfree(d_pool), dfree(d_mz), dfree(d_status), dfree(d_next);
 				if (e != cudaSuccess) { set_error(std::string("index build on the device: ") + cudaGetErrorString(e)); throw MgbError{MGB_E_INTERNAL}; }
@@ -879,38 +994,11 @@ static Model *model_build(gfa_t *g, int k, int w)
 		}
 	}
 	// the sketch arenas are not needed again (every mapping slot owns its arenas)
-	dfree(M->W.arena), dfree(M->W.peak);
-	memset(&M->W, 0, sizeof(Workers));
-	// group by minimizer; occurrence lists ascending (reference: index.c:115-165 mg_idx_a2h)
-	std::sort(mz.begin(), mz.end(), [](const u128 &a, const u128 &b) { return (a.x >> 8) != (b.x >> 8)? (a.x >> 8) < (b.x >> 8) : a.y < b.y; });
-	size_t n_keys = 0;
-	for (size_t i = 0; i < mz.size(); ++i) if (i == 0 || (mz[i].x >> 8) != (mz[i-1].x >> 8)) ++n_keys;
-	uint64_t n_slots = 16;
-	while (n_slots < n_keys * 2) n_slots <<= 1;
-	M->n_slots_mask = n_slots - 1;
-	M->slot.assign(n_slots, u128{~0ULL, ~0ULL});
-	M->occ.reserve(n_keys);
-	for (size_t i = 0; i < mz.size();) {
-		size_t j = i;
-		uint64_t key = mz[i].x >> 8;
-		while (j < mz.size() && (mz[j].x >> 8) == key) ++j;
-		uint64_t h = idx_slot_hash(key) & M->n_slots_mask;
-		while (M->slot[h].x != ~0ULL) h = (h + 1) & M->n_slots_mask;
-		if (j - i == 1) {
-			M->slot[h].x = key << 1 | 1, M->slot[h].y = mz[i].y;
-			M->occ.push_back(1);
-		} else {
-			M->slot[h].x = key << 1, M->slot[h].y = (uint64_t)M->pos.size() << 32 | (uint64_t)(j - i);
-			for (size_t t = i; t < j; ++t) M->pos.push_back(mz[t].y);
-			M->occ.push_back((uint32_t)(j - i));
-		}
-		i = j;
-	}
-	M->ix.n_slots_mask = M->n_slots_mask;
-	M->ix.slot = dalloc_copy(M->slot), M->dev_ptrs.push_back((void*)M->ix.slot);
-	M->ix.pos = dalloc_copy(M->pos), M->dev_ptrs.push_back((void*)M->ix.pos);
+	M->W.release();
+	index_on_host(M, mz);
 	return M;
 }
+
 
 static const Model *model_of(const mg_idx_t *gi) { return (const Model*)gi->B; }
 
@@ -1071,29 +1159,6 @@ extern "C" void mgb_free_batch(int n_reads, mg_gchains_t **gcs)
 // batch dispatcher
 // ---------------------------------------------------------------------------------------------------------------
 
-static double now_ms() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
-
-#ifndef MGB_HOSTSIM
-struct EvTimer {
-	cudaEvent_t a, b; bool used;
-	EvTimer() : used(false) { cudaEventCreate(&a); cudaEventCreate(&b); }
-	~EvTimer() { cudaEventDestroy(a); cudaEventDestroy(b); }
-	void start() { cudaEventRecord(a, t_stream); used = true; }
-	void stop() { cudaEventRecord(b, t_stream); }
-	double ms() { if (!used) return 0; float t = 0; cudaEventSynchronize(b); cudaEventElapsedTime(&t, a, b); return t; }
-	void clear() { used = false; }
-};
-#else
-struct EvTimer { double t0 = 0, t1 = 0; void start() { t0 = now_ms(); } void stop() { t1 = now_ms(); } double ms() { return t1 - t0; } void clear() { t0 = t1 = 0; } };
-#endif
-
-struct SlotTimers {
-	EvTimer h2d, seed, chain, align, wfa, fin, d2h, lab, k[10];
-	void reset() { EvTimer *all[] = {&h2d, &seed, &chain, &align, &wfa, &fin, &d2h, &lab}; for (EvTimer *t : all) t->clear(); for (int i = 0; i < 10; ++i) k[i].clear(); }
-};
-
-static void timers_free(SlotTimers *t) { delete t; }
-
 static void fill_opt(MapOptDev &o, const mg_mapopt_t *opt, int k)
 {
 	memset(&o, 0, sizeof(o));
@@ -1198,447 +1263,470 @@ static void lab_after_batch(Model *M, unsigned int n_new)
 	h2d(M->d_lab_hdr, &hp, sizeof(Pool));
 }
 
+enum { P_ANCHOR, P_MINIPOS, P_LCHAIN, P_OUT, P_PLAN, P_JOBS, P_CIG, P_GSTATE, P_GJOBS, P_WALK, N_POOLS };
+
+// What the phases of one sub-batch share: its reads, where they and the per-read arrays live on both sides, the pool capacities
+// and the launch arguments of the pass.  All buffers are the slot's and persistent: cudaMalloc/cudaFree would serialise the slots.
+struct Batch {
+	Model *M; Model::Slot &sl; mgb_stats_t &S; SlotTimers &TM; const MapOptDev &o;
+	int n_reads; const int *qlens; const char *const *seqs; const char *const *names; mg_gchains_t **gcs; int host_threads;
+	const std::vector<int32_t> *seg_off, *seg_len;
+	int32_t skip1_len, skip2_len; // the tier routing this batch runs with
+	double t_host0;
+	// host side, page-locked
+	uint64_t *seq_off = 0; char *hseq = 0; size_t hseq_bytes = 0;
+	ReadOut *routs = 0; ReadMeta *meta = 0; Mail *mail = 0; char *hout = 0;
+	std::vector<uint64_t> pack_off;
+	// device side
+	bool packed = false, use_lab = false, first_kernel = true;
+	char *d_seq = 0; uint64_t *d_pk = 0, *d_pk_off = 0, *d_seq_off = 0; int32_t *d_seq_len = 0; uint32_t *d_name_hash = 0;
+	int32_t *d_list_buf = 0, *d_self_id = 0, *d_rescue = 0, *d_seg_off = 0, *d_seg_len = 0, *d_lab_new = 0;
+	unsigned int *d_next = 0, *d_jobq_n = 0, *d_rescue_n = 0, *d_cnt = 0, *d_tier_hist = 0, *d_lab_n = 0;
+	unsigned long long *d_prof = 0; Pool *d_pools = 0; ReadMeta *d_meta = 0; ReadOut *d_routs = 0;
+	uint64_t cap[N_POOLS] = {}; void *d_buf[N_POOLS] = {};
+	int64_t max_jobs = 0, jobs_done = 0, gjobs_done = 0; int32_t *jobq_buf = 0, *order_buf = 0;
+	LaunchArgs L = {};
+	MailSrc msrc = {};
+	int read_status(int i) const { return meta[i].status < 0? meta[i].status : routs[i].status; }
+	void pfor(int64_t n, const std::function<void(int64_t)> &fn)
+	{
+		if (n < 256 || host_threads <= 1) { for (int64_t i = 0; i < n; ++i) fn(i); return; }
+		sl.host_pool.run(n, host_threads, fn);
+	}
+};
+
+// Reads go to and results come from the device in a few pieces, so that the copy of one piece overlaps the host work on the next.
+template<typename F> static void for_pieces(int n_reads, const F &fn)
+{
+	const int n_piece = n_reads >= 2048? 4 : 1;
+	for (int pc = 0; pc < n_piece; ++pc) fn(pc, (int64_t)n_reads * pc / n_piece, (int64_t)n_reads * (pc + 1) / n_piece);
+}
+// fill(r) writes read r into the staging copy h, at element off[r]; each piece goes up as soon as it is filled.  Returns the host
+// time spent filling.
+template<typename T, typename F> static double upload_pieces(Batch &B, T *d, const T *h, const uint64_t *off, uint64_t end, const F &fill)
+{
+	double t = 0;
+	for_pieces(B.n_reads, [&](int, int64_t r0, int64_t r1) {
+		const double t0 = now_ms();
+		B.pfor(r1 - r0, [&](int64_t i) { fill(r0 + i); });
+		t += now_ms() - t0;
+		const uint64_t e0 = off[r0], e1 = r1 < B.n_reads? off[r1] : end;
+		h2d_async(d + e0, h + e0, (e1 - e0) * sizeof(T));
+	});
+	return t;
+}
+
+// Phase 2: the per-read arrays and the counters of the sub-batch, carved from one device buffer
+static void carve_small(Batch &B)
+{
+	const int n = B.n_reads;
+	char *ds = (char*)B.sl.d_small.ensure((size_t)n * (8 + 4 + 4 + 4 + 4 + 4) + 4096 + 1024);
+	B.d_seq_off = (uint64_t*)ds;
+	B.d_seq_len = (int32_t*)(B.d_seq_off + n);
+	B.d_name_hash = (uint32_t*)(B.d_seq_len + n);
+	B.d_list_buf = (int32_t*)(B.d_name_hash + n); // n entries: read list of the retry pass
+	B.d_self_id = B.d_list_buf + n; // n entries, MG_M_NO_DIAG only
+	B.d_rescue = B.d_self_id + n; // n entries: reads handed from k_chain to k_chain_rescue
+	char *dsm = (char*)(((uintptr_t)(B.d_rescue + n) + 255) & ~(uintptr_t)255);
+	B.d_next = (unsigned int*)dsm;
+	B.d_jobq_n = B.d_next + 4;
+	B.d_rescue_n = B.d_next + 8;
+	B.d_cnt = B.d_next + 10; // [0] bridging jobs, [1] gap jobs the next job kernel has to take
+	B.d_prof = (unsigned long long*)(dsm + 64);
+	B.d_pools = (Pool*)(dsm + 64 + sizeof(unsigned long long) * PROF_N);
+	B.d_tier_hist = (unsigned int*)((char*)(B.d_pools + 16) + 64); // 32 x 4 counters behind the pool headers
+}
+
+// Phase 1, packed: 2 bits per base (a quarter of the bytes; k_unpack writes the ASCII copy on the device).  A read with any byte
+// other than A/C/G/T goes up as ASCII; false when such reads are too many to be worth a copy each: the whole batch goes up as ASCII.
+static bool upload_packed(Batch &B)
+{
+	mgb_stats_t &S = B.S;
+	const int n = B.n_reads;
+	const size_t n8 = ((size_t)n + 7) & ~(size_t)7;
+	uint64_t *pk_off = (uint64_t*)B.sl.h_pk.ensure((size_t)n * 8 + 64 + (size_t)(S.n_bases / 4) + (size_t)n * 16);
+	uint64_t wtot = 0;
+	for (int i = 0; i < n; ++i) { pk_off[i] = wtot; wtot += (uint64_t)((B.qlens[i] > 0? B.qlens[i] : 0) + 31) / 32 + 1; }
+	uint64_t *hpk = pk_off + n8;
+	B.d_pk_off = (uint64_t*)B.sl.d_pk.ensure((n8 + wtot + 8) * 8);
+	B.d_pk = B.d_pk_off + n8;
+	std::vector<uint8_t> raw((size_t)n, 0);
+	const double t_pack = upload_pieces(B, B.d_pk, hpk, pk_off, wtot, [&](int64_t r) {
+		if (B.qlens[r] > 0 && !pack_read(B.seqs[r], B.qlens[r], hpk + pk_off[r])) raw[(size_t)r] = 1;
+	});
+	int64_t n_raw = 0;
+	for (int i = 0; i < n; ++i) n_raw += raw[(size_t)i];
+	if (n_raw > 64) return false;
+	S.t_pack_ms = t_pack;
+	S.h2d_bytes = (int64_t)(wtot * 8);
+	for (int i = 0; i < n; ++i)
+		if (raw[(size_t)i]) {
+			memcpy(B.hseq + B.seq_off[i], B.seqs[i], (size_t)B.qlens[i]);
+			h2d_async(B.d_seq + B.seq_off[i], B.hseq + B.seq_off[i], (size_t)B.qlens[i]);
+			pk_off[i] = ~0ULL, S.h2d_bytes += B.qlens[i];
+		}
+	h2d(B.d_pk_off, pk_off, (size_t)n * 8);
+	return true;
+}
+
+// Phase 1: the reads into page-locked memory and to the device, 2 bits per base unless the fragments have segments
+static void upload_reads(Batch &B)
+{
+	mgb_stats_t &S = B.S;
+	const int n = B.n_reads;
+	uint64_t *seq_off = B.seq_off = (uint64_t*)B.sl.h_small.ensure((size_t)n * (8 + 4 + 4) + 256);
+	int32_t *seq_len = (int32_t*)(seq_off + n);
+	uint32_t *name_hash = (uint32_t*)(seq_len + n);
+	uint64_t tot = 0;
+	for (int i = 0; i < n; ++i) {
+		seq_off[i] = tot, seq_len[i] = B.qlens[i];
+		tot += (uint64_t)(B.qlens[i] > 0? B.qlens[i] : 0) + 8;
+		tot = (tot + 15) & ~(uint64_t)15;
+		name_hash[i] = B.names && B.names[i]? hash_str(B.names[i]) : 0;
+		S.n_bases += B.qlens[i] > 0? B.qlens[i] : 0;
+	}
+	S.n_reads = n;
+	B.hseq_bytes = tot + 16;
+	B.hseq = (char*)B.sl.h_seq.ensure(B.hseq_bytes);
+	B.d_seq = (char*)B.sl.d_seq.ensure(B.hseq_bytes);
+	B.TM.h2d.start();
+	B.packed = p_pack2 && B.seg_off == 0 && upload_packed(B);
+	if (!B.packed) {
+		S.t_pack_ms += upload_pieces(B, B.d_seq, B.hseq, B.seq_off, B.hseq_bytes, [&](int64_t r) {
+			if (B.qlens[r] > 0) memcpy(B.hseq + B.seq_off[r], B.seqs[r], (size_t)B.qlens[r]);
+		});
+		dsync();
+		S.h2d_bytes = (int64_t)B.hseq_bytes;
+	}
+	carve_small(B);
+	h2d(B.d_seq_off, seq_off, (size_t)n * 16); // seq_off, seq_len and name_hash are contiguous on both sides
+	S.h2d_bytes += (int64_t)n * 16;
+	if (B.packed) {
+		UnpackArgs U;
+		U.pk = B.d_pk, U.pk_off = B.d_pk_off, U.seq_off = B.d_seq_off, U.seq_len = B.d_seq_len, U.seq = B.d_seq, U.n_reads = n;
+		unpack_reads(U);
+	}
+	B.TM.h2d.stop();
+	if (B.o.flag & F_NO_DIAG) { // which segment name, if any, is the read's own (exact string match on the host)
+		std::vector<int32_t> self((size_t)n, -1);
+		for (int i = 0; i < n; ++i)
+			if (B.names && B.names[i]) { auto it = B.M->name_ids.find(B.names[i]); if (it != B.M->name_ids.end()) self[(size_t)i] = it->second; }
+		h2d(B.d_self_id, self.data(), sizeof(int32_t) * (size_t)n);
+	}
+	if (B.seg_off && B.seg_len) { // multi-segment fragments only (mg_map_frag with n_segs > 1)
+		B.d_seg_off = (int32_t*)B.sl.d_segs.ensure(sizeof(int32_t) * (B.seg_off->size() + B.seg_len->size()));
+		B.d_seg_len = B.d_seg_off + B.seg_off->size();
+		h2d(B.d_seg_off, B.seg_off->data(), sizeof(int32_t) * B.seg_off->size());
+		h2d(B.d_seg_len, B.seg_len->data(), sizeof(int32_t) * B.seg_len->size());
+	}
+	B.d_meta = (ReadMeta*)B.sl.d_meta.ensure(sizeof(ReadMeta) * (size_t)n);
+	B.d_routs = (ReadOut*)B.sl.d_routs.ensure(sizeof(ReadOut) * (size_t)n);
+	dzero(B.d_meta, sizeof(ReadMeta) * (size_t)n);
+	dzero(B.d_routs, sizeof(ReadOut) * (size_t)n);
+	dzero(B.d_prof, sizeof(unsigned long long) * PROF_N);
+	dzero(B.d_tier_hist, sizeof(unsigned int) * 128);
+}
+
+// Phase 3: the first pool sizes, and what every pass of the sub-batch reports into (statuses, label sources, mailbox)
+static void size_pools(Batch &B)
+{
+	const uint64_t nb = (uint64_t)B.S.n_bases, nr = (uint64_t)B.n_reads;
+	uint64_t *cap = B.cap;
+	cap[P_ANCHOR] = std::max<uint64_t>(nb / 4 * sizeof(u128), (uint64_t)1 << 22);
+	cap[P_MINIPOS] = std::max<uint64_t>(nb * sizeof(int32_t) / 2, (uint64_t)1 << 20);
+	cap[P_LCHAIN] = std::max<uint64_t>(nr * 64 * sizeof(LChain), (uint64_t)1 << 20);
+	cap[P_OUT] = std::max<uint64_t>(nb * 4, (uint64_t)1 << 22);
+	cap[P_PLAN] = std::max<uint64_t>(nb / 8 * 8, (uint64_t)1 << 20);
+	cap[P_JOBS] = std::max<uint64_t>(nb / 40 * sizeof(WfaJob), (uint64_t)1 << 20);
+	cap[P_CIG] = std::max<uint64_t>(nb, (uint64_t)1 << 20) + (uint64_t)B.sl.W.n_workers * CIG_CHUNK_BYTES * 4; // + the unused ends of the warps' slices (three tier kernels per pass)
+	cap[P_GSTATE] = std::max<uint64_t>(nr * 2048, (uint64_t)1 << 20);
+	cap[P_GJOBS] = std::max<uint64_t>(nr * 24 * sizeof(GwfaJob), (uint64_t)1 << 20);
+	cap[P_WALK] = std::max<uint64_t>(nr * 256, (uint64_t)1 << 20);
+	for (int i = 0; i < N_POOLS; ++i) if (B.sl.d_pool[i].cap > cap[i]) cap[i] = B.sl.d_pool[i].cap & ~(size_t)4095; // keep what earlier batches needed
+	B.routs = (ReadOut*)B.sl.h_routs.ensure((sizeof(ReadOut) + sizeof(ReadMeta)) * nr + 64); // page-locked: a pageable destination makes the copy a blocking, staged one
+	B.meta = (ReadMeta*)(B.routs + B.n_reads);
+	B.use_lab = p_lab_cache && lab_prepare(B.M, B.o.bw_long);
+	B.mail = (Mail*)B.sl.h_mail.ensure(sizeof(Mail));
+	if (B.use_lab) { // this call's list of sources to search
+		B.d_lab_n = (unsigned int*)B.sl.d_lab_new.ensure(((size_t)B.M->g.n_seg * 2 + 4) * sizeof(int32_t));
+		B.d_lab_new = (int32_t*)(B.d_lab_n + 4);
+	}
+	MailSrc &m = B.msrc;
+	m.pools = B.d_pools, m.jobq_n = B.d_jobq_n, m.lab_n = B.d_lab_n, m.prof = B.d_prof, m.tier_hist = B.d_tier_hist, m.peak = B.sl.W.peak, m.n_workers = B.sl.W.n_workers;
+}
+
+// Phase 4: empty pools of the current sizes and the launch arguments of a pass over them
+static void fill_launch_args(Batch &B)
+{
+	const Model *M = B.M;
+	const uint64_t *cap = B.cap;
+	Pool hp[N_POOLS];
+	for (int i = 0; i < N_POOLS; ++i) B.d_buf[i] = B.sl.d_pool[i].ensure(cap[i]), hp[i].used = 0, hp[i].cap = cap[i];
+	h2d(B.d_pools, hp, sizeof(hp));
+	dfill(B.d_buf[P_GJOBS], 0xff, cap[P_GJOBS]); // reserved-but-unused bridging job slots read as rid == -1
+	dfill(B.d_buf[P_JOBS], 0xff, cap[P_JOBS]);   // the same for gap jobs: slots of an allocation that overflowed the pool are never written
+	LaunchArgs &L = B.L;
+	memset(&L, 0, sizeof(L));
+	L.c.g = M->g, L.c.ix = M->ix, L.c.opt = B.o;
+	L.c.b.n_reads = B.n_reads, L.c.b.seq = B.d_seq, L.c.b.seq_off = B.d_seq_off, L.c.b.seq_len = B.d_seq_len, L.c.b.name_hash = B.d_name_hash;
+	L.c.b.seg_off = B.d_seg_off, L.c.b.seg_len = B.d_seg_len, L.c.b.self_id = (B.o.flag & F_NO_DIAG)? B.d_self_id : 0;
+	L.c.b.pk = B.packed? B.d_pk : 0, L.c.b.pk_off = B.packed? B.d_pk_off : 0;
+	L.c.meta = B.d_meta;
+	L.c.pool_anchor = &B.d_pools[P_ANCHOR], L.c.anchor = (u128*)B.d_buf[P_ANCHOR];
+	L.c.pool_minipos = &B.d_pools[P_MINIPOS], L.c.minipos = (int32_t*)B.d_buf[P_MINIPOS];
+	L.c.pool_lchain = &B.d_pools[P_LCHAIN], L.c.lchain = (LChain*)B.d_buf[P_LCHAIN];
+	L.c.pool_out = &B.d_pools[P_OUT], L.c.out = (char*)B.d_buf[P_OUT];
+	L.c.pool_plan = &B.d_pools[P_PLAN], L.c.plan = (uint64_t*)B.d_buf[P_PLAN];
+	L.c.pool_jobs = &B.d_pools[P_JOBS], L.c.jobs = (WfaJob*)B.d_buf[P_JOBS];
+	L.c.pool_cig = &B.d_pools[P_CIG], L.c.cig = (uint32_t*)B.d_buf[P_CIG];
+	L.c.pool_gstate = &B.d_pools[P_GSTATE], L.c.gstate = (char*)B.d_buf[P_GSTATE];
+	L.c.pool_gjobs = &B.d_pools[P_GJOBS], L.c.gjobs = (GwfaJob*)B.d_buf[P_GJOBS];
+	L.c.pool_walk = &B.d_pools[P_WALK], L.c.walk = (int32_t*)B.d_buf[P_WALK];
+	L.c.next_read = B.d_next;
+	L.c.rescue_list = B.d_rescue, L.c.rescue_n = B.d_rescue_n;
+	if (B.use_lab) {
+		L.c.lab.src_off = M->d_lab_off, L.c.lab.pool_hdr = M->d_lab_hdr, L.c.lab.pool = M->d_lab_pool, L.c.lab.new_src = B.d_lab_new, L.c.lab.n_new = B.d_lab_n;
+		L.c.lab.max_dist_g = M->lab_max_dist_g, L.c.lab.cap_new = M->g.n_seg * 2;
+		dzero(B.d_lab_n, 2 * sizeof(unsigned int));
+	}
+	L.c.prof = B.d_prof;
+	L.c.tier_hist = B.d_tier_hist, L.c.skip1_len = B.skip1_len, L.c.skip2_len = B.skip2_len;
+	L.c.jobq_n = B.d_jobq_n;
+	L.routs = B.d_routs;
+	B.jobs_done = B.gjobs_done = 0;
+	B.max_jobs = (int64_t)(cap[P_JOBS] / sizeof(WfaJob)) + 1;
+	const int64_t max_gjobs = (int64_t)(cap[P_GJOBS] / sizeof(GwfaJob)) + 1;
+	B.jobq_buf = (int32_t*)B.sl.d_jobq.ensure(sizeof(int32_t) * 2 * (size_t)B.max_jobs);
+	B.order_buf = (int32_t*)B.sl.d_order.ensure(sizeof(int32_t) * (size_t)std::max<int64_t>(std::max<int64_t>(B.max_jobs, max_gjobs), B.n_reads));
+}
+
+// One stage of a pass, timed by t if given.  order: its items go longest first (make_job_order of that kind, inside the timed span).
+template<int STAGE> static void launch(Batch &B, const Workers &W, EvTimer *t, int order = NO_ORDER)
+{
+	Span span(t);
+	LaunchArgs &L = B.L;
+	const int32_t *list = L.rid_list;
+	if (order != NO_ORDER) {
+		make_job_order(L, order, order == ORDER_GAPS? L.c.jobq[1] : 0, L.n_work, B.order_buf, L.n_work_dev);
+		L.rid_list = B.order_buf;
+	}
+	launch_stage<STAGE>(L, W);
+	L.rid_list = list;
+}
+
+// Phase 5: one pass over a set of reads (d_list == 0: the whole sub-batch).  T: the timers of the first pass; the retry pass is
+// not timed.  From k_gchain on every kernel reads its number of units on the device: the whole pass is queued without a host
+// round trip, so nothing another thread does in the driver (large copies, blocking waits) can open gaps between its kernels.
+static void run_pass(Batch &B, const int32_t *d_list, int32_t n_list, const Workers &W, SlotTimers *T)
+{
+	LaunchArgs &L = B.L;
+	auto tm = [T](EvTimer SlotTimers::*m) { return T? &(T->*m) : (EvTimer*)0; };
+	auto tk = [T](int stage) { return T? &T->k[stage] : (EvTimer*)0; }; // (one per kernel slot)
+	auto counts = [&]() { count_jobs(B.d_pools, (int)P_GJOBS, (int)P_JOBS, (unsigned int)B.gjobs_done, (unsigned int)B.jobs_done, B.d_cnt); };
+	L.rid_list = d_list, L.n_work = n_list;
+	if (B.first_kernel) ev_record(B.sl.ev_first), B.first_kernel = false;
+	{ Span s(tm(&SlotTimers::seed)); launch<ST_SEED>(B, W, tk(ST_SEED)); }
+	{
+		Span s(tm(&SlotTimers::chain)), k(tk(ST_CHAIN)); // t_kernel_ms[1]: both chaining kernels
+		dzero(B.d_rescue_n, sizeof(unsigned int));
+		launch<ST_CHAIN>(B, W, 0);
+		L.n_work_dev = B.d_rescue_n, L.rid_list = 0; // the reads k_chain put on the rescue list (count known on the device only)
+		launch<ST_CHAIN_RESCUE>(B, W, 0);
+		L.n_work_dev = 0, L.rid_list = d_list;
+	}
+	{
+		Span s(tm(&SlotTimers::align));
+		if (B.use_lab) { // labels of the sources k_chain listed (count known on the device only)
+			L.n_work_dev = B.d_lab_n, L.rid_list = 0;
+			Span lab(tm(&SlotTimers::lab));
+			launch<ST_LABELS>(B, W, 0);
+			L.n_work_dev = B.d_lab_n + 1;
+			launch<ST_LABELS_BIG>(B, W, 0);
+			L.n_work_dev = 0, L.rid_list = d_list;
+		}
+		// whole batch: reads with many linear chains first (a few of them set the time of this kernel)
+		launch<ST_GCHAIN>(B, W, tk(ST_GCHAIN), d_list == 0 && n_list >= 1024? ORDER_READS : NO_ORDER);
+		counts(); // bridging jobs planned by k_gchain, then materialisation
+		L.rid_list = 0, L.job_start = B.gjobs_done, L.n_work = 0, L.n_work_dev = B.d_cnt;
+		launch<ST_GWFA>(B, W, tk(ST_GWFA), ORDER_BRIDGES);
+		L.rid_list = d_list, L.n_work = n_list, L.n_work_dev = 0;
+		launch<ST_GCHAIN_GEN>(B, W, tk(ST_GCHAIN_GEN));
+	}
+	{ // three tiers; a job that does not fit one tier is queued for the next
+		Span s(tm(&SlotTimers::wfa));
+		counts();
+		L.c.jobq[0] = B.jobq_buf, L.c.jobq[1] = B.jobq_buf + B.max_jobs;
+		dzero(B.d_jobq_n, 2 * sizeof(unsigned int));
+		L.rid_list = 0, L.job_start = B.jobs_done, L.n_work = 0, L.n_work_dev = B.d_cnt + 1;
+		launch<ST_WFA1>(B, W, tk(ST_WFA1));
+		L.n_work_dev = B.d_jobq_n;
+		launch<ST_WFA2>(B, W, tk(ST_WFA2));
+		L.n_work_dev = B.d_jobq_n + 1;
+		launch<ST_WFA3>(B, W, tk(ST_WFA3), ORDER_GAPS);
+		L.rid_list = 0, L.n_work_dev = 0;
+	}
+	L.rid_list = d_list, L.n_work = n_list;
+	{ Span s(tm(&SlotTimers::fin)); launch<ST_FINISH>(B, W, tk(ST_FINISH)); }
+	ev_record(B.sl.ev_last);
+	fetch_mail(B.msrc, B.mail); // (also the one wait of the pass)
+	const Pool &pg = B.mail->pools[P_GJOBS], &pj = B.mail->pools[P_JOBS];
+	B.gjobs_done = (int64_t)(std::min<uint64_t>(pg.used, pg.cap) / sizeof(GwfaJob));
+	B.jobs_done = (int64_t)(std::min<uint64_t>(pj.used, pj.cap) / sizeof(WfaJob));
+	if (T) B.S.n_jobs_mid = B.mail->jobq_n[0], B.S.n_jobs_big = B.mail->jobq_n[1];
+}
+
+// Phase 6: the reads whose worker arena overflowed run again with large arenas and few workers (shared by the slots).  Returns
+// whether an output pool overflowed: then the whole sub-batch runs again with larger pools.
+static bool redo_arena_overflows(Batch &B)
+{
+	const int n = B.n_reads;
+	auto fetch_status = [&]() {
+		d2h(B.routs, B.d_routs, sizeof(ReadOut) * (size_t)n);
+		d2h(B.meta, B.d_meta, sizeof(ReadMeta) * (size_t)n);
+	};
+	fetch_status();
+	std::vector<int32_t> redo;
+	bool pool_full = false;
+	for (int i = 0; i < n; ++i) {
+		const int st = B.read_status(i);
+		if (st == MGB_E_ARENA) redo.push_back(i);
+		else if (st == MGB_E_POOL) pool_full = true;
+	}
+	if (pool_full || redo.empty()) return pool_full;
+	Model *M = B.M;
+	std::lock_guard<std::mutex> lock(M->big_mutex);
+	const uint64_t big = (uint64_t)p_arena_big_mb << 20;
+	const int nw = (int)std::min<uint64_t>(16, std::max<uint64_t>(1, dev_free_mem() / 2 / big)); // a handful of reads per batch at most come here
+	if (M->Wbig.arena == 0 || M->Wbig.arena_bytes != big) ensure_workers(M->Wbig, std::max(1, nw), big);
+	h2d(B.d_list_buf, redo.data(), redo.size() * sizeof(int32_t));
+	{
+		std::unique_lock<std::mutex> gpu(M->gpu_mutex, std::defer_lock);
+		if (p_gpu_lock) gpu.lock();
+		const double tw = now_ms();
+		run_pass(B, B.d_list_buf, (int32_t)redo.size(), M->Wbig, 0);
+		B.S.w_redo_ms += now_ms() - tw;
+	}
+	B.S.n_retry += (int64_t)redo.size();
+	fetch_status();
+	for (int i = 0; i < n; ++i) if (B.read_status(i) == MGB_E_POOL) pool_full = true;
+	return pool_full;
+}
+
+// Phase 7: the result blobs into read order, then to the host in pieces (the assembly follows piece by piece)
+static void download_results(Batch &B)
+{
+	const int n = B.n_reads;
+	B.TM.d2h.start();
+	const size_t pool_bytes = (size_t)std::min<uint64_t>(B.mail->pools[P_OUT].used, B.cap[P_OUT]);
+	PackArgs P;
+	P.routs = B.d_routs, P.meta = B.d_meta, P.n = n, P.pool = (const char*)B.d_buf[P_OUT];
+	P.packed = (char*)B.sl.d_packed.ensure(pool_bytes + 64), P.off = (uint64_t*)B.sl.d_packoff.ensure(sizeof(uint64_t) * ((size_t)n + 1));
+	pack_results(P);
+	d2h(B.routs, B.d_routs, sizeof(ReadOut) * (size_t)n);
+	B.pack_off.resize((size_t)n + 1);
+	d2h(B.pack_off.data(), P.off, sizeof(uint64_t) * ((size_t)n + 1));
+	const size_t out_bytes = (size_t)B.pack_off[n];
+	B.hout = (char*)B.sl.h_out.ensure(out_bytes + 64);
+	for_pieces(n, [&](int pc, int64_t r0, int64_t r1) {
+		const uint64_t b0 = B.pack_off[r0], b1 = B.pack_off[r1];
+		d2h_async(B.hout + b0, P.packed + b0, b1 - b0);
+		ev_record(B.sl.ev_piece[pc]);
+	});
+	B.TM.d2h.stop();
+	B.S.out_bytes = (int64_t)out_bytes;
+}
+
+// Phase 8: tier routing for the next batch: the first length bucket in which the sampled gaps mostly ended beyond a tier
+static void learn_tier_routing(Batch &B)
+{
+	const unsigned int *h = B.mail->tier_hist;
+	int32_t t1 = INT32_MAX, t2 = INT32_MAX;
+	for (int b = 0; b < 32 && t1 == INT32_MAX; ++b) { unsigned int in = h[b * 4 + 1], out = h[b * 4 + 2] + h[b * 4 + 3]; if (in + out >= 8 && in < out) t1 = b * 16; }
+	for (int b = 0; b < 32 && t2 == INT32_MAX; ++b) { unsigned int in = h[b * 4 + 1] + h[b * 4 + 2], out = h[b * 4 + 3]; if (in + out >= 8 && in < out) t2 = b * 16; }
+	unsigned int tot = 0;
+	for (int i = 0; i < 128; ++i) tot += h[i];
+	if (tot >= 64 && p_tier_learn) { std::lock_guard<std::mutex> lock(B.M->big_mutex); B.M->skip1_len = t1, B.M->skip2_len = t2 < t1? t1 : t2; }
+	B.S.skip1_len = B.skip1_len, B.S.skip2_len = B.skip2_len;
+}
+
+// Phase 9: mg_gchains_t of every read, piece by piece as the copies land
+static int assemble_results(Batch &B)
+{
+	mgb_stats_t &S = B.S;
+	const double t_asm0 = now_ms();
+	S.w_download_ms = t_asm0 - B.t_host0 - S.w_upload_ms - S.w_pass_ms - S.w_redo_ms - S.w_gpu_wait_ms;
+	for (int i = 0; i < B.n_reads; ++i) {
+		const int st = B.read_status(i);
+		if (st < 0) {
+			char buf[256];
+			snprintf(buf, sizeof(buf), "read '%s' (%d bp) failed on the device with code %d%s", B.names && B.names[i]? B.names[i] : "", B.qlens[i], st,
+					 st == MGB_E_ARENA? " (worker arena exhausted even in the retry pass; raise arena_big_mb)" : "");
+			set_error(buf);
+			return st;
+		}
+		const ReadMeta &m = B.meta[i];
+		S.n_seeds += m.n_seed0, S.n_anchors_out += m.n_a, S.n_chains_out += m.n_u0, S.n_minimizers += m.n_mz;
+	}
+	for_pieces(B.n_reads, [&](int pc, int64_t r0, int64_t r1) {
+		ev_wait(B.sl.ev_piece[pc]);
+		B.pfor(r1 - r0, [&](int64_t k) {
+			const int64_t i = r0 + k;
+			if (B.read_status((int)i) == 1) B.gcs[i] = 0; // empty or over-long read: reference returns before allocating (map-algo.c:359-360)
+			else B.gcs[i] = build_result(B.routs[i], B.hout);
+		});
+	});
+	S.t_asm_ms = now_ms() - t_asm0;
+	S.t_d2h_ms = B.TM.d2h.ms(); // pack kernels + the pieces of the copy (they overlap the assembly above)
+	S.t_host_ms = now_ms() - B.t_host0;
+	return 0;
+}
+
 // Map reads [0, n_reads) of one sub-batch on the calling thread's stream (slot `sl`).
 static int map_range(Model *M, Model::Slot &sl, const MapOptDev &o, int n_reads, const int *qlens, const char *const *seqs, const char *const *names,
 					 mg_gchains_t **gcs, int host_threads, const std::vector<int32_t> *seg_off = 0, const std::vector<int32_t> *seg_len = 0)
 {
 	mgb_stats_t &S = sl.st;
 	memset(&S, 0, sizeof(S));
-	sl.ev_first_ms = sl.ev_last_ms = 0;
 	if (n_reads <= 0) return 0;
-	const int32_t L_skip1 = M->skip1_len, L_skip2 = M->skip2_len; // thresholds this batch runs with
-	double t_host0 = now_ms();
-	// ---- pack the sub-batch into page-locked memory ----
-	uint64_t tot = 0;
-	uint64_t *seq_off; int32_t *seq_len; uint32_t *name_hash;
-	{
-		size_t small = (size_t)n_reads * (8 + 4 + 4) + 256;
-		char *hs = (char*)sl.h_small.ensure(small);
-		seq_off = (uint64_t*)hs, seq_len = (int32_t*)(seq_off + n_reads), name_hash = (uint32_t*)(seq_len + n_reads);
-	}
-	for (int i = 0; i < n_reads; ++i) {
-		seq_off[i] = tot, seq_len[i] = qlens[i];
-		tot += (uint64_t)(qlens[i] > 0? qlens[i] : 0) + 8;
-		tot = (tot + 15) & ~(uint64_t)15;
-		name_hash[i] = names && names[i]? hash_str(names[i]) : 0;
-		S.n_bases += qlens[i] > 0? qlens[i] : 0;
-	}
-	S.n_reads = n_reads;
-	const size_t hseq_bytes = tot + 16;
-	char *hseq = (char*)sl.h_seq.ensure(hseq_bytes);
-	auto pfor = [&](int64_t n, const std::function<void(int64_t)> &fn) {
-		if (n < 256 || host_threads <= 1) { for (int64_t i = 0; i < n; ++i) fn(i); return; }
-		sl.host_pool.run(n, host_threads, fn);
-	};
 	// the event pairs live in the slot: creating and destroying three dozen events per call contends on the driver's lock with the other calls in flight
 	if (sl.timers == 0) sl.timers = new SlotTimers();
-	SlotTimers &TM = *sl.timers;
-	TM.reset();
-	EvTimer &tm_h2d = TM.h2d, &tm_seed = TM.seed, &tm_chain = TM.chain, &tm_align = TM.align, &tm_wfa = TM.wfa, &tm_fin = TM.fin, &tm_d2h = TM.d2h, &tm_lab = TM.lab;
-	EvTimer *tm_k = TM.k; // one per kernel (first pass only)
-	// ---- device buffers (all persistent: cudaMalloc/cudaFree would serialise the slots) ----
-	enum { P_ANCHOR, P_MINIPOS, P_LCHAIN, P_OUT, P_PLAN, P_JOBS, P_CIG, P_GSTATE, P_GJOBS, P_WALK, N_POOLS };
-	char *d_seq = (char*)sl.d_seq.ensure(hseq_bytes);
-	tm_h2d.start();
-	// The reads go up 2 bits per base (a quarter of the bytes) and k_unpack writes their ASCII copy on the device; a read with any
-	// byte other than A/C/G/T goes up as ASCII, and so does the whole batch when such reads are many or the fragments have segments.
-	uint64_t *pk_off = 0, *d_pk = 0, *d_pk_off = 0;
-	bool packed_mode = p_pack2 && seg_off == 0;
-	if (packed_mode) {
-		pk_off = (uint64_t*)sl.h_pk.ensure((size_t)n_reads * 8 + 64 + (size_t)(S.n_bases / 4) + (size_t)n_reads * 16);
-		uint64_t wtot = 0;
-		for (int i = 0; i < n_reads; ++i) { pk_off[i] = wtot; wtot += (uint64_t)((qlens[i] > 0? qlens[i] : 0) + 31) / 32 + 1; }
-		uint64_t *hpk = pk_off + (((size_t)n_reads + 7) & ~(size_t)7);
-		d_pk_off = (uint64_t*)sl.d_pk.ensure(((((size_t)n_reads + 7) & ~(size_t)7) + wtot + 8) * 8);
-		d_pk = d_pk_off + (((size_t)n_reads + 7) & ~(size_t)7);
-		std::vector<uint8_t> raw((size_t)n_reads, 0);
-		const int n_piece = n_reads >= 2048? 4 : 1;
-		double t_pack = 0;
-		for (int pc = 0; pc < n_piece; ++pc) {
-			const int64_t r0 = (int64_t)n_reads * pc / n_piece, r1 = (int64_t)n_reads * (pc + 1) / n_piece;
-			if (r0 >= r1) continue;
-			const double tp0 = now_ms();
-			pfor(r1 - r0, [&](int64_t i) { const int64_t r = r0 + i; if (qlens[r] > 0 && !pack_read(seqs[r], qlens[r], hpk + pk_off[r])) raw[(size_t)r] = 1; });
-			t_pack += now_ms() - tp0;
-			const uint64_t w0 = pk_off[r0], w1 = r1 < n_reads? pk_off[r1] : wtot;
-#ifndef MGB_HOSTSIM
-			CUDA_OK(cudaMemcpyAsync(d_pk + w0, hpk + w0, (w1 - w0) * 8, cudaMemcpyHostToDevice, t_stream));
-#else
-			memcpy(d_pk + w0, hpk + w0, (w1 - w0) * 8);
-#endif
-		}
-		int64_t n_raw = 0;
-		for (int i = 0; i < n_reads; ++i) n_raw += raw[(size_t)i];
-		if (n_raw > 64) packed_mode = false; // not worth a copy per read
-		else {
-			S.t_pack_ms = t_pack;
-			S.h2d_bytes = (int64_t)(wtot * 8);
-			for (int i = 0; i < n_reads; ++i)
-				if (raw[(size_t)i]) {
-					memcpy(hseq + seq_off[i], seqs[i], (size_t)qlens[i]);
-#ifndef MGB_HOSTSIM
-					CUDA_OK(cudaMemcpyAsync(d_seq + seq_off[i], hseq + seq_off[i], (size_t)qlens[i], cudaMemcpyHostToDevice, t_stream));
-#else
-					memcpy(d_seq + seq_off[i], hseq + seq_off[i], (size_t)qlens[i]);
-#endif
-					pk_off[i] = ~0ULL, S.h2d_bytes += qlens[i];
-				}
-			h2d(d_pk_off, pk_off, (size_t)n_reads * 8);
-		}
-	}
-	if (!packed_mode) { // pack and upload in a few pieces: the copy of one piece runs while the host threads pack the next
-		const int n_piece = n_reads >= 2048? 4 : 1;
-		double t_pack = 0;
-		for (int pc = 0; pc < n_piece; ++pc) {
-			const int64_t r0 = (int64_t)n_reads * pc / n_piece, r1 = (int64_t)n_reads * (pc + 1) / n_piece;
-			if (r0 >= r1) continue;
-			const double tp0 = now_ms();
-			pfor(r1 - r0, [&](int64_t i) { if (qlens[r0 + i] > 0) memcpy(hseq + seq_off[r0 + i], seqs[r0 + i], (size_t)qlens[r0 + i]); });
-			t_pack += now_ms() - tp0;
-			const uint64_t b0 = seq_off[r0], b1 = r1 < n_reads? seq_off[r1] : (uint64_t)hseq_bytes;
-#ifndef MGB_HOSTSIM
-			CUDA_OK(cudaMemcpyAsync(d_seq + b0, hseq + b0, b1 - b0, cudaMemcpyHostToDevice, t_stream));
-#else
-			memcpy(d_seq + b0, hseq + b0, b1 - b0);
-#endif
-		}
-		dsync();
-		S.t_pack_ms += t_pack;
-		S.h2d_bytes = (int64_t)hseq_bytes;
-	}
-	size_t small_dev = (size_t)n_reads * (8 + 4 + 4 + 4 + 4 + 4) + 4096 + 1024;
-	char *ds = (char*)sl.d_small.ensure(small_dev);
-	uint64_t *d_seq_off = (uint64_t*)ds;
-	int32_t *d_seq_len = (int32_t*)(d_seq_off + n_reads);
-	uint32_t *d_name_hash = (uint32_t*)(d_seq_len + n_reads);
-	int32_t *d_list_buf = (int32_t*)(d_name_hash + n_reads); // n_reads entries: read list of the retry pass
-	int32_t *d_self_id = d_list_buf + n_reads; // n_reads entries, MG_M_NO_DIAG only
-	int32_t *d_rescue = d_self_id + n_reads; // n_reads entries: reads handed from k_chain to k_chain_rescue
-	char *dsm = (char*)(((uintptr_t)(d_rescue + n_reads) + 255) & ~(uintptr_t)255);
-	unsigned int *d_next = (unsigned int*)dsm;
-	unsigned int *d_jobq_n = d_next + 4;
-	unsigned int *d_rescue_n = d_next + 8;
-	unsigned int *d_cnt = d_next + 10; // [0] bridging jobs, [1] gap jobs the next job kernel has to take
-	unsigned long long *d_prof = (unsigned long long*)(dsm + 64);
-	Pool *d_pools = (Pool*)(dsm + 64 + sizeof(unsigned long long) * PROF_N);
-	unsigned int *d_tier_hist = (unsigned int*)((char*)(d_pools + 16) + 64); // 32 x 4 counters behind the pool headers
-	h2d(d_seq_off, seq_off, (size_t)n_reads * 16); // seq_off, seq_len and name_hash are contiguous on both sides
-	S.h2d_bytes += (int64_t)n_reads * 16;
-	if (packed_mode) {
-		UnpackArgs U;
-		U.pk = d_pk, U.pk_off = d_pk_off, U.seq_off = d_seq_off, U.seq_len = d_seq_len, U.seq = d_seq, U.n_reads = n_reads;
-#ifndef MGB_HOSTSIM
-		k_unpack<<<dev_sm_count() * 8, 256, 0, t_stream>>>(U);
-		CUDA_OK(cudaGetLastError());
-#else
-		for (int r = 0; r < n_reads; ++r) if (pk_off[r] != ~0ULL) for (int64_t wd = 0; wd * 32 < qlens[r]; ++wd) unpack_word(U, r, wd);
-#endif
-		S.n_launches += 1;
-	}
-	tm_h2d.stop();
-	const bool no_diag = (o.flag & F_NO_DIAG) != 0;
-	if (no_diag) { // which segment name, if any, is the read's own (exact string match on the host)
-		std::vector<int32_t> self((size_t)n_reads, -1);
-		for (int i = 0; i < n_reads; ++i)
-			if (names && names[i]) { auto it = M->name_ids.find(names[i]); if (it != M->name_ids.end()) self[(size_t)i] = it->second; }
-		h2d(d_self_id, self.data(), sizeof(int32_t) * (size_t)n_reads);
-	}
-	int32_t *d_seg_off = 0, *d_seg_len = 0; // multi-segment fragments only (mg_map_frag with n_segs > 1)
-	if (seg_off && seg_len) {
-		d_seg_off = (int32_t*)sl.d_segs.ensure(sizeof(int32_t) * (seg_off->size() + seg_len->size()));
-		d_seg_len = d_seg_off + seg_off->size();
-		h2d(d_seg_off, seg_off->data(), sizeof(int32_t) * seg_off->size());
-		h2d(d_seg_len, seg_len->data(), sizeof(int32_t) * seg_len->size());
-	}
-	ReadMeta *d_meta = (ReadMeta*)sl.d_meta.ensure(sizeof(ReadMeta) * (size_t)n_reads);
-	ReadOut *d_routs = (ReadOut*)sl.d_routs.ensure(sizeof(ReadOut) * (size_t)n_reads);
-	dzero(d_meta, sizeof(ReadMeta) * (size_t)n_reads);
-	dzero(d_routs, sizeof(ReadOut) * (size_t)n_reads);
-	dzero(d_prof, sizeof(unsigned long long) * PROF_N);
-	dzero(d_tier_hist, sizeof(unsigned int) * 128);
-	uint64_t cap[N_POOLS];
-	cap[P_ANCHOR] = std::max<uint64_t>((uint64_t)S.n_bases / 4 * sizeof(u128), (uint64_t)1 << 22);
-	cap[P_MINIPOS] = std::max<uint64_t>((uint64_t)S.n_bases * sizeof(int32_t) / 2, (uint64_t)1 << 20);
-	cap[P_LCHAIN] = std::max<uint64_t>((uint64_t)n_reads * 64 * sizeof(LChain), (uint64_t)1 << 20);
-	cap[P_OUT] = std::max<uint64_t>((uint64_t)S.n_bases * 4, (uint64_t)1 << 22);
-	cap[P_PLAN] = std::max<uint64_t>((uint64_t)S.n_bases / 8 * 8, (uint64_t)1 << 20);
-	cap[P_JOBS] = std::max<uint64_t>((uint64_t)S.n_bases / 40 * sizeof(WfaJob), (uint64_t)1 << 20);
-	cap[P_CIG] = std::max<uint64_t>((uint64_t)S.n_bases, (uint64_t)1 << 20) + (uint64_t)sl.W.n_workers * CIG_CHUNK_BYTES * 4; // + the unused ends of the warps' slices (three tier kernels per pass)
-	cap[P_GSTATE] = std::max<uint64_t>((uint64_t)n_reads * 2048, (uint64_t)1 << 20);
-	cap[P_GJOBS] = std::max<uint64_t>((uint64_t)n_reads * 24 * sizeof(GwfaJob), (uint64_t)1 << 20);
-	cap[P_WALK] = std::max<uint64_t>((uint64_t)n_reads * 256, (uint64_t)1 << 20);
-	for (int i = 0; i < N_POOLS; ++i) if (sl.d_pool[i].cap > cap[i]) cap[i] = sl.d_pool[i].cap & ~(size_t)4095; // keep what earlier batches needed
-	ReadOut *routs = (ReadOut*)sl.h_routs.ensure((sizeof(ReadOut) + sizeof(ReadMeta)) * (size_t)n_reads + 64); // page-locked: a pageable destination makes the copy a blocking, staged one
-	ReadMeta *meta = (ReadMeta*)(routs + n_reads);
-	char *hout = 0;
-	int rc_final = 0, n_piece = 1;
-	std::vector<uint64_t> pack_off;
-	bool first_kernel = true;
-	(void)first_kernel;
-
-	const bool use_lab = p_lab_cache && lab_prepare(M, o.bw_long);
-	int32_t *d_lab_new = 0; unsigned int *d_lab_n = 0; // this call's list of sources to search
-	Mail *mail = (Mail*)sl.h_mail.ensure(sizeof(Mail));
-	if (use_lab) { d_lab_n = (unsigned int*)sl.d_lab_new.ensure(((size_t)M->g.n_seg * 2 + 4) * sizeof(int32_t)); d_lab_new = (int32_t*)(d_lab_n + 4); }
-	MailSrc msrc;
-	msrc.pools = d_pools, msrc.jobq_n = d_jobq_n, msrc.lab_n = d_lab_n, msrc.prof = d_prof, msrc.tier_hist = d_tier_hist, msrc.peak = sl.W.peak, msrc.n_workers = sl.W.n_workers;
-	for (int attempt = 0; attempt < 8; ++attempt) {
-		void *d_buf[N_POOLS];
-		Pool hp[N_POOLS];
-		for (int i = 0; i < N_POOLS; ++i) d_buf[i] = sl.d_pool[i].ensure(cap[i]), hp[i].used = 0, hp[i].cap = cap[i];
-		h2d(d_pools, hp, sizeof(hp));
-		dfill(d_buf[P_GJOBS], 0xff, cap[P_GJOBS]); // reserved-but-unused bridging job slots read as rid == -1
-		dfill(d_buf[P_JOBS], 0xff, cap[P_JOBS]);   // the same for gap jobs: slots of an allocation that overflowed the pool are never written
-		LaunchArgs L;
-		memset(&L, 0, sizeof(L));
-		L.c.g = M->g, L.c.ix = M->ix, L.c.opt = o;
-		L.c.b.n_reads = n_reads, L.c.b.seq = d_seq, L.c.b.seq_off = d_seq_off, L.c.b.seq_len = d_seq_len, L.c.b.name_hash = d_name_hash;
-		L.c.b.seg_off = d_seg_off, L.c.b.seg_len = d_seg_len, L.c.b.self_id = no_diag? d_self_id : 0;
-		L.c.b.pk = packed_mode? d_pk : 0, L.c.b.pk_off = packed_mode? d_pk_off : 0;
-		L.c.meta = d_meta;
-		L.c.pool_anchor = &d_pools[P_ANCHOR], L.c.anchor = (u128*)d_buf[P_ANCHOR];
-		L.c.pool_minipos = &d_pools[P_MINIPOS], L.c.minipos = (int32_t*)d_buf[P_MINIPOS];
-		L.c.pool_lchain = &d_pools[P_LCHAIN], L.c.lchain = (LChain*)d_buf[P_LCHAIN];
-		L.c.pool_out = &d_pools[P_OUT], L.c.out = (char*)d_buf[P_OUT];
-		L.c.pool_plan = &d_pools[P_PLAN], L.c.plan = (uint64_t*)d_buf[P_PLAN];
-		L.c.pool_jobs = &d_pools[P_JOBS], L.c.jobs = (WfaJob*)d_buf[P_JOBS];
-		L.c.pool_cig = &d_pools[P_CIG], L.c.cig = (uint32_t*)d_buf[P_CIG];
-		L.c.pool_gstate = &d_pools[P_GSTATE], L.c.gstate = (char*)d_buf[P_GSTATE];
-		L.c.pool_gjobs = &d_pools[P_GJOBS], L.c.gjobs = (GwfaJob*)d_buf[P_GJOBS];
-		L.c.pool_walk = &d_pools[P_WALK], L.c.walk = (int32_t*)d_buf[P_WALK];
-		L.c.next_read = d_next;
-		L.c.rescue_list = d_rescue, L.c.rescue_n = d_rescue_n;
-		memset(&L.c.lab, 0, sizeof(L.c.lab));
-		if (use_lab) {
-			L.c.lab.src_off = M->d_lab_off, L.c.lab.pool_hdr = M->d_lab_hdr, L.c.lab.pool = M->d_lab_pool, L.c.lab.new_src = d_lab_new, L.c.lab.n_new = d_lab_n;
-			L.c.lab.max_dist_g = M->lab_max_dist_g, L.c.lab.cap_new = M->g.n_seg * 2;
-			dzero(d_lab_n, 2 * sizeof(unsigned int));
-		}
-		L.c.prof = d_prof;
-		L.c.tier_hist = d_tier_hist, L.c.skip1_len = L_skip1, L.c.skip2_len = L_skip2;
-		L.c.jobq[0] = 0, L.c.jobq[1] = 0, L.c.jobq_n = d_jobq_n;
-		L.routs = d_routs;
-		int64_t jobs_done = 0, gjobs_done = 0;
-		const int64_t max_jobs = (int64_t)(cap[P_JOBS] / sizeof(WfaJob)) + 1, max_gjobs = (int64_t)(cap[P_GJOBS] / sizeof(GwfaJob)) + 1;
-		int32_t *jobq_buf = (int32_t*)sl.d_jobq.ensure(sizeof(int32_t) * 2 * (size_t)max_jobs);
-		int32_t *order_buf = (int32_t*)sl.d_order.ensure(sizeof(int32_t) * (size_t)std::max<int64_t>(std::max<int64_t>(max_jobs, max_gjobs), n_reads));
-		// one pass over a set of reads; job counts are read back between the planning and the job kernels
-		auto run_pass = [&](const int32_t *d_list, int32_t n_list, const Workers &W, bool timed) {
-			L.rid_list = d_list, L.n_work = n_list;
-#ifndef MGB_HOSTSIM
-			if (first_kernel) { CUDA_OK(cudaEventRecord(sl.ev_first, t_stream)); first_kernel = false; }
-#endif
-			if (timed) tm_seed.start();
-			{ if (timed) tm_k[0].start(); launch_stage<0>(L, W); if (timed) tm_k[0].stop(); }
-			if (timed) tm_seed.stop(), tm_chain.start();
-			{
-				if (timed) tm_k[1].start();
-				dzero(d_rescue_n, sizeof(unsigned int));
-				launch_stage<1>(L, W);
-				L.n_work_dev = d_rescue_n, L.rid_list = 0; // the reads k_chain put on the rescue list (count known on the device only)
-				launch_stage<19>(L, W);
-				L.n_work_dev = 0, L.rid_list = d_list;
-				if (timed) tm_k[1].stop();
-				S.n_launches += 1;
-			}
-			if (timed) tm_chain.stop(), tm_align.start();
-			if (use_lab) { // labels of the sources k_chain listed (count known on the device only)
-				L.n_work_dev = d_lab_n, L.rid_list = 0;
-				if (timed) tm_lab.start();
-				launch_stage<17>(L, W);
-				L.n_work_dev = d_lab_n + 1;
-				launch_stage<18>(L, W);
-				if (timed) tm_lab.stop();
-				L.n_work_dev = 0, L.rid_list = d_list;
-				S.n_launches += 2;
-			}
-			if (d_list == 0 && n_list >= 1024) { // whole batch: reads with many linear chains first (a few of them set the time of this kernel)
-				if (timed) tm_k[2].start();
-				make_job_order(L, 2, 0, n_list, order_buf);
-				L.rid_list = order_buf;
-				launch_stage<2>(L, W);
-				L.rid_list = d_list;
-				if (timed) tm_k[2].stop();
-				S.n_launches += 1;
-			} else { if (timed) tm_k[2].start(); launch_stage<2>(L, W); if (timed) tm_k[2].stop(); }
-			auto counts = [&]() {
-#ifndef MGB_HOSTSIM
-				k_job_counts<<<1, 1, 0, t_stream>>>(d_pools, (int)P_GJOBS, (int)P_JOBS, (unsigned int)gjobs_done, (unsigned int)jobs_done, d_cnt);
-				CUDA_OK(cudaGetLastError());
-#else
-				job_counts(d_pools, (int)P_GJOBS, (int)P_JOBS, (unsigned int)gjobs_done, (unsigned int)jobs_done, d_cnt);
-#endif
-			};
-			// From here on every kernel reads its number of units on the device: the whole pass is queued without a host round trip, so
-			// nothing another thread does in the driver (large copies, blocking waits) can open gaps between its kernels.
-			{ // bridging jobs planned by k_gchain, then materialisation
-				counts();
-				L.rid_list = 0, L.job_start = gjobs_done, L.n_work = 0, L.n_work_dev = d_cnt;
-				if (timed) tm_k[8].start();
-				make_job_order(L, 0, 0, 0, order_buf, d_cnt);
-				L.rid_list = order_buf;
-				launch_stage<8>(L, W);
-				if (timed) tm_k[8].stop();
-				L.rid_list = d_list, L.n_work = n_list, L.n_work_dev = 0;
-				{ if (timed) tm_k[9].start(); launch_stage<9>(L, W); if (timed) tm_k[9].stop(); }
-				S.n_launches += 4;
-			}
-			if (timed) tm_align.stop();
-			if (timed) tm_wfa.start();
-			{ // three tiers; a job that does not fit one tier is queued for the next
-				counts();
-				L.c.jobq[0] = jobq_buf, L.c.jobq[1] = jobq_buf + max_jobs;
-				dzero(d_jobq_n, 2 * sizeof(unsigned int));
-				L.rid_list = 0, L.job_start = jobs_done, L.n_work = 0, L.n_work_dev = d_cnt + 1;
-				{ if (timed) tm_k[4].start(); launch_stage<4>(L, W); if (timed) tm_k[4].stop(); }
-				L.n_work_dev = d_jobq_n;
-				{ if (timed) tm_k[6].start(); launch_stage<6>(L, W); if (timed) tm_k[6].stop(); }
-				L.n_work_dev = d_jobq_n + 1;
-				if (timed) tm_k[7].start();
-				make_job_order(L, 1, L.c.jobq[1], 0, order_buf, d_jobq_n + 1);
-				L.rid_list = order_buf;
-				launch_stage<7>(L, W);
-				if (timed) tm_k[7].stop();
-				L.rid_list = 0, L.n_work_dev = 0;
-				S.n_launches += 5;
-			}
-			if (timed) tm_wfa.stop(), tm_fin.start();
-			L.rid_list = d_list, L.n_work = n_list;
-			{ if (timed) tm_k[5].start(); launch_stage<5>(L, W); if (timed) tm_k[5].stop(); }
-			if (timed) tm_fin.stop();
-			S.n_launches += 4;
-#ifndef MGB_HOSTSIM
-			CUDA_OK(cudaEventRecord(sl.ev_last, t_stream));
-#endif
-			fetch_mail(msrc, mail); // (also the one wait of the pass)
-			gjobs_done = (int64_t)(std::min<uint64_t>(mail->pools[P_GJOBS].used, mail->pools[P_GJOBS].cap) / sizeof(GwfaJob));
-			jobs_done = (int64_t)(std::min<uint64_t>(mail->pools[P_JOBS].used, mail->pools[P_JOBS].cap) / sizeof(WfaJob));
-			if (timed) S.n_jobs_mid = mail->jobq_n[0], S.n_jobs_big = mail->jobq_n[1];
-		};
+	sl.timers->reset();
+	const int64_t launches0 = t_launches;
+	Batch B{M, sl, S, *sl.timers, o, n_reads, qlens, seqs, names, gcs, host_threads, seg_off, seg_len, M->skip1_len, M->skip2_len, now_ms()};
+	upload_reads(B);
+	size_pools(B);
+	int rc = 0;
+	for (int attempt = 0;; ++attempt) {
+		fill_launch_args(B);
 		{
 			const double tq = now_ms();
-			if (attempt == 0) S.w_upload_ms = tq - t_host0;
+			if (attempt == 0) S.w_upload_ms = tq - B.t_host0;
 			std::unique_lock<std::mutex> gpu(M->gpu_mutex, std::defer_lock);
 			if (p_gpu_lock) gpu.lock();
 			const double tw = now_ms();
 			S.w_gpu_wait_ms += tw - tq;
-			run_pass(0, n_reads, sl.W, true);
+			run_pass(B, 0, n_reads, sl.W, &B.TM);
 			S.w_pass_ms += now_ms() - tw;
 		}
-		S.n_jobs = jobs_done;
-		d2h(routs, d_routs, sizeof(ReadOut) * (size_t)n_reads);
-		d2h(meta, d_meta, sizeof(ReadMeta) * (size_t)n_reads);
-
-		// reads whose worker arena overflowed: run them again with large arenas and few workers (shared by the slots)
-		std::vector<int32_t> redo;
-		bool pool_full = false;
-		for (int i = 0; i < n_reads; ++i) {
-			int st = meta[i].status < 0? meta[i].status : routs[i].status;
-			if (st == MGB_E_ARENA) redo.push_back(i);
-			else if (st == MGB_E_POOL) pool_full = true;
-		}
-		if (!pool_full && !redo.empty()) {
-			std::lock_guard<std::mutex> lock(M->big_mutex);
-			uint64_t big = (uint64_t)p_arena_big_mb << 20;
-			int nw = (int)std::min<uint64_t>(16, std::max<uint64_t>(1, dev_free_mem() / 2 / big)); // a handful of reads per batch at most come here
-			if (M->Wbig.arena == 0 || M->Wbig.arena_bytes != big) ensure_workers(M->Wbig, std::max(1, nw), big);
-			h2d(d_list_buf, redo.data(), redo.size() * sizeof(int32_t));
-			{ std::unique_lock<std::mutex> gpu(M->gpu_mutex, std::defer_lock); if (p_gpu_lock) gpu.lock(); const double tw = now_ms(); run_pass(d_list_buf, (int32_t)redo.size(), M->Wbig, false); S.w_redo_ms += now_ms() - tw; }
-			S.n_retry += (int64_t)redo.size();
-			d2h(routs, d_routs, sizeof(ReadOut) * (size_t)n_reads);
-			d2h(meta, d_meta, sizeof(ReadMeta) * (size_t)n_reads);
-			for (int i = 0; i < n_reads; ++i) {
-				int st = meta[i].status < 0? meta[i].status : routs[i].status;
-				if (st == MGB_E_POOL) pool_full = true;
-			}
-		}
-		fetch_mail(msrc, mail);
-		memcpy(hp, mail->pools, sizeof(hp));
-		if (use_lab) { unsigned int nn[2] = {mail->lab_n[0], mail->lab_n[1]}; S.n_lab_new = (int64_t)nn[0], S.n_lab_big = (int64_t)nn[1]; lab_after_batch(M, nn[0]); }
-		bool done = !pool_full;
-		if (done) { // blobs into read order, then to the host in pieces (the assembly below follows piece by piece)
-			tm_d2h.start();
-			const size_t pool_bytes = (size_t)std::min<uint64_t>(hp[P_OUT].used, cap[P_OUT]);
-			PackArgs P;
-			P.routs = d_routs, P.meta = d_meta, P.n = n_reads, P.pool = (const char*)d_buf[P_OUT];
-			P.packed = (char*)sl.d_packed.ensure(pool_bytes + 64), P.off = (uint64_t*)sl.d_packoff.ensure(sizeof(uint64_t) * ((size_t)n_reads + 1));
-			pack_results(P);
-			S.n_launches += 2;
-			d2h(routs, d_routs, sizeof(ReadOut) * (size_t)n_reads);
-			pack_off.resize((size_t)n_reads + 1);
-			d2h(pack_off.data(), P.off, sizeof(uint64_t) * ((size_t)n_reads + 1));
-			const size_t out_bytes = (size_t)pack_off[n_reads];
-			hout = (char*)sl.h_out.ensure(out_bytes + 64);
-			n_piece = n_reads >= 2048? 4 : 1;
-			for (int pc = 0; pc < n_piece; ++pc) {
-				const int64_t r0 = (int64_t)n_reads * pc / n_piece, r1 = (int64_t)n_reads * (pc + 1) / n_piece;
-				const uint64_t b0 = pack_off[r0], b1 = pack_off[r1];
-#ifndef MGB_HOSTSIM
-				if (b1 > b0) CUDA_OK(cudaMemcpyAsync(hout + b0, P.packed + b0, b1 - b0, cudaMemcpyDeviceToHost, t_stream));
-				CUDA_OK(cudaEventRecord(sl.ev_piece[pc], t_stream));
-#else
-				if (b1 > b0) memcpy(hout + b0, P.packed + b0, b1 - b0);
-#endif
-			}
-			tm_d2h.stop();
-			S.out_bytes = (int64_t)out_bytes;
-		}
-		if (done) break;
+		S.n_jobs = B.jobs_done;
+		const bool pool_full = redo_arena_overflows(B);
+		fetch_mail(B.msrc, B.mail);
+		if (B.use_lab) { S.n_lab_new = (int64_t)B.mail->lab_n[0], S.n_lab_big = (int64_t)B.mail->lab_n[1]; lab_after_batch(M, B.mail->lab_n[0]); }
+		if (!pool_full) { download_results(B); break; }
 		// grow whatever overflowed (used counts keep growing past cap, so they tell how much was wanted)
-		for (int i = 0; i < N_POOLS; ++i) if (hp[i].used > cap[i]) cap[i] = (hp[i].used * 3 / 2 + 4095) & ~(uint64_t)4095;
-		if (attempt == 7) { set_error("output pools kept overflowing"); rc_final = -2; }
+		for (int i = 0; i < N_POOLS; ++i) if (B.mail->pools[i].used > B.cap[i]) B.cap[i] = (B.mail->pools[i].used * 3 / 2 + 4095) & ~(uint64_t)4095;
+		if (attempt == 7) { set_error("output pools kept overflowing"); rc = -2; break; }
 	}
-	S.t_h2d_ms = tm_h2d.ms(), S.t_seed_ms = tm_seed.ms(), S.t_chain_ms = tm_chain.ms(), S.t_align_ms = tm_align.ms();
-	S.t_wfa_ms = tm_wfa.ms(), S.t_finish_ms = tm_fin.ms();
-	for (int i = 0; i < 10; ++i) S.t_kernel_ms[i] = tm_k[i].ms();
-	S.t_lab_ms = tm_lab.ms();
-	S.arena_peak = mail->arena_peak; // (the mailbox was last filled after the last pass of the batch)
-	for (int i = 0; i < 32; ++i) S.prof[i] = (uint64_t)mail->prof[i];
-	{ // tier routing for the next batch: the first length bucket in which the sampled gaps mostly ended beyond a tier
-		const unsigned int *h = mail->tier_hist;
-		int32_t t1 = INT32_MAX, t2 = INT32_MAX;
-		for (int b = 0; b < 32 && t1 == INT32_MAX; ++b) { unsigned int in = h[b * 4 + 1], out = h[b * 4 + 2] + h[b * 4 + 3]; if (in + out >= 8 && in < out) t1 = b * 16; }
-		for (int b = 0; b < 32 && t2 == INT32_MAX; ++b) { unsigned int in = h[b * 4 + 1] + h[b * 4 + 2], out = h[b * 4 + 3]; if (in + out >= 8 && in < out) t2 = b * 16; }
-		unsigned int tot = 0;
-		for (int i = 0; i < 128; ++i) tot += h[i];
-		if (tot >= 64 && p_tier_learn) { std::lock_guard<std::mutex> lock(M->big_mutex); M->skip1_len = t1, M->skip2_len = t2 < t1? t1 : t2; }
-		S.skip1_len = L_skip1, S.skip2_len = L_skip2;
-	}
-	if (rc_final < 0) return rc_final;
-
-	// ---- results ----
-	double t_asm0 = now_ms();
-	S.w_download_ms = t_asm0 - t_host0 - S.w_upload_ms - S.w_pass_ms - S.w_redo_ms - S.w_gpu_wait_ms;
-	int first_bad = -1;
-	for (int i = 0; i < n_reads; ++i) {
-		int st = meta[i].status < 0? meta[i].status : routs[i].status;
-		if (st < 0) { first_bad = i; break; }
-		S.n_seeds += meta[i].n_seed0, S.n_anchors_out += meta[i].n_a, S.n_chains_out += meta[i].n_u0, S.n_minimizers += meta[i].n_mz;
-	}
-	if (first_bad >= 0) {
-		int i = first_bad, st = meta[i].status < 0? meta[i].status : routs[i].status;
-		char buf[256];
-		snprintf(buf, sizeof(buf), "read '%s' (%d bp) failed on the device with code %d%s", names && names[i]? names[i] : "", qlens[i], st,
-				 st == MGB_E_ARENA? " (worker arena exhausted even in the retry pass; raise arena_big_mb)" : "");
-		set_error(buf);
-		return st;
-	}
-	for (int pc = 0; pc < n_piece; ++pc) {
-		const int64_t r0 = (int64_t)n_reads * pc / n_piece, r1 = (int64_t)n_reads * (pc + 1) / n_piece;
-#ifndef MGB_HOSTSIM
-		CUDA_OK(cudaEventSynchronize(sl.ev_piece[pc]));
-#endif
-		pfor(r1 - r0, [&](int64_t k) {
-			const int64_t i = r0 + k;
-			int st = meta[i].status < 0? meta[i].status : routs[i].status;
-			if (st == 1) gcs[i] = 0; // empty or over-long read: reference returns before allocating (map-algo.c:359-360)
-			else gcs[i] = build_result(routs[i], hout);
-		});
-	}
-	S.t_asm_ms = now_ms() - t_asm0;
-	S.t_d2h_ms = tm_d2h.ms(); // pack kernels + the pieces of the copy (they overlap the assembly above)
-	S.t_host_ms = now_ms() - t_host0;
-	return 0;
+	SlotTimers &TM = B.TM;
+	S.t_h2d_ms = TM.h2d.ms(), S.t_seed_ms = TM.seed.ms(), S.t_chain_ms = TM.chain.ms(), S.t_align_ms = TM.align.ms();
+	S.t_wfa_ms = TM.wfa.ms(), S.t_finish_ms = TM.fin.ms();
+	for (int i = 0; i < 10; ++i) S.t_kernel_ms[i] = TM.k[i].ms();
+	S.t_lab_ms = TM.lab.ms();
+	S.arena_peak = B.mail->arena_peak; // (the mailbox was last filled after the last pass of the batch)
+	for (int i = 0; i < 32; ++i) S.prof[i] = (uint64_t)B.mail->prof[i];
+	S.n_launches = t_launches - launches0;
+	learn_tier_routing(B);
+	return rc < 0? rc : assemble_results(B);
 }
 
 static void slot_prepare(Model *M, Model::Slot &sl, int n_workers)
@@ -1680,15 +1768,11 @@ static int map_batch_on(Model *M, int n_reads, const int *qlens, const char *con
 	}
 	Model::Slot &sl = M->slots[k];
 	const double t_slot = now_ms();
-#ifndef MGB_HOSTSIM
-	cudaSetDevice(M->device);
-#endif
+	set_device(M->device);
 	int rc = 0;
 	try {
 		slot_prepare(M, sl, p_slot_workers > 0? (int)p_slot_workers : default_workers());
-#ifndef MGB_HOSTSIM
-		t_stream = sl.stream;
-#endif
+		set_stream(sl.stream);
 		MapOptDev o;
 		fill_opt(o, opt, M->k);
 		{ // glibc logf table for mapq (reference: gcmisc.c:216-217); grown under the lock, old copies are kept until the model dies
@@ -1703,25 +1787,14 @@ static int map_batch_on(Model *M, int n_reads, const int *qlens, const char *con
 			}
 			o.logf_tab = M->d_logf, o.n_logf_tab = M->n_logf;
 		}
-		int nt = (int)p_host_threads;
-		if (nt <= 0) { nt = (int)std::thread::hardware_concurrency(); if (nt > 16) nt = 16; if (nt < 1) nt = 1; }
-		rc = map_range(M, sl, o, n_reads, qlens, seqs, names, gcs, nt, seg_off, seg_len);
-#ifndef MGB_HOSTSIM
-		t_stream = 0; // the slot's stream dies with the model; later calls on this thread (mg_index of another graph) use the default one
-#endif
+		rc = map_range(M, sl, o, n_reads, qlens, seqs, names, gcs, n_host_threads(), seg_off, seg_len);
 	} catch (const MgbError &e) {
 		rc = e.code;
-#ifndef MGB_HOSTSIM
-		t_stream = 0;
-#endif
 	}
+	set_stream(0); // the slot's stream dies with the model; later calls on this thread (mg_index of another graph) use the default one
 	mgb_stats_t S = sl.st;
 	S.w_slot_wait_ms = t_slot - t0;
-#ifndef MGB_HOSTSIM
-	if (rc == 0 && sl.ready) { float a = 0; if (cudaEventElapsedTime(&a, sl.ev_first, sl.ev_last) == cudaSuccess) S.t_dev_span_ms = a; }
-#else
-	S.t_dev_span_ms = S.t_seed_ms + S.t_chain_ms + S.t_align_ms + S.t_wfa_ms + S.t_finish_ms;
-#endif
+	if (rc == 0 && sl.ready) S.t_dev_span_ms = ev_elapsed_ms(sl.ev_first, sl.ev_last);
 	S.n_slots = k;
 	S.t_host_ms = now_ms() - t0;
 	t_last_stats = S, t_has_stats = true;
@@ -1768,9 +1841,7 @@ static int map_batch_impl(const mg_idx_t *gi, int n_reads, const int *qlens, con
 	int rc = 0;
 	for (int d = 0; d < n_dev; ++d) if (rcs[(size_t)d] < 0 && rc == 0) rc = rcs[(size_t)d];
 	if (rc < 0) for (int i = 0; i < n_reads; ++i) if (gcs[i]) { mg_gchain_free(gcs[i]); gcs[i] = 0; } // no partial results are left behind
-#ifndef MGB_HOSTSIM
-	cudaSetDevice(M->device);
-#endif
+	set_device(M->device);
 	return rc;
 }
 
