@@ -212,6 +212,20 @@ int mg_map_batch_frag(const mg_idx_t *gi, int n_frag, const int *n_seg, const in
 /* mg_gchain_free() over a whole batch (what step 2 of the reference pipeline does read by read, gmap.c:130); entries are set to NULL */
 void mgb_free_batch(int n_reads, mg_gchains_t **gcs);
 
+/* Map n_reads single-segment reads and return their GAF text, formatted on the device: byte for byte what
+ * mg_map_batch(gi, n_reads, qlens, seqs, names, gcs, opt) followed by
+ * mgb_write_gaf_batch(gi->g, n_reads, gcs, qlens, names, opt->flag, ...) produces, for every flag bit mgb_write_gaf() handles
+ * except MG_M_WRITE_LCHAIN / MG_M_WRITE_MZ (-S, --write-mz), which are refused with a negative code.  The flags are opt->flag,
+ * as the reference passes them to mg_write_gaf (gmap.c); a NULL names or names[i] prints as "*".
+ * (*out, *out_len, *out_cap) as in mgb_write_gaf_batch(). Returns 0, or a negative code with the reason in mgb_last_error();
+ * on failure *out_len is 0 and no text is left behind.
+ * The call follows the rules of mg_map_batch(): slots and concurrent callers, MGB_DEVICES (the text comes back in input order),
+ * the large-arena retry pass, growth of overflowing pools, error reporting.  No mg_gchains_t is built: the text is formatted
+ * from the device's result blobs, and only the text (plus 16 bytes per record for the dv:f field, which the host prints because
+ * its value comes from the host's libm) crosses PCIe.  The graph's names go to the device at the first call on an index. */
+int mgb_map_batch_gaf(const mg_idx_t *gi, int n_reads, const int *qlens, const char *const *seqs, const char *const *names,
+                      const mg_mapopt_t *opt, char **out, size_t *out_len, size_t *out_cap);
+
 /* ------------------------------------------------------------------------------------------------------------
  * Engine controls and instrumentation (not part of the reference API)
  * ---------------------------------------------------------------------------------------------------------- */
@@ -223,7 +237,7 @@ typedef struct {
 	int64_t skip1_len, skip2_len; /* WFA tier routing this batch ran with: gaps at or above these lengths skipped tier 1 / tier 2 */
 	int64_t n_jobs_side;    /* gaps aligned by the tier-3 launch that runs beside tiers 1/2 */
 	int64_t n_slots;        /* sub-batches the batch was cut into (each on its own stream and host thread) */
-	double t_pack_ms, t_asm_ms; /* host: packing reads into the staging buffer; building mg_gchains_t objects */
+	double t_pack_ms, t_asm_ms; /* host: packing reads into the staging buffer; building mg_gchains_t objects (mgb_map_batch_gaf: inserting dv:f and copying the text to the caller) */
 	int64_t n_jobs;         /* WFA jobs of the batch */
 	int64_t n_jobs_mid, n_jobs_big; /* jobs that went to tier 2 / tier 3 */
 	int64_t n_reads, n_bases;
@@ -231,8 +245,8 @@ typedef struct {
 	int64_t n_anchors_out;  /* sum of anchors kept in linear chains */
 	int64_t n_chains_out;   /* sum of linear chains out of the DP */
 	int64_t n_minimizers;
-	int64_t out_bytes;      /* result bytes copied back */
-	int64_t n_launches;     /* kernels launched for the batch */
+	int64_t out_bytes;      /* result bytes copied back (mgb_map_batch_gaf: the text and its dv:f fix-up records) */
+	int64_t n_launches;     /* kernels launched for the batch (mgb_map_batch_gaf: one more, k_gaf_size + scan + k_gaf_write in place of the two blob kernels) */
 	int64_t n_retry;        /* reads re-run with a larger arena */
 	uint64_t arena_peak;    /* largest per-worker arena use */
 	double t_kernel_ms[10]; /* CUDA-event time of each kernel of the first pass: k_seed, k_chain, k_gchain, (index), k_wfa_small, k_finish, k_wfa_mid, k_wfa_big, k_gwfa, k_gchain_gen */
@@ -244,6 +258,7 @@ typedef struct {
 	double w_gpu_wait_ms;   /* host wall clock spent waiting for the kernels of another call in flight to finish */
 	double w_slot_wait_ms, w_upload_ms, w_pass_ms, w_redo_ms, w_download_ms; /* host wall clock of the call: waiting for a slot; packing + H2D; the kernels of the first pass
 	                           with the host syncs between them; the large-arena pass over reads that outgrew their arena; result packing + D2H up to the assembly */
+	double t_gaf_ms;        /* mgb_map_batch_gaf: CUDA-event time of the GAF kernels (k_gaf_size with its scan, k_gaf_write); 0 for mg_map_batch */
 } mgb_stats_t;
 
 /* test hook: align one gap through the tier-3 WFA path (exact up to max_iter cells, then the reference's chaining

@@ -8,6 +8,11 @@ import os
 MG_M_RMQ = 0x8000
 MG_M_CIGAR = 0x4000000
 MG_M_PRINT_2ND = 0x2000
+MG_M_VERTEX_COOR = 0x800
+MG_M_SHOW_UNMAP = 0x100000
+MG_M_NO_COMP_PATH = 0x200000
+MG_M_WRITE_LCHAIN = 0x800000
+MG_M_WRITE_MZ = 0x1000000
 
 
 class mg128_t(C.Structure):
@@ -92,7 +97,8 @@ class mgb_stats_t(C.Structure):
                 ("n_reads", C.c_int64), ("n_bases", C.c_int64), ("n_seeds", C.c_int64), ("n_anchors_out", C.c_int64),
                 ("n_chains_out", C.c_int64), ("n_minimizers", C.c_int64), ("out_bytes", C.c_int64),
                 ("n_launches", C.c_int64), ("n_retry", C.c_int64), ("arena_peak", C.c_uint64), ("t_kernel_ms", C.c_double * 10), ("prof", C.c_uint64 * 32), ("t_lab_ms", C.c_double), ("n_lab_new", C.c_int64), ("n_lab_big", C.c_int64), ("h2d_bytes", C.c_int64),
-                ("w_gpu_wait_ms", C.c_double), ("w_slot_wait_ms", C.c_double), ("w_upload_ms", C.c_double), ("w_pass_ms", C.c_double), ("w_redo_ms", C.c_double), ("w_download_ms", C.c_double)]
+                ("w_gpu_wait_ms", C.c_double), ("w_slot_wait_ms", C.c_double), ("w_upload_ms", C.c_double), ("w_pass_ms", C.c_double), ("w_redo_ms", C.c_double), ("w_download_ms", C.c_double),
+                ("t_gaf_ms", C.c_double)]
 
 
 class mgb_reads_t(C.Structure):
@@ -183,4 +189,7 @@ def bind_engine_api(lib):
     lib.mgb_write_gaf_batch.restype = None
     lib.mgb_write_gaf_batch.argtypes = [C.POINTER(gfa_t), C.c_int, C.POINTER(C.POINTER(mg_gchains_t)), C.POINTER(C.c_int),
                                         C.POINTER(C.c_char_p), C.c_uint64, C.c_int, C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
+    lib.mgb_map_batch_gaf.restype = C.c_int
+    lib.mgb_map_batch_gaf.argtypes = [C.POINTER(mg_idx_t), C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_char_p), C.POINTER(C.c_char_p),
+                                      C.POINTER(mg_mapopt_t), C.POINTER(C.c_void_p), C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]
     return lib

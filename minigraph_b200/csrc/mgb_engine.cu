@@ -21,6 +21,7 @@
 
 #include "../../include/mgb200.h"
 #include "mgb_galign.cuh"
+#include "mgb_gaf.cuh"
 
 #ifndef MGB_HOSTSIM
 #include <cuda_runtime.h>
@@ -75,7 +76,9 @@ static int64_t p_lab_cache = 1;        // 0: graph chaining searches its walks p
 	X(k_gchain_gen,    ST_GCHAIN_GEN,    9, (128, 4),             4, 4,             0,                       ENTER_WARP,   1) /* K7b: graph-chain materialisation, post filters, mapq, alignment plan */ \
 	X(k_gc_labels,     ST_LABELS,       17, (128, 8),             4, 8,             0,                       ENTER_THREAD, 1) /* reachability labels of new source vertices (mgb_gclabel.cuh) */ \
 	X(k_gc_labels_big, ST_LABELS_BIG,   18, (128, 8),             4, 8,             0,                       ENTER_LANE0,  1) /* the few sources whose search outgrew a thread's share of the arena */ \
-	X(k_chain_rescue,  ST_CHAIN_RESCUE, 19, (192, 2),             6, 2,             CHAIN_RESCUE_SMEM_BYTES, ENTER_WARP,   1) /* K5: long-join rescue (RMQ chaining) of the reads k_chain listed (2 x 6 slices of 18 KB) */
+	X(k_chain_rescue,  ST_CHAIN_RESCUE, 19, (192, 2),             6, 2,             CHAIN_RESCUE_SMEM_BYTES, ENTER_WARP,   1) /* K5: long-join rescue (RMQ chaining) of the reads k_chain listed (2 x 6 slices of 18 KB) */ \
+	X(k_gaf_size,      ST_GAF_SIZE,     10, (128, 8),             4, 8,             0,                       ENTER_WARP,   1) /* mgb_map_batch_gaf: bytes and dv:f fix-ups of a read's GAF text (mgb_gaf.cuh) */ \
+	X(k_gaf_write,     ST_GAF_WRITE,    11, (128, 8),             4, 8,             0,                       ENTER_WARP,   1) /* mgb_map_batch_gaf: the text itself, at the read's place after the scan */
 enum StageEntry { ENTER_WARP, ENTER_LANE0, ENTER_THREAD };
 enum Stage {
 #define MGB_STAGE_ENUM(kern, st, num, ...) st = num,
@@ -192,8 +195,8 @@ static size_t dev_free_mem() { size_t f = 0, t = 0; CUDA_OK(cudaMemGetInfo(&f, &
 
 // the timers of a batch's first pass
 struct SlotTimers {
-	EvTimer h2d, seed, chain, align, wfa, fin, d2h, lab, k[10]; // k: per kernel slot of mgb_stats_t::t_kernel_ms
-	void reset() { EvTimer *all[] = {&h2d, &seed, &chain, &align, &wfa, &fin, &d2h, &lab}; for (EvTimer *t : all) t->clear(); for (int i = 0; i < 10; ++i) k[i].clear(); }
+	EvTimer h2d, seed, chain, align, wfa, fin, d2h, lab, gaf_size, gaf_write, k[10]; // k: per kernel slot of mgb_stats_t::t_kernel_ms
+	void reset() { EvTimer *all[] = {&h2d, &seed, &chain, &align, &wfa, &fin, &d2h, &lab, &gaf_size, &gaf_write}; for (EvTimer *t : all) t->clear(); for (int i = 0; i < 10; ++i) k[i].clear(); }
 };
 // a timer around a scope; none: the scope is not timed
 struct Span {
@@ -274,6 +277,7 @@ struct LaunchArgs {
 	int64_t job_start;       // first job of this launch (stage 4)
 	// segment sketch (index build)
 	Pool *pool_mz; u128 *mz;
+	const GafCtx *gaf;       // k_gaf_size / k_gaf_write (device memory)
 };
 
 // the columns of the stage table that the device code reads
@@ -299,6 +303,8 @@ MG_HD inline int run_stage(const LaunchArgs &L, int item, Arena &A, int lane, in
 	case ST_WFA1: return wfa_job_run(A, L.c, L.job_start + item, lane, smem, 1);
 	case ST_WFA2: return wfa_job_run(A, L.c, L.c.jobq[0][item], lane, smem, 2);
 	case ST_WFA3: return wfa_job_run(A, L.c, L.c.jobq[1][item], lane, smem, 3);
+	case ST_GAF_SIZE: return stage_gaf_size(*L.gaf, L.c, L.routs, item, lane);
+	case ST_GAF_WRITE: return stage_gaf_write(*L.gaf, L.c, L.routs, item, lane);
 	case ST_INDEX_SKETCH: { // sketch one graph segment for the index (reference: index.c:200-205)
 		AVec<u128> mv;
 		avec_init(mv);
@@ -534,6 +540,40 @@ static void pack_results(const PackArgs &P)
 	for (int r = 0; r < P.n; ++r) { P.off[r] = acc; acc += pack_size(P, r); }
 	P.off[P.n] = acc;
 	for (int r = 0; r < P.n; ++r) pack_read(P, r, 0, 1);
+#endif
+}
+
+// ---- GAF text: exclusive scan of the per-read sizes and fix-up counts, in place ([n] receives the totals), shaped like k_out_scan ----
+#ifndef MGB_HOSTSIM
+__global__ void __launch_bounds__(1024) k_gaf_scan(uint64_t *a, uint64_t *b, int n)
+{
+	__shared__ uint64_t pa[1024], pb[1024];
+	const int tid = threadIdx.x, per = (n + 1023) / 1024;
+	const int r0 = tid * per < n? tid * per : n, r1 = r0 + per < n? r0 + per : n;
+	uint64_t sa = 0, sb = 0;
+	for (int r = r0; r < r1; ++r) sa += a[r], sb += b[r];
+	pa[tid] = sa, pb[tid] = sb;
+	__syncthreads();
+	if (tid == 0) {
+		uint64_t xa = 0, xb = 0;
+		for (int i = 0; i < 1024; ++i) { const uint64_t ca = pa[i], cb = pb[i]; pa[i] = xa, pb[i] = xb; xa += ca, xb += cb; }
+		a[n] = xa, b[n] = xb;
+	}
+	__syncthreads();
+	uint64_t xa = pa[tid], xb = pb[tid];
+	for (int r = r0; r < r1; ++r) { const uint64_t ca = a[r], cb = b[r]; a[r] = xa, b[r] = xb; xa += ca, xb += cb; }
+}
+#endif
+static void gaf_scan(uint64_t *a, uint64_t *b, int n)
+{
+	++t_launches;
+#ifndef MGB_HOSTSIM
+	k_gaf_scan<<<1, 1024, 0, t_stream>>>(a, b, n);
+	CUDA_OK(cudaGetLastError());
+#else
+	uint64_t xa = 0, xb = 0;
+	for (int r = 0; r < n; ++r) { const uint64_t ca = a[r], cb = b[r]; a[r] = xa, b[r] = xb; xa += ca, xb += cb; }
+	a[n] = xa, b[n] = xb;
 #endif
 }
 
@@ -783,6 +823,7 @@ struct Model {
 	// so that kernels, copies and host-side result assembly of different sub-batches overlap
 	struct Slot {
 		GrowBuf h_seq{true}, h_out{true}, h_small{true}, h_pk{true}, h_mail{true}, h_routs{true}, d_pk, d_seq, d_meta, d_routs, d_small, d_jobq, d_order, d_packed, d_packoff, d_segs, d_lab_new, d_pool[10];
+		GrowBuf h_rname{true}, d_rname, d_gafctx, d_gafoff, d_text, d_fix; // the text route (mgb_map_batch_gaf)
 		mgb::HostPool host_pool; // packing and result assembly of the batch on this slot
 		Workers W;
 		mgb_stats_t st;
@@ -813,6 +854,8 @@ struct Model {
 	// reachability labels of the graph (mgb_gclabel.cuh): built on demand, kept across batches, grown between them
 	long long *d_lab_off = 0; Pool *d_lab_hdr = 0; char *d_lab_pool = 0;
 	uint64_t lab_cap = 0; int32_t lab_max_dist_g = -1; int64_t lab_sources = 0;
+	// the names the GAF kernels print (graph part of GafCtx): uploaded at the first mgb_map_batch_gaf() on this device
+	GafCtx gaf_graph = {}; bool gaf_ready = false;
 };
 
 static void model_free(Model *M)
@@ -1177,6 +1220,13 @@ static void fill_opt(MapOptDev &o, const mg_mapopt_t *opt, int k)
 	o.mask_level = opt->mask_level, o.sub_diff = opt->sub_diff, o.best_n = opt->best_n, o.pri_ratio = opt->pri_ratio, o.ref_bonus = opt->ref_bonus;
 }
 
+// mg_gchain_t::div (reference: gchain1.c:295) with the host's libm log (SURVEY H3): the result objects and the `dv:f` fix-ups of
+// the text route both take it from here
+static float gchain_div(int32_t n_mini, int32_t n_anchor, int32_t q_span)
+{
+	return n_mini >= n_anchor? (float)(log((double)n_mini / n_anchor) / q_span) : (float)(log((double)n_anchor / n_mini) / q_span);
+}
+
 static mg_gchains_t *build_result(const ReadOut &ro, const char *pool)
 {
 	const char *blob = pool + ro.blob_off;
@@ -1198,8 +1248,7 @@ static mg_gchains_t *build_result(const ReadOut &ro, const char *pool)
 		p->id = s->id, p->parent = s->parent, p->off = s->off, p->cnt = s->cnt, p->n_anchor = s->n_anchor, p->score = s->score;
 		p->qs = s->qs, p->qe = s->qe, p->plen = s->plen, p->ps = s->ps, p->pe = s->pe, p->blen = s->blen, p->mlen = s->mlen;
 		p->hash = s->hash, p->subsc = s->subsc, p->n_sub = s->n_sub, p->mapq = (uint32_t)s->mapq, p->flt = (uint32_t)s->flt;
-		// reference: gchain1.c:295 (host libm log, SURVEY H3)
-		p->div = s->n_mini >= s->n_anchor? (float)(log((double)s->n_mini / s->n_anchor) / s->q_span) : (float)(log((double)s->n_anchor / s->n_mini) / s->q_span);
+		p->div = gchain_div(s->n_mini, s->n_anchor, s->q_span);
 		if (s->has_cigar) {
 			p->p = (mg_cigar_t*)calloc(1, (size_t)s->n_cigar * 8 + sizeof(mg_cigar_t));
 			p->p->n_cigar = s->n_cigar, p->p->mlen = s->c_mlen, p->p->blen = s->c_blen, p->p->aplen = s->c_aplen, p->p->ss = s->c_ss, p->p->ee = s->c_ee;
@@ -1214,6 +1263,51 @@ static mg_gchains_t *build_result(const ReadOut &ro, const char *pool)
 	return gs;
 }
 
+// The text route (mgb_map_batch_gaf): the graph whose names are printed, and the caller's buffer, with the rules of
+// mgb_write_gaf_batch() for (*out, *out_len, *out_cap)
+struct GafRoute { const gfa_t *g; char **out; size_t *len, *cap; };
+// room for tot bytes and the terminator: the caller's buffer if out_cap says it is large enough, else a fresh malloc() block
+static char *gaf_reserve(const GafRoute &R, size_t tot)
+{
+	char *o = R.cap? *R.out : 0;
+	size_t cap = o? *R.cap : 0;
+	if (cap < tot + 1) {
+		free(o);
+		cap = tot + tot / 8 + 1;
+		o = (char*)malloc(cap);
+		if (o == 0) { set_error("out of host memory for the GAF text"); throw MgbError{MGB_E_INTERNAL}; }
+	}
+	*R.out = o;
+	if (R.cap) *R.cap = cap;
+	o[tot] = 0;
+	return o;
+}
+
+// The names the GAF kernels print, on the model's device, once (mg_index is not asked to pay for them)
+static void gaf_upload_graph(Model *M, const gfa_t *g)
+{
+	std::lock_guard<std::mutex> lk(M->big_mutex);
+	if (M->gaf_ready) return;
+	std::vector<char> sn, qn;
+	std::vector<uint64_t> sn_off(1, 0), qn_off(1, 0);
+	std::vector<int32_t> snid(g->n_seg), soff(g->n_seg), rank(g->n_sseq), mn(g->n_sseq), mx(g->n_sseq);
+	for (uint32_t i = 0; i < g->n_seg; ++i) {
+		const char *nm = g->seg[i].name? g->seg[i].name : "";
+		sn.insert(sn.end(), nm, nm + strlen(nm)), sn_off.push_back(sn.size());
+		snid[i] = g->seg[i].snid, soff[i] = g->seg[i].soff;
+	}
+	for (uint32_t i = 0; i < g->n_sseq; ++i) {
+		const char *nm = g->sseq[i].name? g->sseq[i].name : "";
+		qn.insert(qn.end(), nm, nm + strlen(nm)), qn_off.push_back(qn.size());
+		rank[i] = g->sseq[i].rank, mn[i] = g->sseq[i].min, mx[i] = g->sseq[i].max;
+	}
+	auto up = [&](const auto &v) { auto *d = dalloc_copy(v); M->dev_ptrs.push_back((void*)d); return d; };
+	GafCtx &x = M->gaf_graph;
+	x.seg_name = up(sn), x.seg_name_off = up(sn_off), x.seg_snid = up(snid), x.seg_soff = up(soff);
+	x.ss_name = up(qn), x.ss_name_off = up(qn_off), x.ss_rank = up(rank), x.ss_min = up(mn), x.ss_max = up(mx);
+	x.comp = up(std::vector<unsigned char>(comp_tab, comp_tab + 256));
+	M->gaf_ready = true;
+}
 
 // The label table of graph chaining: allocated at the first batch, emptied when a batch asks for longer walks than it was built for.
 static bool lab_prepare(Model *M, int32_t max_dist_g)
@@ -1269,7 +1363,7 @@ enum { P_ANCHOR, P_MINIPOS, P_LCHAIN, P_OUT, P_PLAN, P_JOBS, P_CIG, P_GSTATE, P_
 // and the launch arguments of the pass.  All buffers are the slot's and persistent: cudaMalloc/cudaFree would serialise the slots.
 struct Batch {
 	Model *M; Model::Slot &sl; mgb_stats_t &S; SlotTimers &TM; const MapOptDev &o;
-	int n_reads; const int *qlens; const char *const *seqs; const char *const *names; mg_gchains_t **gcs; int host_threads;
+	int n_reads; const int *qlens; const char *const *seqs; const char *const *names; mg_gchains_t **gcs; GafRoute *gaf; int host_threads; // gaf: the text route (gcs == NULL)
 	const std::vector<int32_t> *seg_off, *seg_len;
 	int32_t skip1_len, skip2_len; // the tier routing this batch runs with
 	double t_host0;
@@ -1277,6 +1371,7 @@ struct Batch {
 	uint64_t *seq_off = 0; char *hseq = 0; size_t hseq_bytes = 0;
 	ReadOut *routs = 0; ReadMeta *meta = 0; Mail *mail = 0; char *hout = 0;
 	std::vector<uint64_t> pack_off;
+	std::vector<uint64_t> gaf_off; size_t fix_at = 0; const uint64_t *d_rname_off = 0; const char *d_rname = 0; // text route: text and fix-up offsets ([n+1] each); where the fix-ups sit in hout; the read names
 	// device side
 	bool packed = false, use_lab = false, first_kernel = true;
 	char *d_seq = 0; uint64_t *d_pk = 0, *d_pk_off = 0, *d_seq_off = 0; int32_t *d_seq_len = 0; uint32_t *d_name_hash = 0;
@@ -1425,6 +1520,23 @@ static void upload_reads(Batch &B)
 	dzero(B.d_routs, sizeof(ReadOut) * (size_t)n);
 	dzero(B.d_prof, sizeof(unsigned long long) * PROF_N);
 	dzero(B.d_tier_hist, sizeof(unsigned int) * 128);
+	if (B.gaf) { // the text route prints the read names: their offsets, then the names back to back (a NULL name travels as "*")
+		uint64_t tot_n = 0;
+		for (int i = 0; i < n; ++i) tot_n += B.names && B.names[i]? strlen(B.names[i]) : 1;
+		const size_t hdr = ((size_t)n + 1) * 8;
+		uint64_t *h = (uint64_t*)B.sl.h_rname.ensure(hdr + tot_n + 16);
+		char *blob = (char*)(h + n + 1);
+		h[0] = 0;
+		for (int i = 0; i < n; ++i) {
+			const char *nm = B.names && B.names[i]? B.names[i] : "*";
+			const size_t l = strlen(nm);
+			memcpy(blob + h[i], nm, l), h[i + 1] = h[i] + l;
+		}
+		char *d = (char*)B.sl.d_rname.ensure(hdr + tot_n + 16);
+		h2d(d, h, hdr + tot_n);
+		B.d_rname_off = (const uint64_t*)d, B.d_rname = d + hdr;
+		S.h2d_bytes += (int64_t)(hdr + tot_n);
+	}
 }
 
 // Phase 3: the first pool sizes, and what every pass of the sub-batch reports into (statuses, label sources, mailbox)
@@ -1636,6 +1748,43 @@ static void download_results(Batch &B)
 	B.S.out_bytes = (int64_t)out_bytes;
 }
 
+// Phase 7, text route: the GAF text of every read, formatted on the device (mgb_gaf.cuh) from the blobs where the kernels left
+// them: k_gaf_size counts each read's bytes and dv:f fix-ups, one scan turns the counts into offsets, the host reads them back
+// once to size the buffers, k_gaf_write writes.  The fix-up records go to the host first, the text follows in pieces.
+static void download_gaf(Batch &B)
+{
+	const int n = B.n_reads;
+	B.TM.d2h.start();
+	GafCtx x = B.M->gaf_graph;
+	x.rname = B.d_rname, x.rname_off = B.d_rname_off, x.flag = B.o.flag;
+	x.text_off = (uint64_t*)B.sl.d_gafoff.ensure(sizeof(uint64_t) * 2 * ((size_t)n + 1)), x.fix_off = x.text_off + n + 1;
+	x.text = 0, x.fix = 0;
+	GafCtx *d_x = (GafCtx*)B.sl.d_gafctx.ensure(sizeof(GafCtx));
+	h2d(d_x, &x, sizeof(x));
+	LaunchArgs &L = B.L;
+	L.gaf = d_x, L.rid_list = 0, L.n_work = n, L.n_work_dev = 0;
+	{
+		Span t(&B.TM.gaf_size);
+		launch<ST_GAF_SIZE>(B, B.sl.W, 0);
+		gaf_scan(x.text_off, x.fix_off, n);
+	}
+	B.gaf_off.resize(2 * ((size_t)n + 1));
+	d2h(B.gaf_off.data(), x.text_off, sizeof(uint64_t) * B.gaf_off.size());
+	const uint64_t *toff = B.gaf_off.data(), text_bytes = toff[n], n_fix = toff[2 * n + 1];
+	x.text = (char*)B.sl.d_text.ensure(text_bytes + 64), x.fix = (GafFix*)B.sl.d_fix.ensure(n_fix * sizeof(GafFix) + 64);
+	h2d(d_x, &x, sizeof(x));
+	{ Span t(&B.TM.gaf_write); launch<ST_GAF_WRITE>(B, B.sl.W, 0); }
+	B.fix_at = (text_bytes + 15) & ~(uint64_t)15;
+	B.hout = (char*)B.sl.h_out.ensure(B.fix_at + n_fix * sizeof(GafFix) + 64);
+	d2h_async(B.hout + B.fix_at, x.fix, n_fix * sizeof(GafFix));
+	for_pieces(n, [&](int pc, int64_t r0, int64_t r1) {
+		d2h_async(B.hout + toff[r0], x.text + toff[r0], toff[r1] - toff[r0]);
+		ev_record(B.sl.ev_piece[pc]);
+	});
+	B.TM.d2h.stop();
+	B.S.out_bytes = (int64_t)(text_bytes + n_fix * sizeof(GafFix));
+}
+
 // Phase 8: tier routing for the next batch: the first length bucket in which the sampled gaps mostly ended beyond a tier
 static void learn_tier_routing(Batch &B)
 {
@@ -1649,12 +1798,10 @@ static void learn_tier_routing(Batch &B)
 	B.S.skip1_len = B.skip1_len, B.S.skip2_len = B.skip2_len;
 }
 
-// Phase 9: mg_gchains_t of every read, piece by piece as the copies land
-static int assemble_results(Batch &B)
+// Before phase 9: a read that failed on the device fails the call
+static int check_reads(Batch &B)
 {
 	mgb_stats_t &S = B.S;
-	const double t_asm0 = now_ms();
-	S.w_download_ms = t_asm0 - B.t_host0 - S.w_upload_ms - S.w_pass_ms - S.w_redo_ms - S.w_gpu_wait_ms;
 	for (int i = 0; i < B.n_reads; ++i) {
 		const int st = B.read_status(i);
 		if (st < 0) {
@@ -1667,6 +1814,16 @@ static int assemble_results(Batch &B)
 		const ReadMeta &m = B.meta[i];
 		S.n_seeds += m.n_seed0, S.n_anchors_out += m.n_a, S.n_chains_out += m.n_u0, S.n_minimizers += m.n_mz;
 	}
+	return 0;
+}
+
+// Phase 9: mg_gchains_t of every read, piece by piece as the copies land
+static int assemble_results(Batch &B)
+{
+	mgb_stats_t &S = B.S;
+	const double t_asm0 = now_ms();
+	S.w_download_ms = t_asm0 - B.t_host0 - S.w_upload_ms - S.w_pass_ms - S.w_redo_ms - S.w_gpu_wait_ms;
+	if (const int rc = check_reads(B)) return rc;
 	for_pieces(B.n_reads, [&](int pc, int64_t r0, int64_t r1) {
 		ev_wait(B.sl.ev_piece[pc]);
 		B.pfor(r1 - r0, [&](int64_t k) {
@@ -1681,9 +1838,56 @@ static int assemble_results(Batch &B)
 	return 0;
 }
 
-// Map reads [0, n_reads) of one sub-batch on the calling thread's stream (slot `sl`).
+// Phase 9, text route: the caller's text, piece by piece as the copies land, with every record's `dv:f` put in at the byte its
+// fix-up names (the fix-ups came first: the final size is known before the first byte is copied)
+static int assemble_gaf(Batch &B)
+{
+	mgb_stats_t &S = B.S;
+	const double t_asm0 = now_ms();
+	S.w_download_ms = t_asm0 - B.t_host0 - S.w_upload_ms - S.w_pass_ms - S.w_redo_ms - S.w_gpu_wait_ms;
+	if (const int rc = check_reads(B)) return rc;
+	const int n = B.n_reads;
+	const uint64_t *toff = B.gaf_off.data(), *foff = toff + n + 1;
+	ev_wait(B.sl.ev_piece[0]); // (the fix-up records were queued in front of the first piece)
+	const GafFix *fx = (const GafFix*)(B.hout + B.fix_at);
+	enum { DV_MAX = 16 };
+	std::vector<char> dv((size_t)foff[n] * DV_MAX);
+	std::vector<uint8_t> dv_len((size_t)foff[n]);
+	std::vector<uint64_t> at((size_t)n + 1); // where each read's text starts in the output
+	B.pfor(n, [&](int64_t r) {
+		uint64_t add = 0;
+		for (uint64_t k = foff[r]; k < foff[r + 1]; ++k)
+			add += dv_len[k] = (uint8_t)gaf_dv_text(gchain_div(fx[k].n_mini, fx[k].n_anchor, fx[k].q_span), &dv[k * DV_MAX]);
+		at[(size_t)r + 1] = add;
+	});
+	for (int r = 0; r < n; ++r) at[(size_t)r + 1] += at[(size_t)r];
+	for (int r = 0; r <= n; ++r) at[(size_t)r] += toff[r];
+	char *o = gaf_reserve(*B.gaf, at[(size_t)n]);
+	for_pieces(n, [&](int pc, int64_t r0, int64_t r1) {
+		ev_wait(B.sl.ev_piece[pc]);
+		B.pfor(r1 - r0, [&](int64_t i) {
+			const int64_t r = r0 + i;
+			const char *src = B.hout + toff[r];
+			char *dst = o + at[(size_t)r];
+			uint64_t pos = 0;
+			for (uint64_t k = foff[r]; k < foff[r + 1]; ++k) {
+				memcpy(dst, src + pos, fx[k].at - pos), dst += fx[k].at - pos, pos = fx[k].at;
+				memcpy(dst, &dv[k * DV_MAX], dv_len[k]), dst += dv_len[k];
+			}
+			memcpy(dst, src + pos, toff[r + 1] - toff[r] - pos);
+		});
+	});
+	*B.gaf->len = at[(size_t)n];
+	S.t_asm_ms = now_ms() - t_asm0;
+	S.t_d2h_ms = B.TM.d2h.ms();
+	S.t_host_ms = now_ms() - B.t_host0;
+	return 0;
+}
+
+// Map reads [0, n_reads) of one sub-batch on the calling thread's stream (slot `sl`).  The output is either the mg_gchains_t
+// objects in gcs[] or, with gaf (the text route), the GAF text in the caller's buffer.
 static int map_range(Model *M, Model::Slot &sl, const MapOptDev &o, int n_reads, const int *qlens, const char *const *seqs, const char *const *names,
-					 mg_gchains_t **gcs, int host_threads, const std::vector<int32_t> *seg_off = 0, const std::vector<int32_t> *seg_len = 0)
+					 mg_gchains_t **gcs, GafRoute *gaf, int host_threads, const std::vector<int32_t> *seg_off = 0, const std::vector<int32_t> *seg_len = 0)
 {
 	mgb_stats_t &S = sl.st;
 	memset(&S, 0, sizeof(S));
@@ -1692,7 +1896,7 @@ static int map_range(Model *M, Model::Slot &sl, const MapOptDev &o, int n_reads,
 	if (sl.timers == 0) sl.timers = new SlotTimers();
 	sl.timers->reset();
 	const int64_t launches0 = t_launches;
-	Batch B{M, sl, S, *sl.timers, o, n_reads, qlens, seqs, names, gcs, host_threads, seg_off, seg_len, M->skip1_len, M->skip2_len, now_ms()};
+	Batch B{M, sl, S, *sl.timers, o, n_reads, qlens, seqs, names, gcs, gaf, host_threads, seg_off, seg_len, M->skip1_len, M->skip2_len, now_ms()};
 	upload_reads(B);
 	size_pools(B);
 	int rc = 0;
@@ -1712,7 +1916,7 @@ static int map_range(Model *M, Model::Slot &sl, const MapOptDev &o, int n_reads,
 		const bool pool_full = redo_arena_overflows(B);
 		fetch_mail(B.msrc, B.mail);
 		if (B.use_lab) { S.n_lab_new = (int64_t)B.mail->lab_n[0], S.n_lab_big = (int64_t)B.mail->lab_n[1]; lab_after_batch(M, B.mail->lab_n[0]); }
-		if (!pool_full) { download_results(B); break; }
+		if (!pool_full) { if (gaf) download_gaf(B); else download_results(B); break; }
 		// grow whatever overflowed (used counts keep growing past cap, so they tell how much was wanted)
 		for (int i = 0; i < N_POOLS; ++i) if (B.mail->pools[i].used > B.cap[i]) B.cap[i] = (B.mail->pools[i].used * 3 / 2 + 4095) & ~(uint64_t)4095;
 		if (attempt == 7) { set_error("output pools kept overflowing"); rc = -2; break; }
@@ -1722,11 +1926,13 @@ static int map_range(Model *M, Model::Slot &sl, const MapOptDev &o, int n_reads,
 	S.t_wfa_ms = TM.wfa.ms(), S.t_finish_ms = TM.fin.ms();
 	for (int i = 0; i < 10; ++i) S.t_kernel_ms[i] = TM.k[i].ms();
 	S.t_lab_ms = TM.lab.ms();
+	S.t_gaf_ms = TM.gaf_size.ms() + TM.gaf_write.ms();
 	S.arena_peak = B.mail->arena_peak; // (the mailbox was last filled after the last pass of the batch)
 	for (int i = 0; i < 32; ++i) S.prof[i] = (uint64_t)B.mail->prof[i];
 	S.n_launches = t_launches - launches0;
 	learn_tier_routing(B);
-	return rc < 0? rc : assemble_results(B);
+	if (rc < 0) return rc;
+	return gaf? assemble_gaf(B) : assemble_results(B);
 }
 
 static void slot_prepare(Model *M, Model::Slot &sl, int n_workers)
@@ -1751,9 +1957,10 @@ static thread_local bool t_has_stats = false;
 // (callers beyond that wait), so a host that maps mini-batch i+1 on a second thread overlaps its packing, copies and result
 // assembly with the kernels of mini-batch i -- what the reference's kt_pipeline does with its step threads (gmap.c:176).
 static int map_batch_on(Model *M, int n_reads, const int *qlens, const char *const *seqs, const char *const *names,
-						mg_gchains_t **gcs, const mg_mapopt_t *opt, const std::vector<int32_t> *seg_off = 0, const std::vector<int32_t> *seg_len = 0)
+						mg_gchains_t **gcs, const mg_mapopt_t *opt, const std::vector<int32_t> *seg_off = 0, const std::vector<int32_t> *seg_len = 0,
+						GafRoute *gaf = 0)
 {
-	for (int i = 0; i < n_reads; ++i) gcs[i] = 0;
+	if (gcs) for (int i = 0; i < n_reads; ++i) gcs[i] = 0;
 	if (n_reads <= 0) return 0;
 	double t0 = now_ms();
 	int32_t max_qlen = 0;
@@ -1773,6 +1980,7 @@ static int map_batch_on(Model *M, int n_reads, const int *qlens, const char *con
 	try {
 		slot_prepare(M, sl, p_slot_workers > 0? (int)p_slot_workers : default_workers());
 		set_stream(sl.stream);
+		if (gaf) gaf_upload_graph(M, gaf->g);
 		MapOptDev o;
 		fill_opt(o, opt, M->k);
 		{ // glibc logf table for mapq (reference: gcmisc.c:216-217); grown under the lock, old copies are kept until the model dies
@@ -1787,7 +1995,7 @@ static int map_batch_on(Model *M, int n_reads, const int *qlens, const char *con
 			}
 			o.logf_tab = M->d_logf, o.n_logf_tab = M->n_logf;
 		}
-		rc = map_range(M, sl, o, n_reads, qlens, seqs, names, gcs, n_host_threads(), seg_off, seg_len);
+		rc = map_range(M, sl, o, n_reads, qlens, seqs, names, gcs, gaf, n_host_threads(), seg_off, seg_len);
 	} catch (const MgbError &e) {
 		rc = e.code;
 	}
@@ -1805,19 +2013,21 @@ static int map_batch_on(Model *M, int n_reads, const int *qlens, const char *con
 	}
 	M->slot_cv.notify_all();
 	if (rc < 0) { // no partial results are left behind
-		for (int i = 0; i < n_reads; ++i) if (gcs[i]) { mg_gchain_free(gcs[i]); gcs[i] = 0; }
+		if (gcs) for (int i = 0; i < n_reads; ++i) if (gcs[i]) { mg_gchain_free(gcs[i]); gcs[i] = 0; }
 		return rc;
 	}
 	return 0;
 }
 
 // The batch on every device of the index: contiguous parts of about equal bases, one host thread per device, results in input order.
+// The text route: every part formats its own text, and the parts are joined in input order.
 static int map_batch_impl(const mg_idx_t *gi, int n_reads, const int *qlens, const char *const *seqs, const char *const *names,
-						  mg_gchains_t **gcs, const mg_mapopt_t *opt, const std::vector<int32_t> *seg_off = 0, const std::vector<int32_t> *seg_len = 0)
+						  mg_gchains_t **gcs, const mg_mapopt_t *opt, const std::vector<int32_t> *seg_off = 0, const std::vector<int32_t> *seg_len = 0,
+						  GafRoute *gaf = 0)
 {
 	Model *M = (Model*)gi->B;
 	const int n_dev = 1 + (int)M->peers.size();
-	if (n_dev == 1 || seg_off || n_reads < 2 * n_dev) return map_batch_on(M, n_reads, qlens, seqs, names, gcs, opt, seg_off, seg_len);
+	if (n_dev == 1 || seg_off || n_reads < 2 * n_dev) return map_batch_on(M, n_reads, qlens, seqs, names, gcs, opt, seg_off, seg_len, gaf);
 	for (Model *P : M->peers) if (P == 0) { set_error("the index is missing on one of the MGB_DEVICES"); return MGB_E_INTERNAL; }
 	int64_t tot = 0;
 	for (int i = 0; i < n_reads; ++i) tot += qlens[i] > 0? qlens[i] : 0;
@@ -1831,16 +2041,31 @@ static int map_batch_impl(const mg_idx_t *gi, int n_reads, const int *qlens, con
 		}
 	}
 	std::vector<int> rcs((size_t)n_dev, 0);
+	std::vector<char*> txt((size_t)n_dev, (char*)0); // the text route: each part's text
+	std::vector<size_t> txt_len((size_t)n_dev, 0);
+	std::vector<GafRoute> part((size_t)n_dev);
 	std::vector<std::thread> th;
 	for (int d = 0; d < n_dev; ++d)
 		th.emplace_back([&, d]() {
 			const int b = bound[(size_t)d], e = bound[(size_t)d + 1];
-			if (e > b) rcs[(size_t)d] = map_batch_on(d == 0? M : M->peers[(size_t)d - 1], e - b, qlens + b, seqs + b, names? names + b : 0, gcs + b, opt);
+			if (gaf) part[(size_t)d] = GafRoute{gaf->g, &txt[(size_t)d], &txt_len[(size_t)d], 0};
+			if (e > b) rcs[(size_t)d] = map_batch_on(d == 0? M : M->peers[(size_t)d - 1], e - b, qlens + b, seqs + b, names? names + b : 0, gcs? gcs + b : 0, opt, 0, 0,
+													 gaf? &part[(size_t)d] : 0);
 		});
 	for (auto &t : th) t.join();
 	int rc = 0;
 	for (int d = 0; d < n_dev; ++d) if (rcs[(size_t)d] < 0 && rc == 0) rc = rcs[(size_t)d];
-	if (rc < 0) for (int i = 0; i < n_reads; ++i) if (gcs[i]) { mg_gchain_free(gcs[i]); gcs[i] = 0; } // no partial results are left behind
+	if (rc < 0 && gcs) for (int i = 0; i < n_reads; ++i) if (gcs[i]) { mg_gchain_free(gcs[i]); gcs[i] = 0; } // no partial results are left behind
+	if (rc == 0 && gaf) {
+		size_t tot = 0;
+		for (size_t l : txt_len) tot += l;
+		try {
+			char *o = gaf_reserve(*gaf, tot);
+			for (int d = 0; d < n_dev; ++d) if (txt_len[(size_t)d]) memcpy(o, txt[(size_t)d], txt_len[(size_t)d]), o += txt_len[(size_t)d];
+			*gaf->len = tot;
+		} catch (const MgbError &e) { rc = e.code; }
+	}
+	for (char *t : txt) free(t);
 	set_device(M->device);
 	return rc;
 }
@@ -1849,6 +2074,27 @@ extern "C" int mg_map_batch(const mg_idx_t *gi, int n_reads, const int *qlens, c
 							mg_gchains_t **gcs, const mg_mapopt_t *opt)
 {
 	return map_batch_impl(gi, n_reads, qlens, seqs, names, gcs, opt);
+}
+
+// The GAF text of a batch, formatted on the device (include/mgb200.h)
+extern "C" int mgb_map_batch_gaf(const mg_idx_t *gi, int n_reads, const int *qlens, const char *const *seqs, const char *const *names,
+								 const mg_mapopt_t *opt, char **out, size_t *out_len, size_t *out_cap)
+{
+	*out_len = 0;
+	GafRoute R{gi->g, out, out_len, out_cap};
+	int rc = 0;
+	if (opt->flag & (F_WRITE_LCHAIN | F_WRITE_MZ)) {
+		set_error("mgb_map_batch_gaf: the -S / --write-mz records are written from mg_gchains_t only (mg_map_batch + mgb_write_gaf_batch)");
+		rc = MGB_E_UNSUPPORTED;
+	} else if (n_reads <= 0) {
+		try { gaf_reserve(R, 0); } catch (const MgbError &e) { rc = e.code; }
+	} else rc = map_batch_impl(gi, n_reads, qlens, seqs, names, 0, opt, 0, 0, &R);
+	if (rc < 0) { // no text is left behind: the caller's reusable buffer is kept, empty; a buffer of the call's own is not made
+		*out_len = 0;
+		if (out_cap && *out && *out_cap) (*out)[0] = 0;
+		else if (!out_cap) *out = 0;
+	}
+	return rc;
 }
 
 // Fragments of several segments (read pairs) in one go: fragment f has n_seg[f] consecutive entries of qlens/seqs/gcs starting at

@@ -427,6 +427,19 @@ const uint64_t F_WRITE_LCHAIN = 0x800000, F_WRITE_MZ = 0x1000000;
 
 } // namespace
 
+namespace mgb {
+// The `dv:f` field of a record as format.c:200-205 prints it: absent unless 0 <= div <= 1, "0" for 0, else "%.4f".  Writes the
+// field with its leading tab to b (16 bytes are enough) and returns its length, 0 when absent.  mgb_write_gaf() and the text route
+// of the engine (mgb_map_batch_gaf) both print it from here.
+int gaf_dv_text(float div, char *b)
+{
+	if (!(div >= 0.0f && div <= 1.0f)) return 0;
+	memcpy(b, "\tdv:f:", 6);
+	if (div == 0.0f) { b[6] = '0'; return 7; }
+	return 6 + snprintf(b + 6, 10, "%.4f", div);
+}
+}
+
 extern "C" void mgb_write_gaf(char **buf, size_t *len, size_t *cap, const gfa_t *g, const mg_gchains_t *gs, int32_t qlen, const char *qname, uint64_t flag)
 {
 	Str s = { *buf, *len, *cap };
@@ -504,11 +517,9 @@ extern "C" void mgb_write_gaf(char **buf, size_t *len, size_t *cap, const gfa_t 
 		s_puts(s, "\ttp:A:"); s_putc(s, p->id == p->parent? 'P' : 'S');
 		if (p->p) { s_puts(s, "\tNM:i:"); s_putd(s, p->p->blen - p->p->mlen); }
 		s_puts(s, "\tcm:i:"); s_putd(s, p->n_anchor); s_puts(s, "\ts1:i:"); s_putd(s, p->score); s_puts(s, "\ts2:i:"); s_putd(s, p->subsc);
-		if (p->div >= 0.0f && p->div <= 1.0f) {
+		{
 			char b[16];
-			if (p->div == 0.0f) b[0] = '0', b[1] = 0;
-			else snprintf(b, 16, "%.4f", p->div);
-			s_puts(s, "\tdv:f:"); s_puts(s, b);
+			s_putn(s, b, (size_t)mgb::gaf_dv_text(p->div, b));
 		}
 		if (p->p) {
 			s_puts(s, "\tcg:Z:");
